@@ -2,6 +2,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--config C1|C2|C3|C4]     ppx arm (this repo's CUDA path)
   python bench.py --impl reference ...                                           CPU arm: the reference itself
+  python bench.py ... --dump-outputs DIR          also write what the last timed step computed to DIR/<name>.npy
 
 Workloads = BASELINE.json `configs` (SURVEY §8d pins their sizes); the headline line is C2, the configuration the
 metric is quoted on.  A default run also measures C1 / C3 / C4 (sub-records under `configs`, N = 1 only) and one
@@ -93,6 +94,30 @@ def synth_rollout(cfg, seed, n_envs=None):
 
 
 ROLLOUT_FIELDS = ("observations", "actions", "rewards", "values", "masks", "action_log_probs", "int_values")
+# --dump-outputs: at most 4 MB per array and at most 9 arrays (PPO_RND) -> well under 64 MB per dump
+DUMP_MAX_BYTES = 4 << 20
+DUMP_TOTAL_BYTES = 64 << 20
+
+
+def dump_array(x):
+    """Tensor / ndarray -> host ndarray, f64 kept, everything else as f32.  An array over DUMP_MAX_BYTES is reduced to a
+    fixed sample of its flattened elements (sorted indices from a private seeded stream): the same elements in every run
+    of the same configuration, and the global numpy stream the learner's shuffles draw from is not touched."""
+    import torch
+    t = torch.as_tensor(x).detach()
+    dt = np.float64 if t.dtype == torch.float64 else np.float32
+    cap = DUMP_MAX_BYTES // np.dtype(dt).itemsize
+    if t.numel() > cap:
+        idx = np.sort(np.random.RandomState(0).choice(t.numel(), cap, replace=False))
+        t = t.reshape(-1)[torch.as_tensor(idx, device=t.device)]
+    return t.cpu().numpy().astype(dt)
+
+
+def write_outputs(out_dir, arrays):
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_TOTAL_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -580,6 +605,19 @@ class PpxPass:
         self.bonus_and_gae()
         self.m.train()
 
+    def outputs(self):
+        """What one learner pass hands its caller: the loss log of train(), the updated weights of every network it trains,
+        and the rollout's rewards (bonus applied), advantages and returns."""
+        m, ro, alg = self.m, self.ro, self.cfg["alg"]
+        out = {"losses": m.last_losses, "policy_params": m.policy.bank.flat}
+        if alg == "rnd":
+            out["rnd_params"] = m.rnd.bank.flat
+        if alg == "icm":
+            out["icm_params"] = m.intrinsic_module.bank.flat
+        names = ["rewards", "advantages", "returns"] + (["int_rewards", "int_advantages", "int_returns"] if alg == "rnd" else [])
+        out.update((k, getattr(ro, k)) for k in names)
+        return {k: dump_array(v) for k, v in out.items()}
+
     def timed(self, fn, steps):
         import torch.distributed as dist
         torch = self.torch
@@ -598,8 +636,9 @@ class PpxPass:
             dist.barrier()
         return float(ms.item())
 
-    def measure(self, steps, warmup, peaks, clocks=None):
-        """warm-up, K resident steps, K end-to-end steps, one per-op timed pass.  Returns the record (dict)."""
+    def measure(self, steps, warmup, peaks, clocks=None, dump_dir=None):
+        """warm-up, K resident steps, K end-to-end steps, one per-op timed pass.  Returns the record (dict).
+        dump_dir: write the outputs of the last resident step there (before the end-to-end steps change them)."""
         cfg, m, L, torch = self.cfg, self.m, self.L, self.torch
         for _ in range(warmup):
             self.step_resident()
@@ -608,6 +647,8 @@ class PpxPass:
         ms = self.timed(self.step_resident, steps)
         launches, rng_wait = L.launch_count() - l0, m.rng_wait_s - w0
         clk = clocks.stop() if clocks is not None else None
+        if dump_dir is not None:
+            write_outputs(dump_dir, self.outputs())
         self.step_e2e()
         ms_e2e = self.timed(self.step_e2e, steps)
         m.use_cuda_graph = False                                # per-op events need the individual launches, not a graph replay
@@ -668,10 +709,13 @@ def run_ppx(args):
     cfg = CONFIGS[args.config]
     bp = PpxPass(args.config, torch, ppx, dev, rank, world)
     m = bp.m
+    dump_dir = args.dump_outputs if rank == 0 else None        # sharded: rank 0's envs
     if args.profile:
         for _ in range(args.warmup):
             bp.step_resident()
         ms = bp.timed(bp.step_resident, args.steps)
+        if dump_dir is not None:
+            write_outputs(dump_dir, bp.outputs())
         if rank == 0:
             print(json.dumps({"profile_run": True, "ms_per_step": ms / args.steps, "launches": L.launch_count()}))
         return
@@ -689,7 +733,7 @@ def run_ppx(args):
     if sharded:
         m.shard_shuffle = headline_mode
         np.random.seed(1000 + rank if headline_mode == "local" else 0)
-    rec = bp.measure(args.steps, warm, peaks, clocks)
+    rec = bp.measure(args.steps, warm, peaks, clocks, dump_dir=dump_dir)
     line = {"metric": METRIC, "value": rec["value"], "unit": "transitions/s", "n_gpus": world, "steps": args.steps,
             "warmup": warm, "ms_per_step": rec["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic", "config": {"workload": cfg["workload"], "name": args.config},
@@ -769,7 +813,14 @@ def main():
     ap.add_argument("--config", default="C2", choices=sorted(CONFIGS))
     ap.add_argument("--no-subconfigs", action="store_true", help="C2 headline only (skip the C1/C3/C4 sub-records)")
     ap.add_argument("--profile", action="store_true", help="short run for ncu: W warm-up + K steps only, no e2e/CPU legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (losses, trained weights, rewards, advantages, "
+                         "returns) as DIR/<name>.npy; arrays over 4 MB as a fixed seeded sample (ppx arm only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ppx":
+        ap.error("--dump-outputs needs --impl ppx")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -251,3 +251,22 @@ def test_partner_pool_and_worker_pool_reuse():
     assert all(np.array_equal(x, y) for x, y in zip(p1, p2))                         # both started from the same global state
     np.random.seed(2)
     assert np.array_equal(p1[0], np.random.permutation(100))
+
+
+def test_bench_dump_array_caps_size_with_a_fixed_sample():
+    """bench.py --dump-outputs: a large array shrinks to the same sorted sample in every call, without a draw from the
+    global numpy stream (the learner's shuffles draw from it); small arrays keep their shape; f64 stays f64, the rest
+    becomes f32."""
+    import torch
+    import bench
+    np.random.seed(4)
+    state = np.random.get_state()
+    big = torch.arange(3 * (bench.DUMP_MAX_BYTES // 4) + 7, dtype=torch.float32)
+    a, b = bench.dump_array(big), bench.dump_array(big)
+    assert a.dtype == np.float32 and a.nbytes == bench.DUMP_MAX_BYTES and np.array_equal(a, b)
+    assert np.all(np.diff(a) > 0) and np.array_equal(a, big.numpy()[a.astype(np.int64)])
+    after = np.random.get_state()
+    assert np.array_equal(state[1], after[1]) and state[2] == after[2]
+    assert bench.dump_array(np.zeros((40, 8))).dtype == np.float64
+    assert bench.dump_array(torch.zeros(5, 3, dtype=torch.uint8)).shape == (5, 3)
+    assert bench.dump_array(torch.zeros(bench.DUMP_MAX_BYTES // 4, dtype=torch.float64)).nbytes == bench.DUMP_MAX_BYTES

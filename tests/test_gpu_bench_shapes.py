@@ -223,3 +223,26 @@ def test_novelty_distribution_and_brain_pick_product():
         np.random.seed(5)
         idx, n = es.pick_brain(nov)
         assert idx == want_idx and n == nov[idx]
+
+
+def test_dump_outputs_are_the_last_timed_step(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: measure(dump_dir=...) writes the outputs of the last timed resident step, before the
+    end-to-end steps move the learner on -- a fresh pass object stepped warm-up + K times by hand computes the same arrays
+    bit for bit (C2 at 64 envs x 64 steps)."""
+    import os
+    import ppo_exploration_b200 as ppx
+    monkeypatch.setitem(bench.CONFIGS, "C2", dict(bench.CONFIGS["C2"], N=64, T=64, batch=1024))
+    dev = torch.device("cuda", 0)
+    bp = bench.PpxPass("C2", torch, ppx, dev, 0, 1)
+    bp.measure(2, 5, {}, dump_dir=str(tmp_path))
+    del bp
+    got = {f[:-4]: np.load(os.path.join(tmp_path, f)) for f in os.listdir(tmp_path)}
+    assert set(got) == {"losses", "policy_params", "rewards", "advantages", "returns"}
+    assert got["losses"].dtype == np.float64 and got["losses"].shape == (40, 8) and got["advantages"].shape == (64, 64)
+    bp = bench.PpxPass("C2", torch, ppx, dev, 0, 1)
+    for _ in range(5 + 2):
+        bp.step_resident()
+    for k, v in bp.outputs().items():
+        assert v.dtype == got[k].dtype and np.array_equal(v, got[k]), k
+    bp.step_resident()
+    assert not np.array_equal(bp.outputs()["policy_params"], got["policy_params"])

@@ -479,6 +479,24 @@ int ppx_vecnorm_reward(const float* rewards, const uint8_t* dones, double* retur
  * `seed`, counter (env, draw): pass a new `draw` number per call. */
 int ppx_policy_sample(const float* actor_out, const float* log_std, int64_t N, int A, int discrete, uint64_t seed,
                       uint64_t draw, double* actions_out, float* logp_out, void* stream);
+/* Device-env rollout step, first half (replaces Policy.act's sampling and value clones, models.py:30-50 / 75-99, and the
+ * obs / action / value / log-prob copies of RolloutStorage.add, buffer.py:165-186, IntrinsicStorage.add, :305-318): from the
+ * policy forward's outputs (actor_out [N,A], value [N], int_value [N] or NULL, log_std [A]; Box only) and the observation the
+ * policy acted on (obs f32 [N,D], contiguous), draw the actions exactly as ppx_policy_sample does for (seed, draw) and write
+ * rollout step `pos`'s rows: obs_row [N,D], actions_row f64 [N,A], logp_row f32 [N,A], value_row [N], int_value_row [N]
+ * (NULL: none).  env_actions receives a separate copy for the env (Box: f64 [N,A]; Discrete: int64 [N]).  One launch. */
+int ppx_policy_act_record(const float* actor_out, const float* value, const float* int_value, const float* log_std,
+                          const float* obs, int64_t N, int A, int D, int discrete, uint64_t seed, uint64_t draw,
+                          float* obs_row, double* actions_row, float* logp_row, float* value_row, float* int_value_row,
+                          void* env_actions, void* stream);
+/* Device-env rollout step, second half (the reward / mask / int-reward copies of buffer.py:165-186, :305-318): rewards
+ * (f32, or f64 if rewards_f64) [N] cast round-to-nearest into rewards_row; with rewards_f64 and rewards_f64_row non-NULL
+ * they go to that f64 row instead (a SimHash bonus is added to them in f64 later).  dones (bool / uint8 [N]) copied byte for
+ * byte into masks_row; their nonzero count added to *episodes.  int_rewards_row (NULL: none) receives int_rewards, or zeros
+ * if int_rewards is NULL.  One launch. */
+int ppx_rollout_record_step(const void* rewards, int rewards_f64, const uint8_t* dones, const float* int_rewards, int64_t N,
+                            float* rewards_row, double* rewards_f64_row, uint8_t* masks_row, float* int_rewards_row,
+                            int64_t* episodes, void* stream);
 
 /* ---------------------------------------------------------------- ES-NSRA ------------------- */
 /* fill a shared noise table with N(0,1) f32 (Philox4x32-10 + Box-Muller); build-side design, the

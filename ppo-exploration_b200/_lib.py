@@ -134,6 +134,8 @@ SIGNATURES = {
     "ppx_vecnorm_obs": (c_i, [c_p, c_l, c_i, c_p, c_p, c_d, c_d, c_p, c_p]),
     "ppx_vecnorm_reward": (c_i, [c_p, c_p, c_p, c_i, c_d, c_p, c_p, c_p, c_d, c_d, c_i, c_p, c_p]),
     "ppx_policy_sample": (c_i, [c_p, c_p, c_l, c_i, c_i, c_u, c_u, c_p, c_p, c_p]),
+    "ppx_policy_act_record": (c_i, [c_p, c_p, c_p, c_p, c_p, c_l, c_i, c_i, c_i, c_u, c_u, c_p, c_p, c_p, c_p, c_p, c_p, c_p]),
+    "ppx_rollout_record_step": (c_i, [c_p, c_i, c_p, c_p, c_l, c_p, c_p, c_p, c_p, c_p, c_p]),
     "ppx_noise_fill": (c_i, [c_p, c_l, c_u, c_p]),
     "ppx_es_perturb": (c_i, [c_p, c_p, c_p, c_d, c_i, c_i, c_p, c_i, c_p]),
     "ppx_es_forward": (c_i, [c_p, c_p, c_p, c_d, c_i, c_p, c_i, c_p, c_i, c_p, c_p]),

@@ -51,6 +51,7 @@ class BaseAlgorithm(object):
         self.ep_info_buffer = deque(maxlen=50)
         self._n_updates = 0
         self.num_timesteps = 0
+        self._episodes_dev = None              # device path: episodes counted on the GPU, resolved when num_episodes is read
         self.num_episodes = 0
         self.obs_rms = RunningMeanStd(shape=(self.state_dim,), device=self.device, sharded=True)
         self.logger = logger
@@ -89,6 +90,30 @@ class BaseAlgorithm(object):
         sp = getattr(self, "_spec", None)
         if sp is not None:
             sp[0].cancel()
+
+    @property
+    def num_episodes(self):
+        """Episodes ended so far.  On the device path the count since the value was last set lives on the GPU
+        (collect_samples never syncs for it); reading it synchronises once."""
+        n = self._num_episodes
+        if self._episodes_dev is not None:
+            n += int(self._episodes_dev.item())
+        return n
+
+    @num_episodes.setter
+    def num_episodes(self, value):
+        self._num_episodes = value
+        if self._episodes_dev is not None:
+            self._episodes_dev.zero_()
+
+    def _reset_env(self):
+        """env.reset().  An env whose observations come back as CUDA tensors is stepped on the device path of
+        collect_samples (INTEGRATION.md §4: CUDA actions in, CUDA observations / rewards / dones out); numpy envs keep the
+        reference's loop."""
+        self.last_obs = self.env.reset()
+        self.device_env = isinstance(self.last_obs, torch.Tensor) and self.last_obs.is_cuda
+        if self.device_env and self._episodes_dev is None:
+            self._episodes_dev = torch.zeros(1, dtype=torch.int64, device=self.device)
 
     # ---- shared pieces of the fused update --------------------------------------------------
     def _record(self, key, value):
@@ -558,13 +583,15 @@ class PPO(BaseAlgorithm):
         self.rollout = RolloutStorage(nstep, self.num_envs, self.env.observation_space, self.env.action_space,
                                       gae_lam=gae_lam, gamma=gamma, sim_hash=sim_hash, device=self.device,
                                       hash_bits=hash_bits)
-        self.last_obs = self.env.reset()
+        self._reset_env()
         self.sim_hash = sim_hash
         self.sil = sil
 
     def collect_samples(self):
         """algorithms.py:166-198."""
         assert self.last_obs is not None
+        if self.device_env:
+            return self._collect_device()
         self.rollout.reset()
         for _ in range(self.nstep):
             actions, values, log_probs = self.policy.act(self.last_obs)
@@ -578,6 +605,24 @@ class PPO(BaseAlgorithm):
                              log_probs.reshape(self.num_envs, A))
             self.last_obs = obs
         self.rollout.compute_returns_and_advantages(values, dones=dones)
+        return True
+
+    def _collect_device(self):
+        """collect_samples for an env on the GPU, line for line: act_into (forward + one launch writing the step's rows),
+        env.step, record_step (one launch) -- no host sync; SimHash once over the whole rollout.  The env's returned
+        tensors are never read after the next step() (envs commonly reuse their output buffers)."""
+        ro = self.rollout
+        ro.reset()
+        for _ in range(self.nstep):
+            actions, values = self.policy.act_into(self.last_obs, ro)
+            obs, rewards, dones, infos = self.env.step(actions)
+            self.num_timesteps += self.num_envs
+            self.update_info_buffer(infos)
+            ro.record_step(rewards, dones, self._episodes_dev)
+            self.last_obs = obs
+        if ro.do_hash:
+            ro.sim_hash_recorded()
+        ro.compute_returns_and_advantages(values, dones=ro.masks[-1])
         return True
 
     def train(self):
@@ -627,7 +672,7 @@ class PPO_RND(BaseAlgorithm):
         self.int_lr = int_lr
         self.rnd_start = rnd_start
         self.int_vf_coef = int_vf_coef
-        self.last_obs = self.env.reset()
+        self._reset_env()
         self.int_rew_rms = RunningMeanStd(device=self.device, sharded=True)
         self.normalize = True
         self.last_dones = np.array([0 for _ in range(self.num_envs)])
@@ -666,6 +711,8 @@ class PPO_RND(BaseAlgorithm):
     def collect_samples(self):
         """algorithms.py:367-407."""
         assert self.last_obs is not None
+        if self.device_env:
+            return self._collect_device()
         self.rollout.reset()
         for _ in range(self.nstep):
             actions, values, int_values, log_probs = self.policy.act(self.last_obs)
@@ -686,6 +733,28 @@ class PPO_RND(BaseAlgorithm):
             self.last_dones = dones
         mean_int = self.rollout.compute_returns_and_advantages(values, int_values, dones)
         self._mean_int_reward = mean_int                            # logged lazily (rollout/mean_int_reward, buffer.py:335)
+        return True
+
+    def _collect_device(self):
+        """collect_samples for an env on the GPU (see PPO._collect_device).  The warm-up statistics read the observation
+        from the rollout row, not from the env's (possibly reused) tensor."""
+        ro = self.rollout
+        ro.reset()
+        for _ in range(self.nstep):
+            p = ro.pos
+            actions, values, int_values = self.policy.act_into(self.last_obs, ro)
+            obs, rewards, dones, infos = self.env.step(actions)
+            self.num_timesteps += self.num_envs
+            self.update_info_buffer(infos)
+            if (self.num_timesteps / self.num_envs) < self.rnd_start:
+                int_rewards = None                                  # zeros
+                self.obs_rms.update(self.env.unnormalize_obs(ro.observations[p]))
+            else:
+                int_rewards = self.rnd_bonus(obs)
+            ro.record_step(rewards, int_rewards, dones, self._episodes_dev)
+            self.last_obs = obs
+            self.last_dones = ro.masks[p]
+        self._mean_int_reward = ro.compute_returns_and_advantages(values, int_values, ro.masks[-1])
         return True
 
     def train_rnd(self, obs, B_total=0):
@@ -743,7 +812,7 @@ class PPO_ICM(BaseAlgorithm):
         self.intrinsic_module = IntrinsicCuriosityModule(self.state_dim, self.action_converter,
                                                          hidden_size=int_hidden_size, device=self.device)
         self.int_lr = int_lr
-        self.last_obs = self.env.reset()
+        self._reset_env()
         self.policy_weight = policy_weight
         self.beta = 0.2                                             # hard-wired, algorithms.py:600
         self._icm_loss = torch.zeros(1, dtype=torch.float64, device=self.device)
@@ -758,6 +827,8 @@ class PPO_ICM(BaseAlgorithm):
     def collect_samples(self):
         """algorithms.py:603-649."""
         assert self.last_obs is not None
+        if self.device_env:
+            return self._collect_device()
         self.rollout.reset()
         ri_means = []
         for _ in range(self.nstep):
@@ -775,6 +846,26 @@ class PPO_ICM(BaseAlgorithm):
             self.last_obs = obs
         self._mean_int_reward = torch.stack(ri_means).mean()
         self.rollout.compute_returns_and_advantages(values, dones=dones)
+        return True
+
+    def _collect_device(self):
+        """collect_samples for an env on the GPU (see PPO._collect_device).  The bonus reads s and a from the rollout rows
+        (the env may reuse its observation tensor and modify the actions it was given)."""
+        ro = self.rollout
+        ro.reset()
+        ri_means = []
+        for _ in range(self.nstep):
+            p = ro.pos
+            actions, values = self.policy.act_into(self.last_obs, ro)
+            obs, rewards, dones, infos = self.env.step(actions)
+            self.num_timesteps += self.num_envs
+            self.update_info_buffer(infos)
+            rewards, ri = self.icm_bonus(ro.observations[p], obs, ro.actions[p], rewards)
+            ri_means.append(ri.mean())
+            ro.record_step(rewards, dones, self._episodes_dev)
+            self.last_obs = obs
+        self._mean_int_reward = torch.stack(ri_means).mean()
+        ro.compute_returns_and_advantages(values, dones=ro.masks[-1])
         return True
 
     def train(self):

@@ -500,6 +500,7 @@ class RolloutStorage(BaseBuffer):
                         ('old_log_probs', 'action_log_probs'), ('advantages', 'advantages'), ('returns', 'returns')]
         self._mb = {}
         self._load_stream, self._load_done = None, None     # load_rollout(overlap=True)
+        self._rewards_f64, self._staged = None, False       # record_step: f64 rewards awaiting the SimHash bonus
 
     # ------------------------------------------------------------------ storage
     def _alloc(self):
@@ -543,6 +544,53 @@ class RolloutStorage(BaseBuffer):
         self.pos += 1
         if self.pos == self.buffer_size:
             self.full = True
+
+    def record_step(self, reward, done, episodes):
+        """The rest of add() (buffer.py:165-186) for a step whose observation, action, log-prob and value rows were written
+        by Policy.act_into: rewards and masks at row `pos` in ONE launch (ppx_rollout_record_step), and the number of
+        nonzero dones added to `episodes` (int64 CUDA [1]).  reward: f32 / f64 [N] (CUDA or numpy); done: bool / uint8 [N]
+        (CUDA or numpy).  No SimHash here: `sim_hash_recorded()` applies the bonus to the whole rollout afterwards."""
+        self._record(reward, done, episodes, None, None)
+
+    def _record(self, reward, done, episodes, int_reward, int_row):
+        self.await_load()
+        p, N, dev = self.pos, self.n_envs, self.device
+        if isinstance(reward, torch.Tensor) and reward.is_cuda and reward.dtype in (torch.float32, torch.float64):
+            r = reward.reshape(N).contiguous()
+        else:
+            f64 = (reward.dtype == torch.float64) if isinstance(reward, torch.Tensor) else np.asarray(reward).dtype == np.float64
+            r = _dev(reward, torch.float64 if f64 else torch.float32, dev).reshape(N)
+        f64 = r.dtype == torch.float64
+        stage = None
+        if f64 and self.do_hash:
+            if self._rewards_f64 is None:
+                self._rewards_f64 = torch.empty(self.buffer_size, N, dtype=torch.float64, device=dev)
+            stage = self._rewards_f64[p]
+        if p == 0:
+            self._staged = stage is not None
+        elif self._staged != (stage is not None):
+            raise RuntimeError("record_step: the reward dtype changed within a rollout")
+        if not isinstance(done, torch.Tensor):
+            done = torch.as_tensor(np.ascontiguousarray(done))
+        d = done.to(dev, non_blocking=True) if done.dtype in (torch.bool, torch.uint8) else _dev(done, torch.uint8, dev)
+        d = d.reshape(N).contiguous()
+        ir = None if int_reward is None else _dev(int_reward, torch.float32, dev).reshape(N)
+        L.call("ppx_rollout_record_step", r.data_ptr(), int(f64), d.data_ptr(), L.ptr(ir), N, self.rewards[p].data_ptr(),
+               L.ptr(stage), self.masks[p].data_ptr(), L.ptr(int_row), episodes.data_ptr(), L.stream())
+        self.pos += 1
+        if self.pos == self.buffer_size:
+            self.full = True
+
+    def sim_hash_recorded(self):
+        """The SimHash bonus (buffer.py:188-200) of a rollout filled through record_step, applied once to the whole rollout
+        in the reference's order (t-major, env-minor) through sim_hash_sharded: on one GPU the per-step updates of add()
+        bit for bit, sharded the global count table.  f64 rewards get the bonus in f64 and are rounded to f32 once, as in
+        add()."""
+        if self._staged:
+            self.sim_hash_sharded(rewards=self._rewards_f64)
+            self.rewards.copy_(self._rewards_f64)
+        else:
+            self.sim_hash_sharded()
 
     def load_rollout(self, overlap=False, **arrays):
         """Bulk fill from [T,N,...] host or device arrays (one H2D copy per field) and mark full.
@@ -628,8 +676,9 @@ class RolloutStorage(BaseBuffer):
         if W == 1:
             return self.sim_hash(obs, rewards)
         T, N = obs.shape[0], obs.shape[1]
-        if not (isinstance(rewards, torch.Tensor) and rewards.is_cuda and rewards.dtype == torch.float32 and rewards.is_contiguous()):
-            raise RuntimeError("sim_hash_sharded: rewards must be a contiguous f32 CUDA tensor [T, N]")
+        if not (isinstance(rewards, torch.Tensor) and rewards.is_cuda and rewards.dtype in (torch.float32, torch.float64)
+                and rewards.is_contiguous()):
+            raise RuntimeError("sim_hash_sharded: rewards must be a contiguous f32 / f64 CUDA tensor [T, N]")
         codes = self.sim_hash_codes(obs).view(T, N)
         allc = D.interleave_env_shards(D.all_gather_cat(codes)).reshape(-1)          # [T, W*N] in global env order
         # bucket-owner ranks: every rank walks the same ordered list but resolves only the codes it owns (1/W of the
@@ -637,7 +686,8 @@ class RolloutStorage(BaseBuffer):
         counts = self.count_table.update_codes_owned(allc, W, r)
         D.all_reduce_sum_(counts)
         counts = counts.view(T, W, N)[:, r].contiguous()
-        L.call("ppx_simhash_bonus", counts.data_ptr(), T * N, float(self.beta), rewards.data_ptr(), 0, L.stream())
+        L.call("ppx_simhash_bonus", counts.data_ptr(), T * N, float(self.beta), rewards.data_ptr(),
+               int(rewards.dtype == torch.float64), L.stream())
         return rewards
 
     def sim_hash_codes(self, obs):
@@ -776,6 +826,11 @@ class IntrinsicStorage(RolloutStorage):
         self.int_rewards[p].copy_(_dev(int_reward, torch.float32, dev).reshape(self.n_envs))
         self.int_values[p].copy_(_dev(int_value, torch.float32, dev).reshape(self.n_envs))
         super().add(obs, action, reward, value, mask, log_prob)
+
+    def record_step(self, reward, int_reward, done, episodes):
+        """RolloutStorage.record_step with the intrinsic-reward row (buffer.py:305-318) in the same launch; int_reward None
+        writes zeros (RND's warm-up)."""
+        self._record(reward, done, episodes, int_reward, self.int_rewards[self.pos])
 
     def compute_returns_and_advantages(self, last_value, last_int_value, dones):
         """buffer.py:321-362.  Returns mean(int_rewards) as a 0-d CUDA tensor (the value the reference

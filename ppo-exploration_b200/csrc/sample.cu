@@ -8,33 +8,26 @@
 // Randomness: Philox4x32-10 keyed by `seed`, counter = (env, draw number) -- a counter-based stream of ppx's own
 // (torch's generator state is not reproducible from a kernel); the log-probability of the drawn action is exact.
 #include "common.cuh"
-#include "philox.cuh"
+#include "sample_math.cuh"
 
 namespace ppx {
 namespace {
-
-constexpr float kProbEps = 1.1920928955078125e-07f;      // torch.finfo(float32).eps (clamp_probs)
-constexpr float kHalfLog2Pi = 0.91893853320467274178f;   // log(sqrt(2*pi))
 
 __global__ void __launch_bounds__(256)
 sample_box_kernel(const float* __restrict__ actor_out, const float* __restrict__ log_std, int64_t N, int A, uint64_t seed, uint64_t draw,
                   double* __restrict__ actions, float* __restrict__ logp) {
   const int64_t total = N * A;
   for (int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 2; i < total; i += (int64_t)gridDim.x * blockDim.x * 2) {
-    uint32_t c[4] = {(uint32_t)i, (uint32_t)(i >> 32), (uint32_t)draw, (uint32_t)(draw >> 32)};
-    philox4x32(c, seed);
     float z[2];
-    box_muller(c[0], c[1], z[0], z[1]);
+    box_pair_normals(i, seed, draw, z);
 #pragma unroll
     for (int e = 0; e < 2; ++e) {
       if (i + e >= total) break;
       const int a = (int)((i + e) % A);
-      const float mu = tanhf(actor_out[i + e]);
-      const float ls = log_std[a], sigma = expf(ls);
-      const float act = mu + sigma * z[e];                          // Normal.sample: mean + std * eps
-      const float d = act - mu;
+      float act, lp;
+      box_sample(actor_out + i + e, log_std + a, z[e], act, lp);
       actions[i + e] = (double)act;
-      logp[i + e] = -(d * d) / (2.f * sigma * sigma) - logf(sigma) - kHalfLog2Pi;   // Normal.log_prob
+      logp[i + e] = lp;
     }
   }
 }
@@ -43,25 +36,10 @@ __global__ void __launch_bounds__(256)
 sample_discrete_kernel(const float* __restrict__ logits, int64_t N, int A, uint64_t seed, uint64_t draw, double* __restrict__ actions,
                        float* __restrict__ logp) {
   for (int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; n < N; n += (int64_t)gridDim.x * blockDim.x) {
-    const float* l = logits + n * A;
-    float mx = l[0];
-    for (int j = 1; j < A; ++j) mx = fmaxf(mx, l[j]);
-    float se = 0.f;
-    for (int j = 0; j < A; ++j) se += expf(l[j] - mx);
-    float sq = 0.f;                                                 // Categorical(probs=softmax): probs / probs.sum()
-    for (int j = 0; j < A; ++j) sq += expf(l[j] - mx) / se;
-    uint32_t c[4] = {(uint32_t)n, (uint32_t)(n >> 32), (uint32_t)draw, (uint32_t)(draw >> 32)};
-    philox4x32(c, seed);
-    const float u = (float)c[0] * 2.3283064365386963e-10f;           // [0,1)
-    float acc = 0.f;
-    int pick = A - 1;
-    for (int j = 0; j < A; ++j) {
-      acc += (expf(l[j] - mx) / se) / sq;
-      if (u < acc) { pick = j; break; }
-    }
-    const float q = (expf(l[pick] - mx) / se) / sq;
+    float lp;
+    const int pick = discrete_sample(logits + n * A, A, n, seed, draw, lp);
     actions[n] = (double)pick;
-    logp[n] = logf(fminf(fmaxf(q, kProbEps), 1.f - kProbEps));
+    logp[n] = lp;
   }
 }
 

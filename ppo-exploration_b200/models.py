@@ -718,6 +718,30 @@ class Policy:
             return actions, vals[0], vals[1], lp
         return actions, vals[0], lp
 
+    def act_into(self, obs, rollout):
+        """`act` for an env that lives on the GPU, writing straight into rollout step `rollout.pos`: the forward, then ONE
+        launch (collect.cu) that draws the actions exactly as `act` would (same Philox stream, same draw numbers) and writes
+        the observation, f64 actions, log-probs and value(s) rows.  obs: CUDA f32 [N,D].  Returns the actions for env.step
+        in a buffer of their own (Box f64 [N,A], Discrete int64 [N]; the env may modify it) and views of the value rows:
+        (actions, values) or, intrinsic, (actions, values, int_values)."""
+        if not obs.is_cuda or tuple(obs.shape) != (rollout.n_envs, self.state_dim):
+            raise RuntimeError(f"act_into: observations must be a CUDA tensor [{rollout.n_envs}, {self.state_dim}], got "
+                               f"{tuple(obs.shape)} on {obs.device}")
+        obs = obs.float().contiguous()
+        outs = self.forward_raw(obs)
+        N, A = outs[0].shape
+        discrete = self.action_type == "Discrete"
+        p = rollout.pos
+        env_actions = torch.empty((N,) if discrete else (N, A), dtype=torch.int64 if discrete else torch.float64, device=self.device)
+        vals = [rollout.values[p]] + ([rollout.int_values[p]] if self.intrinsic else [])
+        self._draws += 1
+        L.call("ppx_policy_act_record", outs[0].data_ptr(), outs[1].data_ptr(), outs[2].data_ptr() if self.intrinsic else None,
+               None if discrete else self.bank.p("action_log_std"), obs.data_ptr(), N, A, self.state_dim, int(discrete),
+               self._sample_seed, self._draws, rollout.observations[p].data_ptr(), rollout.actions[p].data_ptr(),
+               rollout.action_log_probs[p].data_ptr(), vals[0].data_ptr(), vals[1].data_ptr() if self.intrinsic else None,
+               env_actions.data_ptr(), L.stream())
+        return (env_actions, *vals)
+
     def evaluate(self, obs, actions):
         """models.py:52-73 / 101-124 as plain tensors (train() uses the fused loss kernel instead)."""
         obs = torch.as_tensor(np.asarray(obs) if not isinstance(obs, torch.Tensor) else obs).to(self.device).float()

@@ -517,6 +517,23 @@ int ppx_es_perturb(const double* theta, const float* noise, const int64_t* offse
  * (Discrete: the categorical draw stays with the host RNG).  out is [P, A] f64. */
 int ppx_es_forward(const double* theta, const float* noise, const int64_t* offsets, double sigma, int P,
                    const int* layer_sizes_host, int n_layers, const double* obs, int squash_tanh, double* out, void* stream);
+/* Episode evaluation on an env that lives on the GPU (evaluate / get_action, evolution_strategies.py:75-95, 153-170), env m
+ * running member m.  ppx_es_act: the population forward of ppx_es_forward (same per-member code, bit-identical logits) on
+ * f32 observations obs [N, D0], for the members with alive[m] != 0 (alive NULL: all); a finished member reads no noise and
+ * gets action 0.  actions: Box (discrete = 0) f64 [N, A] = tanh(logits); Discrete int64 [N] = numpy's RandomState.choice
+ * over softmax(logits) -- p = exp(l) / sum(exp(l)) in f64, cdf = cumsum(p) / its last entry, the number of cdf entries
+ * <= u -- with u = uniforms[m] (f64 [N], e.g. numpy's own draws) or, uniforms NULL, the 53-bit uniform of
+ * Philox4x32-10 keyed by `seed` at counter (member_lo + m, step, *draw_dev) (draw_dev NULL: 0).  One launch. */
+int ppx_es_act(const double* theta, const float* noise, const int64_t* offsets, double sigma, int N, const int* layer_sizes_host,
+               int n_layers, const float* obs, const uint8_t* alive, int discrete, uint64_t seed, const int64_t* draw_dev,
+               int64_t step, int64_t member_lo, const double* uniforms, void* actions, void* stream);
+/* ppx_es_episode_step, after env.step, for every member with alive[n] != 0: fitness[n] += reward (f32 or f64 rewards [N],
+ * f64 sum), lengths[n] += 1; when dones[n] != 0 or last_step != 0 the behaviour row behavior[n, 0..k) (NULL: none) is copied
+ * to behavior_out[n] and alive[n] = 0.  state: int64 [3], zero before the first step; state[2] receives the number of
+ * members still running (the other two words are re-armed scratch).  One launch. */
+int ppx_es_episode_step(const void* rewards, int rewards_f64, const uint8_t* dones, const double* behavior, int k, int64_t N,
+                        int last_step, uint8_t* alive, double* fitness, int64_t* lengths, double* behavior_out, int64_t* state,
+                        void* stream);
 /* _update_weights (evolution_strategies.py:217-239): z-score rewards (ddof 0); skip entirely if std==0;
  * theta += lr/(P*sigma) * sum_p w_p eps_p with w_p = ((1-nw)*z_p + nw*novelty)/2 (use_novelty=1) or z_p;
  * then *lr_inout *= decay.  rank_mode=1 replaces the z-score by centred ranks (BASELINE north_star;

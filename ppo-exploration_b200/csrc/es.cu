@@ -13,6 +13,7 @@
 //                                                      split over members, fixed-order reduction)
 // Parity mode passes a dense [P,D] eps (offsets == NULL) holding the very values given to the
 // reference.  All state (theta, lr) stays on device; the std==0 early-out of :225-226 is a device flag.
+#include "es_walk.cuh"
 #include "p2p.cuh"
 #include "philox.cuh"
 
@@ -90,13 +91,10 @@ perturb_vec_kernel(const double* __restrict__ theta, const float* __restrict__ n
 // ---------------- population forward (FeedForwardNetwork.predict, evolution_strategies.py:48-61) ----------------
 // Every member p acts on its own observation with weights theta + sigma*eps_p formed on the fly from the noise table --
 // the perturbed weights are never materialised (ppx_es_perturb writes 8 D bytes per member for the same purpose).
-// One warp per member: theta and the layer plan are staged once per CTA in shared memory; a layer  out = a . W
-// (W [in, out] row-major inside the flat vector, bias-free) is walked 8 inputs at a time -- lane j owns output columns
-// j, j+32, ... so a warp reads 128 contiguous bytes of eps per input, all loads of a step in flight before the math.
+// The per-member layer walk is es_walk.cuh (shared with ppx_es_act).
 // fp32 arithmetic (the reference is f64; the B200's FP64 pipe made an f64 version 6x slower than this one -- 250 us vs
 // 40 us at C5 -- and the path's bound is 1e-5 relative): hidden layers arctan (:57), last layer linear, then tanh for
 // Box action spaces (continuous_action :84-89).
-constexpr int kFwdMaxLayers = 8, kFwdMaxWidth = 256;
 struct EsFwdP {
   const double* theta; const float* noise; const int64_t* offsets; float sigma; int P, D, n_layers;
   int sizes[kFwdMaxLayers + 1];
@@ -117,106 +115,8 @@ __global__ void __launch_bounds__(256) es_forward_kernel(EsFwdP p) {
     const float* eps = p.noise + (p.offsets ? __ldg(p.offsets + m) : (int64_t)m * p.D);
     for (int i = lane; i < p.sizes[0]; i += 32) a0[i] = (float)__ldg(p.obs + (size_t)m * p.sizes[0] + i);
     __syncwarp();
-    float* in = a0;
-    float* outv = a1;
-    int woff = 0;
-    for (int l = 0; l < p.n_layers; ++l) {
-      const int ni = p.sizes[l], no = p.sizes[l + 1];
-      if (p.vec[l] == 4) {
-        // 16-byte path (no = 4 nq, nq a power of two <= 32): lane = (row slot rs = lane / nq, column quad q = lane % nq), a warp
-        // instruction covers 32 / nq consecutive input rows = 512 contiguous bytes; 8 steps of loads in flight before the math
-        const int nq = no >> 2, rps = 32 / nq, rs = lane / nq, q = lane - rs * nq;
-        float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-        for (int i0 = 0; i0 < ni; i0 += 8 * rps) {
-          float4 e[8];
-#pragma unroll
-          for (int u = 0; u < 8; ++u) {
-            const int i = i0 + u * rps + rs;
-            e[u] = i < ni ? ld_stream4(reinterpret_cast<const float4*>(eps + woff + (size_t)i * no) + q) : make_float4(0.f, 0.f, 0.f, 0.f);
-          }
-#pragma unroll
-          for (int u = 0; u < 8; ++u) {
-            const int i = i0 + u * rps + rs;
-            if (i < ni) {
-              const float ai = in[i];
-              const float4 t = *reinterpret_cast<const float4*>(th + woff + (size_t)i * no + 4 * q);
-              acc.x = fmaf(ai, fmaf(p.sigma, e[u].x, t.x), acc.x); acc.y = fmaf(ai, fmaf(p.sigma, e[u].y, t.y), acc.y);
-              acc.z = fmaf(ai, fmaf(p.sigma, e[u].z, t.z), acc.z); acc.w = fmaf(ai, fmaf(p.sigma, e[u].w, t.w), acc.w);
-            }
-          }
-        }
-        for (int d = nq; d < 32; d <<= 1) {                  // combine the row slots (fixed order)
-          acc.x += __shfl_xor_sync(0xffffffffu, acc.x, d); acc.y += __shfl_xor_sync(0xffffffffu, acc.y, d);
-          acc.z += __shfl_xor_sync(0xffffffffu, acc.z, d); acc.w += __shfl_xor_sync(0xffffffffu, acc.w, d);
-        }
-        if (rs == 0) {
-          const float v[4] = {acc.x, acc.y, acc.z, acc.w};
-#pragma unroll
-          for (int c = 0; c < 4; ++c) {
-            const int j = 4 * q + c;
-            if (l + 1 < p.n_layers) outv[j] = atanf(v[c]);
-            else p.out[(size_t)m * no + j] = (double)(p.squash ? tanhf(v[c]) : v[c]);
-          }
-        }
-      } else if (p.vec[l] == 1) {
-        // narrow layer (no a power of two <= 32, e.g. the action head): the same slot scheme with one column per lane, so the
-        // whole warp streams the layer's contiguous weights instead of `no` lanes walking them row by row
-        const int rps = 32 / no, rs = lane / no, j = lane - rs * no;
-        float acc = 0.f;
-        for (int i0 = 0; i0 < ni; i0 += 8 * rps) {
-          float e[8];
-#pragma unroll
-          for (int u = 0; u < 8; ++u) {
-            const int i = i0 + u * rps + rs;
-            e[u] = i < ni ? ld_stream(eps + woff + (size_t)i * no + j) : 0.f;
-          }
-#pragma unroll
-          for (int u = 0; u < 8; ++u) {
-            const int i = i0 + u * rps + rs;
-            if (i < ni) acc = fmaf(in[i], fmaf(p.sigma, e[u], th[woff + (size_t)i * no + j]), acc);
-          }
-        }
-        for (int d = no; d < 32; d <<= 1) acc += __shfl_xor_sync(0xffffffffu, acc, d);
-        if (rs == 0) {
-          if (l + 1 < p.n_layers) outv[j] = atanf(acc);
-          else p.out[(size_t)m * no + j] = (double)(p.squash ? tanhf(acc) : acc);
-        }
-      } else
-      for (int j0 = 0; j0 < no; j0 += 64) {                 // scalar path: 2 output columns per lane per sweep
-        const bool l0 = j0 + lane < no, l1 = j0 + lane + 32 < no;
-        float acc0 = 0.f, acc1 = 0.f;
-        for (int i0 = 0; i0 < ni; i0 += 8) {
-          float e0[8], e1[8];
-#pragma unroll
-          for (int u = 0; u < 8; ++u) {
-            const float* er = eps + woff + (size_t)(i0 + u) * no + j0 + lane;
-            e0[u] = (i0 + u < ni && l0) ? ld_stream(er) : 0.f;
-            e1[u] = (i0 + u < ni && l1) ? ld_stream(er + 32) : 0.f;
-          }
-#pragma unroll
-          for (int u = 0; u < 8; ++u) {
-            if (i0 + u < ni) {
-              const float ai = in[i0 + u];
-              const float* tr = th + woff + (size_t)(i0 + u) * no + j0 + lane;
-              if (l0) acc0 = fmaf(ai, fmaf(p.sigma, e0[u], tr[0]), acc0);
-              if (l1) acc1 = fmaf(ai, fmaf(p.sigma, e1[u], tr[32]), acc1);
-            }
-          }
-        }
-#pragma unroll
-        for (int c = 0; c < 2; ++c) {
-          const int j = j0 + lane + 32 * c;
-          if (j < no) {
-            float v = c ? acc1 : acc0;
-            if (l + 1 < p.n_layers) outv[j] = atanf(v);
-            else p.out[(size_t)m * no + j] = (double)(p.squash ? tanhf(v) : v);
-          }
-        }
-      }
-      __syncwarp();
-      woff += ni * no;
-      float* t = in; in = outv; outv = t;
-    }
+    es_member_walk(p, eps, th, a0, a1, lane,
+                   [&](int j, int no, float v) { p.out[(size_t)m * no + j] = (double)(p.squash ? tanhf(v) : v); });
   }
 }
 
@@ -507,28 +407,13 @@ extern "C" int ppx_es_forward(const double* theta, const float* noise, const int
                               const int* layer_sizes, int n_layers, const double* obs, int squash_tanh, double* out,
                               void* stream) {
   PPX_REQUIRE(theta && noise && layer_sizes && obs && out, "es_forward: null pointer");
-  PPX_REQUIRE(P >= 1 && n_layers >= 1 && n_layers <= kFwdMaxLayers, "es_forward: P=%d n_layers=%d", P, n_layers);
+  PPX_REQUIRE(P >= 1, "es_forward: P=%d", P);
   EsFwdP p{};
-  p.theta = theta; p.noise = noise; p.offsets = offsets; p.sigma = (float)sigma; p.P = P; p.n_layers = n_layers;
+  p.theta = theta; p.noise = noise; p.offsets = offsets; p.sigma = (float)sigma; p.P = P;
   p.obs = obs; p.out = out; p.squash = squash_tanh;
-  int D = 0;
-  for (int l = 0; l <= n_layers; ++l) {
-    PPX_REQUIRE(layer_sizes[l] >= 1 && layer_sizes[l] <= kFwdMaxWidth, "es_forward: layer width %d not in [1, %d]", layer_sizes[l], kFwdMaxWidth);
-    p.sizes[l] = layer_sizes[l];
-    if (l) D += layer_sizes[l - 1] * layer_sizes[l];
-  }
-  p.D = D;
-  {
-    int woff = 0;
-    const bool base_ok = (((uintptr_t)noise & 15) == 0) && (offsets != nullptr || D % 4 == 0);   // table offsets are multiples of 4
-    for (int l = 0; l < n_layers; ++l) {
-      const int no = layer_sizes[l + 1], nq = no / 4;
-      if (base_ok && no % 4 == 0 && nq <= 32 && (nq & (nq - 1)) == 0 && woff % 4 == 0) p.vec[l] = 4;
-      else if (no <= 32 && (no & (no - 1)) == 0) p.vec[l] = 1;
-      else p.vec[l] = 0;
-      woff += layer_sizes[l] * no;
-    }
-  }
+  int rc = es_plan(p, noise, offsets, layer_sizes, n_layers, "es_forward");
+  if (rc) return rc;
+  const int D = p.D;
   const size_t smem = sizeof(float) * ((size_t)((D + 3) & ~3) + 8 * 2 * kFwdMaxWidth);
   PPX_REQUIRE(smem <= 227 * 1024, "es_forward: %d parameters do not fit in shared memory", D);
   static size_t configured = 0;

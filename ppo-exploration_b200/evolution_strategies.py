@@ -4,9 +4,10 @@ Mirrors EvolutionStrategy of evolution_strategies.py (:100-384) for the parts on
 path: _get_population (:172-182), _get_weights_try (:137-145), _update_weights (:217-239), get_kNN
 (:264-281), the novelty lines (:318-325) and calc_noveltiy_distribution (:283-290), plus the policy forward
 of episode evaluation (FeedForwardNetwork.predict :48-61) batched over the population
-(`predict_population`, SURVEY §8f.4).  Stepping the environments (evaluate / get_behavior_char / run's env
-loop) is the simulator side and stays with the caller: feed the fitness vector back through
-`_update_weights`.
+(`predict_population`, SURVEY §8f.4).  For a batched env that lives on the GPU, `evaluate` runs the episode loop of
+evaluate / get_behavior_char (:153-170) on the device -- fitness, episode lengths and behaviour characterisations -- and
+`run_generation` chains ask -> evaluate -> tell.  For an env on the host, the caller steps it with `predict_population` /
+`discrete_action` and feeds the fitness vector back through `_update_weights` or `tell`.
 
 Build-side design (SURVEY §0.1): the population is a vector of offsets into ONE resident f32 noise
 table instead of P fresh f64 randn tensors; theta is one flat f64 device vector over all layers.
@@ -287,6 +288,148 @@ class EvolutionStrategy(object):
             nov = self._novelty[brain:brain + 1] if self._novelty is not None else None
             self._update_weights(r_all, self._ask_off, novelty=nov)
         return self._graph(key, fn)
+
+    # ---- episode evaluation on an env that lives on the GPU (INTEGRATION.md §4) ----
+    def evaluate(self, env, population=None, *, max_steps, sigma=None, check_every=8, member_lo=None, uniforms=None):
+        """evaluate / get_behavior_char (:153-170) with get_action (:75-95) for a batched env on the GPU: env i runs member i
+        (global member member_lo + i) for ONE episode.  Per step two libppx launches and no host sync: `ppx_es_act` (the
+        forward of the members still running on the env's f32 observations; Box: tanh(logits) f64 [N, A], Discrete: one
+        categorical draw int64 [N]; finished members get action 0) and, after env.step, `ppx_es_episode_step`.
+
+        A member's fitness is the f64 sum, in step order, of its rewards up to and including its first done; later rewards,
+        dones and behaviours of its env are ignored.  If the env has `behavior()` (CUDA f64 [N, k], the state reached by the
+        last step(), before any auto-reset), a member's row is latched at its terminating step.  A member still running after
+        `max_steps` steps keeps the sum so far and the behaviour of that step.  Every `check_every` steps the device count of
+        running members is copied into pinned memory without blocking, and the loop stops once a copy reads 0; the steps
+        issued after the last member ended change nothing, so the results do not depend on `check_every`.
+
+        population: offsets or dense eps as in `predict_population`; default this rank's slice of the last `ask()` (with
+        member_lo = rank * P/W), or with sigma=0.0 and no ask() yet, theta itself on every env (the meta-member behaviour of
+        :318-325).  The Discrete draw is numpy's RandomState.choice arithmetic on u = a Philox uniform keyed by (noise seed,
+        the device draw counter, step, global member), so every rank draws the same action for the same member; `uniforms`
+        (CUDA f64 [max_steps, N]) supplies u instead, e.g. numpy's own draws.
+        Returns (fitness f64 [N], lengths int64 [N], behaviour f64 [N, k] or None), CUDA buffers that the next evaluate()
+        of the same shape overwrites -- `tell(fitness)` replays its captured graph."""
+        if max_steps < 1 or check_every < 1:
+            raise ValueError(f"max_steps={max_steps} and check_every={check_every} must be >= 1")
+        sig = float(self.SIGMA if sigma is None else sigma)
+        N = int(env.num_envs)
+        if population is None:
+            if hasattr(self, "_ask_off"):
+                W = D.world_size()
+                population = self.shard_population(self._ask_off) if W > 1 else self._ask_off
+                if member_lo is None:
+                    member_lo = D.rank() * (self.POPULATION_SIZE // W)
+            elif sig == 0.0:
+                population = torch.zeros(N, dtype=torch.int64, device=self.device)
+            else:
+                raise ValueError("evaluate() needs a population: call ask() first or pass one")
+        noise, off = self._as_eps(population)
+        P = off.numel() if off is not None else noise.shape[0]
+        if P != N:
+            raise ValueError(f"the env runs {N} envs but the population has {P} members (one env per member)")
+        space = env.action_space
+        discrete = getattr(space, "n", None) is not None and not getattr(space, "shape", ())
+        A = int(space.n) if discrete else int(space.shape[-1])
+        if A != self.shapes[-1][1]:
+            raise ValueError(f"the env has {A} actions, the network {self.shapes[-1][1]}")
+        if uniforms is not None:
+            L.require_cuda(uniforms, torch.float64, "uniforms")
+            if tuple(uniforms.shape) != (max_steps, N):
+                raise ValueError(f"uniforms must be [{max_steps}, {N}], got {tuple(uniforms.shape)}")
+        obs = env.reset()
+        if not (isinstance(obs, torch.Tensor) and obs.is_cuda):
+            raise TypeError("evaluate() steps environments that live on the GPU: env.reset() must return a CUDA tensor "
+                            f"(got {type(obs).__name__}); for an env returning numpy, loop over predict_population / "
+                            "discrete_action on the host")
+        buf = self._eval_buffers(N, A, discrete)
+        buf["fitness"].zero_()
+        buf["lengths"].zero_()
+        buf["alive"].fill_(1)
+        buf["state"].zero_()
+        has_bc = callable(getattr(env, "behavior", None))
+        bc_out = None
+        sizes = [self.shapes[0][0]] + [sh[1] for sh in self.shapes]
+        import ctypes as C
+        sizes_c = (C.c_int * len(sizes))(*sizes)
+        st = L.stream()
+        acts = buf["actions"]
+        t = 0
+        while t < max_steps:
+            o = self._device_input(obs, torch.float32, (N, sizes[0]), "observations")
+            L.call("ppx_es_act", self.theta.data_ptr(), noise.data_ptr(), off.data_ptr() if off is not None else None, sig, N,
+                   sizes_c, len(sizes) - 1, o.data_ptr(), buf["alive"].data_ptr(), int(discrete), self._noise_seed + 2,
+                   self._draw.data_ptr(), t, int(member_lo or 0), uniforms[t].data_ptr() if uniforms is not None else None,
+                   acts.data_ptr(), st)
+            obs, rew, done, _ = env.step(acts)
+            rew = self._device_input(rew, None, (N,), "rewards")
+            done = self._device_input(done, torch.uint8, (N,), "dones")
+            bc = None
+            if has_bc:
+                bc = env.behavior()
+                if not (isinstance(bc, torch.Tensor) and bc.is_cuda):
+                    raise TypeError("env.behavior() must return a CUDA tensor [N, k]")
+                bc = bc.reshape(N, -1).to(torch.float64).contiguous()
+                if bc_out is None:
+                    bc_out = self._eval_bc(N, bc.shape[1])
+            L.call("ppx_es_episode_step", rew.data_ptr(), int(rew.dtype == torch.float64), done.data_ptr(),
+                   bc.data_ptr() if bc is not None else None, bc.shape[1] if bc is not None else 0, N, int(t == max_steps - 1),
+                   buf["alive"].data_ptr(), buf["fitness"].data_ptr(), buf["lengths"].data_ptr(),
+                   bc_out.data_ptr() if bc is not None else None, buf["state"].data_ptr(), st)
+            t += 1
+            if t % check_every == 0 and t < max_steps:
+                if buf["polled"] and buf["event"].query() and int(buf["host"][0]) == 0:
+                    break
+                buf["host"].copy_(buf["state"][2:3], non_blocking=True)
+                buf["event"].record()
+                buf["polled"] = True
+        buf["polled"] = False
+        self.last_eval_steps = t
+        return buf["fitness"], buf["lengths"], bc_out
+
+    def _eval_buffers(self, N, A, discrete):
+        if not hasattr(self, "_eval"):
+            self._eval = {}
+        key = (N, A, discrete)
+        if key not in self._eval:
+            dev = self.device
+            self._eval[key] = dict(
+                fitness=torch.zeros(N, dtype=torch.float64, device=dev), lengths=torch.zeros(N, dtype=torch.int64, device=dev),
+                alive=torch.ones(N, dtype=torch.uint8, device=dev), state=torch.zeros(3, dtype=torch.int64, device=dev),
+                actions=torch.zeros(N, dtype=torch.int64, device=dev) if discrete else
+                torch.zeros(N, A, dtype=torch.float64, device=dev),
+                host=torch.zeros(1, dtype=torch.int64).pin_memory(), event=torch.cuda.Event(), polled=False)
+        return self._eval[key]
+
+    def _eval_bc(self, N, k):
+        key = ("bc", N, k)
+        if key not in self._eval:
+            self._eval[key] = torch.zeros(N, k, dtype=torch.float64, device=self.device)
+        return self._eval[key]
+
+    def _device_input(self, x, dtype, shape, name):
+        """An env output as a contiguous CUDA tensor of `shape`: dtype None keeps f32 / f64 (other types become f64); uint8
+        accepts bool as is.  Numpy arrays are copied up (an env on the GPU returns CUDA tensors)."""
+        if not isinstance(x, torch.Tensor):
+            x = torch.as_tensor(np.asarray(x)).to(self.device)
+        if dtype is None:
+            dtype = x.dtype if x.dtype in (torch.float32, torch.float64) else torch.float64
+        if dtype == torch.uint8 and x.dtype == torch.bool:
+            x = x.view(torch.uint8)
+        elif dtype == torch.uint8 and x.dtype != torch.uint8:
+            x = (x != 0).to(torch.uint8)
+        x = x.to(dtype).reshape(shape).contiguous()
+        if x.device != self.theta.device:
+            raise ValueError(f"{name} live on {x.device}, the ES on {self.theta.device}")
+        return x
+
+    def run_generation(self, env, *, max_steps, archive=None, queries=None, brain=0, check_every=8):
+        """One ES generation on an env that lives on the GPU: ask() -> evaluate() of this rank's members -> tell().  Sharded,
+        every rank evaluates its P/W envs and tell() gathers the fitness.  Returns what evaluate() returned."""
+        self.ask(archive, queries)
+        out = self.evaluate(env, max_steps=max_steps, check_every=check_every)
+        self.tell(out[0], brain=brain)
+        return out
 
     @property
     def update_skipped(self):

@@ -498,6 +498,31 @@ int ppx_rollout_record_step(const void* rewards, int rewards_f64, const uint8_t*
                             float* rewards_row, double* rewards_f64_row, uint8_t* masks_row, float* int_rewards_row,
                             int64_t* episodes, void* stream);
 
+/* ---------------------------------------------------------------- classic control ----------- */
+/* Gym 0.17 classic-control envs with TimeLimit, on the device (classic_control.cu; DESIGN.md §3.13).  env: 0 CartPole-v1,
+ * 1 MountainCar-v0, 2 MountainCarContinuous-v0, 3 Pendulum-v0.  State f64 [S, N] (S = 4, 2, 2, 2), observations f32 [N, D]
+ * (D = 4, 2, 2, 3).  Per env: elapsed steps, episode number, monitor accumulators (f64 return, length) and the return / length
+ * of the last finished episode.  Reset draws: Philox4x32-10 under `seed`, counter (global env env_offset + n, episode number).
+ * step: actions int64 [N] (Discrete) or f64 [N, 1] (Box); reward f32 (rounded once from f64) or f64 [N] (reward_f64); done
+ * uint8 [N]; behavior (NULL: none) f64 [N, S] receives the pre-reset state; finished envs are reset in place.  reset: every
+ * env starts its next episode.  One launch each. */
+int ppx_classic_step(int env, int64_t N, int64_t env_offset, uint64_t seed, const void* actions, double* state, int64_t* elapsed,
+                     int64_t* episode, double* mon_ret, int64_t* mon_len, double* ep_ret, int64_t* ep_len, float* obs, void* reward,
+                     int reward_f64, uint8_t* done, double* behavior, void* stream);
+int ppx_classic_reset(int env, int64_t N, int64_t env_offset, uint64_t seed, double* state, int64_t* elapsed, int64_t* episode,
+                      double* mon_ret, int64_t* mon_len, float* obs, void* stream);
+/* Episode monitor of any env on the device: acc_ret += reward (f32 or f64 [N], f64 sum), acc_len += 1; where dones[n] != 0
+ * the sums go to ep_ret[n] / ep_len[n] and restart from 0.  One launch. */
+int ppx_episode_monitor_step(const void* rewards, int rewards_f64, const uint8_t* dones, int64_t N, double* acc_ret, int64_t* acc_len,
+                             double* ep_ret, int64_t* ep_len, void* stream);
+/* Learner episode log.  record: where dones[n] != 0, ep_ret[n] / ep_len[n] -> log rows (one step, [N]).  tail: over the flat
+ * t-major done flags [total] and the log, the newest min(K, #dones) finished episodes go to out_ret / out_len [K], newest
+ * first, and their number to *out_count.  One launch each (tail: one block). */
+int ppx_episode_log_record(const uint8_t* dones, const double* ep_ret, const int64_t* ep_len, int64_t N, double* log_ret_row,
+                           int64_t* log_len_row, void* stream);
+int ppx_episode_log_tail(const uint8_t* dones, const double* log_ret, const int64_t* log_len, int64_t total, int64_t K,
+                         double* out_ret, int64_t* out_len, int64_t* out_count, void* stream);
+
 /* ---------------------------------------------------------------- ES-NSRA ------------------- */
 /* fill a shared noise table with N(0,1) f32 (Philox4x32-10 + Box-Muller); build-side design, the
  * reference draws fresh randn per member (evolution_strategies.py:172-182). */

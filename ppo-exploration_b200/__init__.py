@@ -13,7 +13,9 @@ from .algorithms import BaseAlgorithm, PPO, PPO_RND, PPO_ICM
 from .evolution_strategies import EvolutionStrategy
 from .spaces import Box, Discrete, SyntheticVecEnv
 from .env import VecNormalize
+from .classic_control import ClassicControlVecEnv, EpisodeMonitor, ToNumpy, make_env
 
 __all__ = ["BaseBuffer", "RolloutStorage", "IntrinsicStorage", "CountTable", "discount_with_dones", "Policy",
            "RndNetwork", "IntrinsicCuriosityModule", "ActionConverter", "RunningMeanStd", "normalize_obs",
-           "BaseAlgorithm", "PPO", "PPO_RND", "PPO_ICM", "EvolutionStrategy", "Box", "Discrete", "SyntheticVecEnv", "logger", "VecNormalize", "ConvTrunk", "ParamBank"]
+           "BaseAlgorithm", "PPO", "PPO_RND", "PPO_ICM", "EvolutionStrategy", "Box", "Discrete", "SyntheticVecEnv", "logger", "VecNormalize", "ConvTrunk", "ParamBank",
+           "ClassicControlVecEnv", "EpisodeMonitor", "ToNumpy", "make_env"]

@@ -136,7 +136,12 @@ SIGNATURES = {
     "ppx_policy_sample": (c_i, [c_p, c_p, c_l, c_i, c_i, c_u, c_u, c_p, c_p, c_p]),
     "ppx_policy_act_record": (c_i, [c_p, c_p, c_p, c_p, c_p, c_l, c_i, c_i, c_i, c_u, c_u, c_p, c_p, c_p, c_p, c_p, c_p, c_p]),
     "ppx_rollout_record_step": (c_i, [c_p, c_i, c_p, c_p, c_l, c_p, c_p, c_p, c_p, c_p, c_p]),
-    "ppx_noise_fill": (c_i, [c_p, c_l, c_u, c_p]),
+    "ppx_classic_step": (c_i, [c_i, c_l, c_l, c_u, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_p, c_p, c_p]),
+    "ppx_classic_reset": (c_i, [c_i, c_l, c_l, c_u, c_p, c_p, c_p, c_p, c_p, c_p, c_p]),
+    "ppx_episode_monitor_step": (c_i, [c_p, c_i, c_p, c_l, c_p, c_p, c_p, c_p, c_p]),
+    "ppx_episode_log_record": (c_i, [c_p, c_p, c_p, c_l, c_p, c_p, c_p]),
+    "ppx_episode_log_tail": (c_i, [c_p, c_p, c_p, c_l, c_l, c_p, c_p, c_p, c_p]),
+    "ppx_noise_fill":(c_i, [c_p, c_l, c_u, c_p]),
     "ppx_es_perturb": (c_i, [c_p, c_p, c_p, c_d, c_i, c_i, c_p, c_i, c_p]),
     "ppx_es_forward": (c_i, [c_p, c_p, c_p, c_d, c_i, c_p, c_i, c_p, c_i, c_p, c_p]),
     "ppx_es_act": (c_i, [c_p, c_p, c_p, c_d, c_i, c_p, c_i, c_p, c_p, c_i, c_u, c_p, c_l, c_l, c_p, c_p, c_p]),

@@ -48,6 +48,7 @@ class BaseAlgorithm(object):
         self.lr, self.nstep, self.batch_size, self.n_epochs = lr, nstep, batch_size, n_epochs
         self.gamma, self.gae_lam, self.clip_range = gamma, gae_lam, clip_range
         self.ent_coef, self.vf_coef, self.max_grad_norm = ent_coef, vf_coef, max_grad_norm
+        self._ep_pending, self._ep_free, self._ep_log = [], [], None   # device episode log (episode_stats() envs)
         self.ep_info_buffer = deque(maxlen=50)
         self._n_updates = 0
         self.num_timesteps = 0
@@ -105,6 +106,74 @@ class BaseAlgorithm(object):
         self._num_episodes = value
         if self._episodes_dev is not None:
             self._episodes_dev.zero_()
+
+    @property
+    def ep_info_buffer(self):
+        """The last finished episodes as {"r": return, "l": length} (the reference's Monitor entries).  On the device path
+        with an env that has `episode_stats()`, each rollout's newest episodes are selected on the GPU and copied to pinned
+        memory without blocking; reading the buffer appends them, waiting for the copy if it is still running."""
+        self._ep_resolve(wait=True)
+        return self._ep_info_buffer
+
+    @ep_info_buffer.setter
+    def ep_info_buffer(self, value):
+        self._ep_free += self._ep_pending
+        self._ep_pending = []
+        self._ep_info_buffer = value
+
+    def _ep_resolve(self, wait):
+        """Append the pending episode-log tails in rollout order (wait=False: only those whose copy has landed)."""
+        while self._ep_pending:
+            slot = self._ep_pending[0]
+            if wait:
+                slot["event"].synchronize()
+            elif not slot["event"].query():
+                return
+            K = slot["ret"].numel()
+            n = int(slot["len"][K])
+            rets, lens = slot["ret"][:n].tolist(), slot["len"][:n].tolist()   # newest first
+            self._ep_info_buffer.extend({"r": round(r, 6), "l": int(l)} for r, l in zip(rets[::-1], lens[::-1]))
+            self._ep_free.append(self._ep_pending.pop(0))
+
+    def _episode_log_begin(self):
+        """Device path: the env's `episode_stats` (None if it has none) and the [T, N] log of this rollout."""
+        stats = getattr(self.env, "episode_stats", None)
+        if not callable(stats):
+            return None
+        T, N = self.rollout.buffer_size, self.num_envs
+        if self._ep_log is None or tuple(self._ep_log[0].shape) != (T, N):
+            self._ep_log = (torch.zeros(T, N, dtype=torch.float64, device=self.device),
+                            torch.zeros(T, N, dtype=torch.int64, device=self.device))
+        self._ep_resolve(wait=False)
+        return stats
+
+    def _episode_log_step(self, stats, t):
+        """One launch after record_step: the finished envs' (return, length) into row t of the log."""
+        ret, lens = stats()
+        if not (ret.is_cuda and ret.dtype == torch.float64 and lens.dtype == torch.int64 and ret.is_contiguous()
+                and lens.is_contiguous() and ret.numel() == lens.numel() == self.num_envs):
+            raise TypeError("env.episode_stats() must return contiguous CUDA (f64 [N] returns, int64 [N] lengths)")
+        L.call("ppx_episode_log_record", self.rollout.masks[t].data_ptr(), ret.data_ptr(), lens.data_ptr(), self.num_envs,
+               self._ep_log[0][t].data_ptr(), self._ep_log[1][t].data_ptr(), L.stream())
+
+    def _episode_log_end(self):
+        """One launch after the rollout: the newest maxlen finished episodes (the rollout's masks are the done flags), then
+        an asynchronous copy to pinned memory; `ep_info_buffer` appends them when read."""
+        masks = self.rollout.masks
+        K = self._ep_info_buffer.maxlen or masks.numel()
+        slot = next((s for s in self._ep_free if s["ret"].numel() == K), None)
+        if slot is None:
+            slot = dict(ret=torch.zeros(K, dtype=torch.float64).pin_memory(), len=torch.zeros(K + 1, dtype=torch.int64).pin_memory(),
+                        d_ret=torch.zeros(K, dtype=torch.float64, device=self.device),
+                        d_len=torch.zeros(K + 1, dtype=torch.int64, device=self.device), event=torch.cuda.Event())
+        else:
+            self._ep_free.remove(slot)
+        L.call("ppx_episode_log_tail", masks.data_ptr(), self._ep_log[0].data_ptr(), self._ep_log[1].data_ptr(), masks.numel(), K,
+               slot["d_ret"].data_ptr(), slot["d_len"].data_ptr(), slot["d_len"].data_ptr() + 8 * K, L.stream())
+        slot["ret"].copy_(slot["d_ret"], non_blocking=True)
+        slot["len"].copy_(slot["d_len"], non_blocking=True)
+        slot["event"].record()
+        self._ep_pending.append(slot)
 
     def _reset_env(self):
         """env.reset().  An env whose observations come back as CUDA tensors is stepped on the device path of
@@ -613,13 +682,19 @@ class PPO(BaseAlgorithm):
         tensors are never read after the next step() (envs commonly reuse their output buffers)."""
         ro = self.rollout
         ro.reset()
+        stats = self._episode_log_begin()
         for _ in range(self.nstep):
+            p = ro.pos
             actions, values = self.policy.act_into(self.last_obs, ro)
             obs, rewards, dones, infos = self.env.step(actions)
             self.num_timesteps += self.num_envs
             self.update_info_buffer(infos)
             ro.record_step(rewards, dones, self._episodes_dev)
+            if stats is not None:
+                self._episode_log_step(stats, p)
             self.last_obs = obs
+        if stats is not None:
+            self._episode_log_end()
         if ro.do_hash:
             ro.sim_hash_recorded()
         ro.compute_returns_and_advantages(values, dones=ro.masks[-1])
@@ -740,6 +815,7 @@ class PPO_RND(BaseAlgorithm):
         from the rollout row, not from the env's (possibly reused) tensor."""
         ro = self.rollout
         ro.reset()
+        stats = self._episode_log_begin()
         for _ in range(self.nstep):
             p = ro.pos
             actions, values, int_values = self.policy.act_into(self.last_obs, ro)
@@ -752,8 +828,12 @@ class PPO_RND(BaseAlgorithm):
             else:
                 int_rewards = self.rnd_bonus(obs)
             ro.record_step(rewards, int_rewards, dones, self._episodes_dev)
+            if stats is not None:
+                self._episode_log_step(stats, p)
             self.last_obs = obs
             self.last_dones = ro.masks[p]
+        if stats is not None:
+            self._episode_log_end()
         self._mean_int_reward = ro.compute_returns_and_advantages(values, int_values, ro.masks[-1])
         return True
 
@@ -853,6 +933,7 @@ class PPO_ICM(BaseAlgorithm):
         (the env may reuse its observation tensor and modify the actions it was given)."""
         ro = self.rollout
         ro.reset()
+        stats = self._episode_log_begin()
         ri_means = []
         for _ in range(self.nstep):
             p = ro.pos
@@ -863,7 +944,11 @@ class PPO_ICM(BaseAlgorithm):
             rewards, ri = self.icm_bonus(ro.observations[p], obs, ro.actions[p], rewards)
             ri_means.append(ri.mean())
             ro.record_step(rewards, dones, self._episodes_dev)
+            if stats is not None:
+                self._episode_log_step(stats, p)
             self.last_obs = obs
+        if stats is not None:
+            self._episode_log_end()
         self._mean_int_reward = torch.stack(ri_means).mean()
         ro.compute_returns_and_advantages(values, dones=ro.masks[-1])
         return True

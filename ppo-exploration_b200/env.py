@@ -6,7 +6,9 @@ observations / rewards (clip 10, epsilon 1e-8, gamma 0.99).  This class does the
 host vec-env (num_envs, observation_space, action_space, reset(), step()): the raw observations and rewards are
 uploaded once per step, the statistics are updated and the normalisation applied by libppx kernels, and the results
 stay on the device -- `Policy.act` and `RolloutStorage.add` take CUDA tensors, so the rollout row is written without
-another host round trip.  `unnormalize_obs` (used by PPO_RND's warm-up, algorithms.py:392) is provided.
+another host round trip.  `unnormalize_obs` (used by PPO_RND's warm-up, algorithms.py:392) is provided.  An inner env
+that lives on the GPU (its reset() returns a CUDA tensor) is wrapped with no upload at all: actions go to it as CUDA
+tensors and its CUDA dones come back; its `episode_stats()` / `behavior()` (raw, unnormalised) are forwarded.
 
 stable_baselines3 is not part of the reference tree nor of this image: the arithmetic follows its published
 VecNormalize.step_wait / RunningMeanStd (same update rule as the reference's util.py:9-44, which IS pinned) and is
@@ -32,6 +34,10 @@ class VecNormalize(object):
         self.ret_rms = RunningMeanStd(shape=(), device=self.device)
         self.ret = torch.zeros(self.num_envs, dtype=torch.float64, device=self.device)
         self.old_obs = None                                     # raw observations of the last step (device)
+        self._cuda_inner = False                                # set by reset(): the inner env returns CUDA tensors
+        for name in ("episode_stats", "behavior"):              # raw episode statistics / states pass through
+            if callable(getattr(venv, name, None)):
+                setattr(self, name, getattr(venv, name))
 
     # ---- helpers ----
     def _up(self, x, dtype):
@@ -58,7 +64,11 @@ class VecNormalize(object):
 
     # ---- VecEnv surface ----
     def reset(self):
-        obs = self._up(self.venv.reset(), torch.float32)
+        o = self.venv.reset()
+        self._cuda_inner = isinstance(o, torch.Tensor) and o.is_cuda
+        if self._cuda_inner:
+            return self._reset_cuda(o)
+        obs = self._up(o, torch.float32)
         self.old_obs = obs
         self.ret.zero_()
         if self.training and self.norm_obs:
@@ -66,7 +76,10 @@ class VecNormalize(object):
         return self.normalize_obs(obs)
 
     def step(self, actions):
-        """actions: CUDA tensor or numpy.  Returns (obs, rewards) as CUDA f32 tensors, dones as the env's numpy bools, infos."""
+        """actions: CUDA tensor or numpy.  Returns (obs, rewards) as CUDA f32 tensors, dones as the env's numpy bools, infos.
+        An inner env on the GPU gets the actions as they are and its CUDA dones come back (no host round trip)."""
+        if self._cuda_inner:
+            return self._step_cuda(actions)
         a = actions.detach().cpu().numpy() if isinstance(actions, torch.Tensor) else actions
         obs, rews, dones, infos = self.venv.step(a)
         obs_d, r_d = self._up(obs, torch.float32), self._up(rews, torch.float32)
@@ -85,3 +98,33 @@ class VecNormalize(object):
             self.ret.mul_(self.gamma).add_(r_d.double())
             self.ret[d_d.bool()] = 0.0
         return obs_n, r_d, dones, infos
+
+    # ---- inner env on the GPU: the same arithmetic, no host upload ----
+    def _reset_cuda(self, o):
+        obs = o.to(torch.float32).contiguous().clone()              # the inner env may overwrite its buffer on step()
+        self.old_obs = obs
+        self.ret.zero_()
+        if self.training and self.norm_obs:
+            self.obs_rms.update(obs)
+        return self.normalize_obs(obs)
+
+    def _step_cuda(self, actions):
+        obs, rews, dones, infos = self.venv.step(actions)
+        obs_d = obs.to(torch.float32).contiguous().clone()
+        r_d = rews.to(torch.float32).reshape(self.num_envs).contiguous()
+        d = dones.reshape(self.num_envs).contiguous()
+        d_d = d.view(torch.uint8) if d.dtype == torch.bool else d if d.dtype == torch.uint8 else (d != 0).to(torch.uint8)
+        self.old_obs = obs_d
+        if self.training and self.norm_obs:
+            self.obs_rms.update(obs_d)
+        obs_n = self.normalize_obs(obs_d)
+        out = torch.empty_like(r_d)
+        if self.norm_reward:
+            L.call("ppx_vecnorm_reward", r_d.data_ptr(), d_d.data_ptr(), self.ret.data_ptr(), self.num_envs, self.gamma,
+                   self.ret_rms.mean_dev.data_ptr(), self.ret_rms.var_dev.data_ptr(), self.ret_rms.count_dev.data_ptr(), self.epsilon,
+                   self.clip_reward, int(self.training), out.data_ptr(), L.stream())
+        else:
+            out.copy_(r_d)
+            self.ret.mul_(self.gamma).add_(r_d.double())
+            self.ret.masked_fill_(d_d.bool(), 0.0)                  # not boolean indexing: that syncs
+        return obs_n, out, d_d, infos

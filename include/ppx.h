@@ -92,6 +92,13 @@ int ppx_simhash_bonus(const uint32_t* counts, int64_t n, double beta, void* rewa
 int ppx_count_table_size(ppx_count_table* t, uint64_t* n_keys_host);
 int ppx_count_table_dump(ppx_count_table* t, uint64_t* keys_dev, uint32_t* counts_dev, uint64_t max_out,
                          uint64_t* n_out_host);
+/* checkpoint restore into an EMPTY table (PPX_ERR_ARG otherwise): grows it until n keys fit at <= 50 % load and inserts
+ * the (key, count) pairs; afterwards updates, growth and ppx_count_table_size behave as on the table that was dumped.
+ * Synchronous.  A duplicate key or a zero count returns PPX_ERR_ARG and leaves the table empty. */
+int ppx_count_table_load(ppx_count_table* t, const uint64_t* keys_dev, const uint32_t* counts_dev, uint64_t n,
+                         void* stream);
+/* the table's current capacity (a power of two; the all-ones key lives in one extra slot) */
+int ppx_count_table_capacity(ppx_count_table* t, uint64_t* capacity_host);
 
 /* ---------------------------------------------------------------- shuffle-gather ------------ */
 /* RolloutStorage._get_samples, buffer.py:256-267 / :384-394, without materialising the env-major

@@ -6,6 +6,7 @@ the C ABI in include/ppx.h; there is no CPU fallback.
 """
 from . import _lib
 from . import logger
+from . import checkpoint
 from .buffer import BaseBuffer, RolloutStorage, IntrinsicStorage, CountTable, discount_with_dones
 from .models import Policy, RndNetwork, IntrinsicCuriosityModule, ActionConverter, ConvTrunk, ParamBank
 from .util import RunningMeanStd, normalize_obs

@@ -63,6 +63,8 @@ SIGNATURES = {
     "ppx_simhash_bonus": (c_i, [c_p, c_l, c_d, c_p, c_i, c_p]),
     "ppx_count_table_size": (c_i, [c_p, C.POINTER(c_u)]),
     "ppx_count_table_dump": (c_i, [c_p, c_p, c_p, c_u, C.POINTER(c_u)]),
+    "ppx_count_table_load": (c_i, [c_p, c_p, c_p, c_u, c_p]),
+    "ppx_count_table_capacity": (c_i, [c_p, C.POINTER(c_u)]),
     "ppx_gather_minibatch": (c_i, [C.POINTER(c_p), C.POINTER(c_p), C.POINTER(c_i), c_i, c_p, c_l, c_i, c_i, c_p]),
     "ppx_gather_minibatch_stats": (c_i, [C.POINTER(c_p), C.POINTER(c_p), C.POINTER(c_i), c_i, c_p, c_l, c_i, c_i, C.POINTER(c_i),
                                          C.POINTER(c_p), c_i, c_p, c_p]),

@@ -87,10 +87,128 @@ class BaseAlgorithm(object):
         self.rng_wait_s = 0.0                  # cumulative host time train() spent waiting for permutations
         self.device_shuffle = device_shuffle_default()         # swaps of the epoch shuffle applied on the GPU (shuffle_dev.cu)
 
+    def __new__(cls, *args, **kwargs):
+        obj = super().__new__(cls)
+        # the constructor's keyword arguments, less the live objects, are what `load` rebuilds a saved learner from
+        obj._init_kwargs = {k: v for k, v in kwargs.items() if k not in ("env", "device", "logger")}
+        return obj
+
     def __del__(self):
         sp = getattr(self, "_spec", None)
         if sp is not None:
             sp[0].cancel()
+
+    # ---- checkpoints (DESIGN.md §3.14) -----------------------------------------------------------
+    def _ckpt_banks(self):
+        return {"policy": self.policy.bank}
+
+    def _ckpt_rms(self):
+        return {"obs_rms": self.obs_rms}
+
+    @staticmethod
+    def _env_shape(env):
+        sp = env.action_space
+        kind = sp.__class__.__name__
+        return {"num_envs": int(env.num_envs), "obs_dim": int(env.observation_space.shape[0]), "action_space": kind,
+                "action_n": int(sp.n) if kind == "Discrete" else int(sp.shape[0]), "world_size": D.world_size(),
+                "rank": D.rank()}
+
+    def _ckpt_shape(self):
+        return dict(self._env_shape(self.env), learner=type(self).__name__, hidden_size=int(self.policy.hidden_size),
+                    nstep=int(self.nstep), hash_bits=int(self.rollout.A.shape[0]))
+
+    @staticmethod
+    def _shape_check(saved, mine):
+        bad = [f"{k}: saved {saved.get(k)!r}, here {v!r}" for k, v in mine.items() if saved.get(k) != v]
+        if bad:
+            raise ValueError("the checkpoint does not fit this learner (" + "; ".join(bad) + ")")
+
+    def save(self, path):
+        """Write everything the run depends on to `path`, one `torch.save` file that loads with `weights_only=True`
+        (DESIGN.md §3.14): every parameter bank with its Adam moments and step counter, the SimHash projection and count
+        table, the running statistics, the counters and rollout-side host state, numpy's global RNG state and -- when the
+        env implements `state_dict()` (INTEGRATION.md §4) -- the env's state.  `Cls.load(path, env=...)` continues the run
+        bit for bit.
+
+        Valid at an iteration boundary: before the first `collect_samples()` or after a `train()` (where `learn()` returns).
+        A collected rollout that was not trained yet is not saved: RuntimeError.  Saving synchronises but draws nothing
+        from numpy, so the run goes on exactly as if it had not been saved.  Under torch.distributed every rank saves its
+        own file: pass a per-rank path."""
+        from .checkpoint import header, np_rng_state, pack, scalar
+        ro = self.rollout
+        if ro.pos > 0 and not ro.generator_ready:
+            raise RuntimeError("save(): the collected rollout has not been trained yet (save before collect_samples() or "
+                               "after train())")
+        save_env = getattr(self.env, "state_dict", None)
+        ck = header(type(self).__name__)
+        ck.update(
+            config={k: scalar(v) for k, v in self._init_kwargs.items()},
+            shape=self._ckpt_shape(),
+            banks={k: b.state_dict() for k, b in self._ckpt_banks().items()},
+            rms={k: r.state_dict() for k, r in self._ckpt_rms().items()},
+            simhash={"A": torch.from_numpy(np.array(ro.A, dtype=np.float64)),
+                     "count_table": ro.count_table.state_dict() if ro.count_table is not None else None},
+            counters={"num_timesteps": int(self.num_timesteps), "num_episodes": int(self.num_episodes),
+                      "n_updates": int(self._n_updates), "draws": int(self.policy._draws),
+                      "sample_seed": int(self.policy._sample_seed)},
+            host={"ep_info_buffer": [{k: scalar(v) for k, v in e.items()} for e in self.ep_info_buffer],
+                  "ep_info_maxlen": self._ep_info_buffer.maxlen, "last_obs": pack(self.last_obs),
+                  "device_env": bool(self.device_env), "last_dones": pack(getattr(self, "last_dones", None)),
+                  "train_stats": {k: scalar(v) for k, v in self.train_stats.items()}, "shard_shuffle": self.shard_shuffle},
+            env=save_env() if callable(save_env) else None,
+            numpy_rng=np_rng_state(),
+        )
+        torch.save(ck, path)
+
+    @classmethod
+    def load(cls, path, env, device="cuda", logger=None):
+        """The learner saved at `path` by `save()`, built from its saved constructor arguments over `env`, with its whole
+        state restored: the next `collect_samples()` / `train()` / `learn()` compute what the saved learner would have.
+
+        Sets numpy's global RNG (`np.random.set_state`) to its state at save(): the reference's shuffle and randn draws
+        continue from there.  If `env` implements `state_dict()` / `load_state_dict()` (INTEGRATION.md §4) its saved state
+        is restored and `resumed_env_state` is True.  Otherwise the learner starts from `env.reset()` (made by the
+        constructor), `resumed_env_state` is False, and the resume is NOT bit-identical to the uninterrupted run.
+        ValueError when the checkpoint does not fit: another learner class or format version, another number of envs,
+        observation dim, action space, hidden size, nstep, hash_bits, world size or rank."""
+        from .checkpoint import read
+        ck = read(path, cls.__name__)
+        cls._shape_check(ck["shape"], cls._env_shape(env))
+        self = cls(env=env, device=device, logger=logger, **ck["config"])
+        self._shape_check(ck["shape"], self._ckpt_shape())
+        self._load_state(ck)
+        return self
+
+    def _load_state(self, ck):
+        from .checkpoint import np_rng_tuple, unpack
+        for k, b in self._ckpt_banks().items():
+            b.load_state_dict(ck["banks"][k])
+        for k, r in self._ckpt_rms().items():
+            r.load_state_dict(ck["rms"][k])
+        ro, sh = self.rollout, ck["simhash"]
+        if tuple(sh["A"].shape) != tuple(ro.A.shape):
+            raise ValueError(f"checkpoint SimHash projection {tuple(sh['A'].shape)}, expected {tuple(ro.A.shape)}")
+        ro.A = sh["A"].numpy().copy()
+        if (sh["count_table"] is None) != (ro.count_table is None):
+            raise ValueError("the checkpoint and this learner disagree on sim_hash")
+        if ro.count_table is not None:
+            ro.count_table.load_state_dict(sh["count_table"])
+        c, h = ck["counters"], ck["host"]
+        self.num_timesteps, self.num_episodes, self._n_updates = c["num_timesteps"], c["num_episodes"], c["n_updates"]
+        self.policy._draws, self.policy._sample_seed = c["draws"], c["sample_seed"]
+        load_env = getattr(self.env, "load_state_dict", None)
+        self.resumed_env_state = callable(load_env) and ck["env"] is not None
+        if self.resumed_env_state:
+            if h["device_env"] != self.device_env:
+                raise ValueError("the saved env and this one differ in where they live (GPU / host)")
+            load_env(ck["env"])
+            self.last_obs = unpack(h["last_obs"], self.device)
+            if hasattr(self, "last_dones"):
+                self.last_dones = unpack(h["last_dones"], self.device)
+        self.ep_info_buffer = deque(h["ep_info_buffer"], maxlen=h["ep_info_maxlen"])
+        self.train_stats = dict(h["train_stats"])
+        self.shard_shuffle = h["shard_shuffle"]
+        np.random.set_state(np_rng_tuple(ck["numpy_rng"]))
 
     @property
     def num_episodes(self):
@@ -753,6 +871,12 @@ class PPO_RND(BaseAlgorithm):
         self.last_dones = np.array([0 for _ in range(self.num_envs)])
         self._rnd_loss = torch.zeros(1, dtype=torch.float64, device=self.device)
 
+    def _ckpt_banks(self):
+        return dict(super()._ckpt_banks(), rnd_predictor=self.rnd.bank, rnd_target=self.rnd.target_bank)
+
+    def _ckpt_rms(self):
+        return dict(super()._ckpt_rms(), int_rew_rms=self.int_rew_rms)
+
     def rnd_bonus(self, obs):
         """The bonus lines of collect_samples after warm-up (algorithms.py:394-398) for one env step:
         normalise -> (pred-target)^2 -> int_rew_rms.update -> divide.  obs [N,D]; returns [N] f32 CUDA."""
@@ -896,6 +1020,9 @@ class PPO_ICM(BaseAlgorithm):
         self.policy_weight = policy_weight
         self.beta = 0.2                                             # hard-wired, algorithms.py:600
         self._icm_loss = torch.zeros(1, dtype=torch.float64, device=self.device)
+
+    def _ckpt_banks(self):
+        return dict(super()._ckpt_banks(), icm=self.intrinsic_module.bank)
 
     def icm_bonus(self, last_obs, obs, actions, rewards):
         """algorithms.py:629-630: r = (1-eta) r + eta * clamp(mean_f((fwd(phi(s),a) - phi(s'))^2), -5, 5).

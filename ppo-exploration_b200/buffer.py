@@ -476,6 +476,44 @@ class CountTable:
                     mine.update(p)
         return mine
 
+    def capacity(self):
+        c = C.c_uint64()
+        L.call("ppx_count_table_capacity", self._h, C.byref(c))
+        return int(c.value)
+
+    def state_dict(self):
+        """This rank's part of the table for a checkpoint: the keys (uint64 codes as int64 bit patterns) and counts, sorted
+        by key on the host so that the file does not depend on the dump's atomic order, the capacity and the `sharded`
+        flag.  Synchronous."""
+        n = len(self)
+        keys = torch.empty(max(n, 1), dtype=torch.int64, device="cuda")
+        counts = torch.empty(max(n, 1), dtype=torch.int32, device="cuda")
+        got = C.c_uint64()
+        L.call("ppx_count_table_dump", self._h, keys.data_ptr(), counts.data_ptr(), n, C.byref(got))
+        k = keys[:n].cpu().numpy().view(np.uint64)
+        order = np.argsort(k, kind="stable")
+        return {"keys": torch.from_numpy(k[order].view(np.int64).copy()), "counts": counts[:n].cpu()[torch.from_numpy(order)],
+                "capacity": self.capacity(), "sharded": bool(getattr(self, "sharded", False))}
+
+    def load_state_dict(self, sd):
+        """Replace the table by the one `state_dict()` described: a new table at the saved capacity (so growth happens at
+        the same calls as on the original), filled by one insert kernel (ppx_count_table_load).  Synchronous."""
+        keys, counts = sd["keys"], sd["counts"]
+        if keys.dtype != torch.int64 or counts.dtype != torch.int32 or keys.dim() != 1 or keys.shape != counts.shape:
+            raise ValueError("count table state: keys must be int64 [n] and counts int32 [n]")
+        h = C.c_void_p()
+        L.call("ppx_count_table_create", int(sd["capacity"]), C.byref(h))
+        try:
+            if keys.numel():
+                k, c = keys.to("cuda"), counts.to("cuda")
+                L.call("ppx_count_table_load", h, k.data_ptr(), c.data_ptr(), keys.numel(), L.stream())
+        except BaseException:
+            L.call("ppx_count_table_destroy", h)
+            raise
+        L.call("ppx_count_table_destroy", self._h)
+        self._h = h
+        self.sharded = bool(sd["sharded"])
+
 
 class RolloutStorage(BaseBuffer):
     """buffer.py:111-267."""

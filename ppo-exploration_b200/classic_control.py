@@ -107,6 +107,31 @@ class ClassicControlVecEnv:
     def unnormalize_obs(self, obs):
         return obs
 
+    # the device tensors that make up the env's state, and the settings a checkpoint must agree with
+    _STATE = ("state", "_elapsed", "_episode", "_mon_ret", "_mon_len", "_ep_ret", "_ep_len", "_obs", "_rew", "_done",
+              "_behavior")
+
+    def _settings(self):
+        return {"env_id": self.env_id, "num_envs": self.num_envs, "seed": self.seed, "env_offset": self.env_offset,
+                "reward_dtype": str(self._rew.dtype).replace("torch.", "")}
+
+    def state_dict(self):
+        """Everything the next step() depends on, as CPU tensors (INTEGRATION.md §4): the f64 state, elapsed steps, episode
+        numbers (they key the reset draws), the monitor accumulators, the last episode statistics and the output buffers,
+        plus env_id, num_envs, seed, env_offset and the reward dtype."""
+        sd = self._settings()
+        sd.update({k.lstrip("_"): getattr(self, k).cpu() for k in self._STATE})
+        return sd
+
+    def load_state_dict(self, sd):
+        """Restore `state_dict()`; ValueError if the settings or shapes differ from this env's."""
+        from .checkpoint import tensor_into
+        for k, mine in self._settings().items():
+            if sd.get(k) != mine:
+                raise ValueError(f"{self.env_id}: the saved env has {k}={sd.get(k)!r}, this one {mine!r}")
+        for k in self._STATE:
+            tensor_into(getattr(self, k), sd[k.lstrip("_")], f"env '{k.lstrip('_')}'")
+
 
 class EpisodeMonitor:
     """`episode_stats()` for any env on the GPU (INTEGRATION.md §4): one extra launch per step accumulates the f64 return
@@ -119,6 +144,8 @@ class EpisodeMonitor:
         dev = getattr(venv, "device", None) or torch.device("cuda")
         self._acc_ret, self._ep_ret = (torch.zeros(N, dtype=torch.float64, device=dev) for _ in range(2))
         self._acc_len, self._ep_len = (torch.zeros(N, dtype=torch.int64, device=dev) for _ in range(2))
+        if callable(getattr(venv, "state_dict", None)):        # the state protocol only if the wrapped env has it
+            self.state_dict, self.load_state_dict = self._state_dict, self._load_state_dict
 
     def __getattr__(self, name):
         return getattr(self.__dict__["venv"], name)
@@ -143,6 +170,17 @@ class EpisodeMonitor:
     def episode_stats(self):
         return self._ep_ret, self._ep_len
 
+    def _state_dict(self):
+        sd = {k.lstrip("_"): getattr(self, k).cpu() for k in ("_acc_ret", "_acc_len", "_ep_ret", "_ep_len")}
+        sd["venv"] = self.venv.state_dict()
+        return sd
+
+    def _load_state_dict(self, sd):
+        from .checkpoint import tensor_into
+        for k in ("_acc_ret", "_acc_len", "_ep_ret", "_ep_len"):
+            tensor_into(getattr(self, k), sd[k.lstrip("_")], f"episode monitor '{k.lstrip('_')}'")
+        self.venv.load_state_dict(sd["venv"])
+
 
 class ToNumpy:
     """A numpy surface over an env on the GPU: numpy obs / rewards / bool dones and SB3-style `infos` whose finished envs
@@ -153,6 +191,8 @@ class ToNumpy:
         self.env = env
         self.num_envs = env.num_envs
         self.observation_space, self.action_space = env.observation_space, env.action_space
+        if callable(getattr(env, "state_dict", None)):          # the state protocol is the wrapped env's
+            self.state_dict, self.load_state_dict = env.state_dict, env.load_state_dict
 
     def reset(self):
         return self.env.reset().cpu().numpy()

@@ -485,6 +485,18 @@ __global__ void rehash_kernel(const uint64_t* __restrict__ okeys, const uint32_t
   ncounts[slot] = ocounts[s];
 }
 
+// checkpoint restore: pair i goes to its slot (the all-ones key to the dedicated slot cap) and its count is stored with a
+// CAS from 0, so a key given twice -- and a zero count, which no table entry can hold -- raises `bad` instead of merging
+__global__ void load_kernel(const uint64_t* __restrict__ keys_in, const uint32_t* __restrict__ counts_in, uint64_t n,
+                            uint64_t* keys, uint32_t* counts, uint64_t cap, uint32_t* ctrl, uint32_t* bad) {
+  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const uint32_t c = counts_in[i];
+  if (c == 0u) { atomicOr(bad, 2u); return; }
+  const uint64_t slot = find_or_claim(keys, cap, ctrl, keys_in[i]);
+  if (atomicCAS(&counts[slot], 0u, c) != 0u) atomicOr(bad, 1u);
+}
+
 int alloc_arrays(uint64_t cap, uint64_t** keys, uint32_t** counts) {
   PPX_CUDA(cudaMalloc((void**)keys, (cap + 1) * sizeof(uint64_t)));
   PPX_CUDA(cudaMalloc((void**)counts, (cap + 1) * sizeof(uint32_t)));
@@ -701,4 +713,52 @@ extern "C" int ppx_count_table_dump(ppx_count_table* t, uint64_t* keys_dev, uint
   cudaFree(n_dev);
   *n_out_host = n_h;
   return rc;
+}
+
+extern "C" int ppx_count_table_capacity(ppx_count_table* t, uint64_t* capacity_host) {
+  PPX_REQUIRE(t && capacity_host, "count_table_capacity: bad arguments");
+  *capacity_host = t->capacity;
+  return PPX_OK;
+}
+
+extern "C" int ppx_count_table_load(ppx_count_table* t, const uint64_t* keys_dev, const uint32_t* counts_dev, uint64_t n,
+                                    void* stream) {
+  PPX_REQUIRE(t && (n == 0 || (keys_dev && counts_dev)), "count_table_load: bad arguments");
+  PPX_REQUIRE(n < (1ull << 31), "count_table_load: %llu keys (at most 2^31 - 1)", (unsigned long long)n);
+  const cudaStream_t st = (cudaStream_t)stream;
+  uint32_t ctrl_h[4], special = 0;
+  PPX_CUDA(cudaMemcpyAsync(ctrl_h, t->ctrl, sizeof(ctrl_h), cudaMemcpyDeviceToHost, st));
+  PPX_CUDA(cudaMemcpyAsync(&special, t->counts + t->capacity, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+  PPX_CUDA(cudaStreamSynchronize(st));
+  PPX_REQUIRE(ctrl_h[2] == 0 && special == 0 && ctrl_h[3] == 0, "count_table_load: the table is not empty (%u keys)",
+              ctrl_h[2] + (special > 0 ? 1u : 0u));
+  if (n == 0) return PPX_OK;
+  t->used_bound = 0;
+  int rc = ppx::reserve(t, (int64_t)n, st);                   // grows until n keys fit at <= 50 % load
+  if (rc) return rc;
+  uint32_t* bad;
+  PPX_CUDA(cudaMalloc((void**)&bad, sizeof(uint32_t)));
+  rc = cudaMemsetAsync(bad, 0, sizeof(uint32_t), st) == cudaSuccess ? PPX_OK : ppx::fail(PPX_ERR_CUDA, "count_table_load memset");
+  if (!rc) {
+    ppx::load_kernel<<<(unsigned)ppx::ceil_div(n, 256), 256, 0, st>>>(keys_dev, counts_dev, n, t->keys, t->counts, t->capacity,
+                                                                    t->ctrl, bad);
+    rc = ppx::after_launch("count_table_load");
+  }
+  uint32_t bad_h = 0;
+  if (!rc && (cudaMemcpyAsync(&bad_h, bad, sizeof(bad_h), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+              cudaMemcpyAsync(ctrl_h, t->ctrl, sizeof(ctrl_h), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+              cudaStreamSynchronize(st) != cudaSuccess))
+    rc = ppx::fail(PPX_ERR_CUDA, "count_table_load readback");
+  cudaFree(bad);
+  if (rc) return rc;
+  if (bad_h || ctrl_h[3]) {                                   // no half-loaded table: back to empty, then report
+    rc = ppx::clear_arrays(t, st);
+    if (rc) return rc;
+    PPX_CUDA(cudaStreamSynchronize(st));
+    if (bad_h & 1u) return ppx::fail(PPX_ERR_ARG, "count_table_load: duplicate key");
+    if (bad_h & 2u) return ppx::fail(PPX_ERR_ARG, "count_table_load: zero count");
+    return ppx::fail(PPX_ERR_CAPACITY, "count_table_load: table overflowed");
+  }
+  t->used_bound = ctrl_h[2];                                  // exact: later growth checks see the keys in use
+  return PPX_OK;
 }

@@ -38,6 +38,8 @@ class VecNormalize(object):
         for name in ("episode_stats", "behavior"):              # raw episode statistics / states pass through
             if callable(getattr(venv, name, None)):
                 setattr(self, name, getattr(venv, name))
+        if callable(getattr(venv, "state_dict", None)):        # the state protocol only if the wrapped env has it
+            self.state_dict, self.load_state_dict = self._state_dict, self._load_state_dict
 
     # ---- helpers ----
     def _up(self, x, dtype):
@@ -61,6 +63,26 @@ class VecNormalize(object):
 
     def get_original_obs(self):
         return self.old_obs
+
+    # ---- checkpoint state (INTEGRATION.md §4): the statistics, the discounted returns, the flags and the inner env ----
+    _FLAGS = ("training", "norm_obs", "norm_reward", "clip_obs", "clip_reward", "gamma", "epsilon", "_cuda_inner")
+
+    def _state_dict(self):
+        from .checkpoint import pack
+        sd = {k.lstrip("_"): getattr(self, k) for k in self._FLAGS}
+        sd.update(obs_rms=self.obs_rms.state_dict(), ret_rms=self.ret_rms.state_dict(), ret=self.ret.cpu(),
+                  old_obs=pack(self.old_obs), venv=self.venv.state_dict())
+        return sd
+
+    def _load_state_dict(self, sd):
+        from .checkpoint import tensor_into, unpack
+        for k in self._FLAGS:
+            setattr(self, k, type(getattr(self, k))(sd[k.lstrip("_")]))
+        self.obs_rms.load_state_dict(sd["obs_rms"])
+        self.ret_rms.load_state_dict(sd["ret_rms"])
+        tensor_into(self.ret, sd["ret"], "VecNormalize 'ret'")
+        self.old_obs = unpack(sd["old_obs"], self.device)
+        self.venv.load_state_dict(sd["venv"])
 
     # ---- VecEnv surface ----
     def reset(self):

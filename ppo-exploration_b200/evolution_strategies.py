@@ -56,6 +56,42 @@ class EvolutionStrategy(object):
         self._graphs = {}
         self.update_mode = "single"
 
+    # ---- checkpoints (DESIGN.md §3.14) ----
+    def save(self, path):
+        """Write theta, the device learning rate, the device draw counter, novelty_param and the constructor configuration
+        to `path` (one `torch.save` file, loadable with `weights_only=True`).  The noise table is not stored: `load`
+        regenerates it from its seed.  Under torch.distributed every rank saves its own file: pass a per-rank path."""
+        from .checkpoint import header
+        ck = header(type(self).__name__)
+        ck.update(
+            config=dict(env_id=self.env_id, hidden_sizes=list(self.hidden_sizes), nsr_plateu=self.nsr_plateu,
+                        nsr_range=list(self.nsr_range), nsr_update=self.nsr_update, population_size=int(self.POPULATION_SIZE),
+                        sigma=float(self.SIGMA), decay=self.decay, obs_dim=int(self.shapes[0][0]),
+                        n_actions=int(self.shapes[-1][1]), noise_table_size=self._noise_size, noise_seed=self._noise_seed,
+                        fitness_shaping=self.fitness_shaping),
+            K=int(self.K), theta=self.theta.cpu(), lr=self._lr.cpu(), draw=self._draw.cpu(),
+            novelty_param=float(self.novelty_param), world_size=D.world_size(), rank=D.rank())
+        torch.save(ck, path)
+
+    @classmethod
+    def load(cls, path, device="cuda"):
+        """The strategy saved at `path` by `save()`: the next ask() / evaluate() / tell() / run_generation() compute what the
+        saved object would have.  numpy's global RNG is left as it was (the constructor's draw of initial weights is
+        undone).  Captured graphs are captured anew.  ValueError for another format version or world size / rank."""
+        from .checkpoint import read, tensor_into
+        ck = read(path, cls.__name__)
+        W, r = D.world_size(), D.rank()
+        if (ck["world_size"], ck["rank"]) != (W, r):
+            raise ValueError(f"the checkpoint was saved by rank {ck['rank']} of {ck['world_size']}, this is rank {r} of {W}")
+        rng = np.random.get_state()
+        es = cls(device=device, **ck["config"])
+        np.random.set_state(rng)
+        es.K, es.novelty_param = ck["K"], ck["novelty_param"]
+        tensor_into(es.theta, ck["theta"], "ES theta")
+        tensor_into(es._lr, ck["lr"], "ES learning rate")
+        tensor_into(es._draw, ck["draw"], "ES draw counter")
+        return es
+
     # ---- state views ----
     @property
     def learning_rate(self):

@@ -67,6 +67,20 @@ class ParamBank:
         for t in self.tc_weights:
             t.refresh()
 
+    _STATE = ("flat", "grad", "exp_avg", "exp_avg_sq", "step_dev")
+
+    def state_dict(self):
+        """Parameters, gradients, Adam moments and the device step counter as CPU tensors (checkpoints)."""
+        return {k: getattr(self, k).cpu() for k in self._STATE}
+
+    def load_state_dict(self, sd):
+        """Restore `state_dict()` in place (addresses, and so captured graphs, stay valid) and refresh the tensor-core
+        weight shadows."""
+        from .checkpoint import tensor_into
+        for k in self._STATE:
+            tensor_into(getattr(self, k), sd[k], f"parameter bank '{k}'")
+        self.refresh_tc()
+
     def view(self, name, grad=False):
         o, s = self.offsets[name], self.shapes[name]
         return (self.grad if grad else self.flat)[o:o + int(np.prod(s))].view(s)

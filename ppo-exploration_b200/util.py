@@ -43,6 +43,15 @@ class RunningMeanStd(object):
         L.call("ppx_obs_istd", self.var_dev.data_ptr(), self.dim, self._istd.data_ptr(), L.stream())
         return self._istd
 
+    def state_dict(self):
+        """The f64 moments as CPU tensors (checkpoints)."""
+        return {"mean": self.mean_dev.cpu(), "var": self.var_dev.cpu(), "count": self.count_dev.cpu()}
+
+    def load_state_dict(self, sd):
+        from .checkpoint import tensor_into
+        for k in ("mean", "var", "count"):
+            tensor_into(getattr(self, k + "_dev"), sd[k], f"running statistics '{k}'")
+
     def set_state(self, mean, var, count):
         self.mean_dev.copy_(torch.as_tensor(np.asarray(mean, dtype=np.float64)).reshape(-1))
         self.var_dev.copy_(torch.as_tensor(np.asarray(var, dtype=np.float64)).reshape(-1))

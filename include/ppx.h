@@ -559,6 +559,13 @@ int ppx_es_forward(const double* theta, const float* noise, const int64_t* offse
 int ppx_es_act(const double* theta, const float* noise, const int64_t* offsets, double sigma, int N, const int* layer_sizes_host,
                int n_layers, const float* obs, const uint8_t* alive, int discrete, uint64_t seed, const int64_t* draw_dev,
                int64_t step, int64_t member_lo, const double* uniforms, void* actions, void* stream);
+/* ppx_es_act_rows: the brains of EvolutionStrategy.run, env row m acting with its own parameter vector thetas[m] (f64 [M, D],
+ * row-major) at sigma = 0 -- for every row the logits and action of ppx_es_act(theta = thetas[m], sigma = 0, table offset 0)
+ * bit for bit, Discrete u from Philox4x32-10 keyed by `seed` at counter (m, step, *draw_dev).  noise: the table (row m reads
+ * its first D floats, multiplied by 0); obs f32 [M, D0]; alive and actions as in ppx_es_act.  One launch, one CTA per row. */
+int ppx_es_act_rows(const double* thetas, const float* noise, int M, const int* layer_sizes_host, int n_layers, const float* obs,
+                    const uint8_t* alive, int discrete, uint64_t seed, const int64_t* draw_dev, int64_t step, void* actions,
+                    void* stream);
 /* ppx_es_episode_step, after env.step, for every member with alive[n] != 0: fitness[n] += reward (f32 or f64 rewards [N],
  * f64 sum), lengths[n] += 1; when dones[n] != 0 or last_step != 0 the behaviour row behavior[n, 0..k) (NULL: none) is copied
  * to behavior_out[n] and alive[n] = 0.  state: int64 [3], zero before the first step; state[2] receives the number of

@@ -147,6 +147,7 @@ SIGNATURES = {
     "ppx_es_perturb": (c_i, [c_p, c_p, c_p, c_d, c_i, c_i, c_p, c_i, c_p]),
     "ppx_es_forward": (c_i, [c_p, c_p, c_p, c_d, c_i, c_p, c_i, c_p, c_i, c_p, c_p]),
     "ppx_es_act": (c_i, [c_p, c_p, c_p, c_d, c_i, c_p, c_i, c_p, c_p, c_i, c_u, c_p, c_l, c_l, c_p, c_p, c_p]),
+    "ppx_es_act_rows": (c_i, [c_p, c_p, c_i, c_p, c_i, c_p, c_p, c_i, c_u, c_p, c_l, c_p, c_p]),
     "ppx_es_episode_step": (c_i, [c_p, c_i, c_p, c_p, c_i, c_l, c_i, c_p, c_p, c_p, c_p, c_p, c_p]),
     "ppx_es_update_workspace": (c_l, [c_i, c_i]),
     "ppx_es_update": (c_i, [c_p, c_p, c_p, c_p, c_i, c_i, c_d, c_d, c_d, c_p, c_i, c_i, c_d, c_p, c_p, c_p, c_p]),

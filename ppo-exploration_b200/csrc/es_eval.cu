@@ -5,6 +5,8 @@
 //                        the fly (es_walk.cuh, the walk of ppx_es_forward: bit-identical logits), actions written into the
 //                        env-facing buffer -- Box tanh(logits) f64, Discrete one categorical draw int64 with numpy's
 //                        RandomState.choice arithmetic.  A finished member reads no noise and gets action 0.
+//   ppx_es_act_rows      the brains of EvolutionStrategy.run: env row m acts with its own parameter vector thetas[m] at
+//                        sigma = 0, through the same walk (bit-identical to ppx_es_act with theta = thetas[m]).
 //   ppx_es_episode_step  after env.step: fitness += reward (f64) and length += 1 while the member runs, its behaviour row
 //                        latched at its terminating step, alive &= !done, and a device count of the members still running.
 #include "common.cuh"
@@ -115,6 +117,45 @@ __global__ void __launch_bounds__(256) es_act_kernel(EsActP p) {
   }
 }
 
+// The brains of EvolutionStrategy.run (§3.15): CTA m stages thetas[m] and its warp 0 runs env row m with it at sigma = 0 --
+// the member walk of es_act_kernel on table offset 0 (fmaf(0, eps, t) = t), so a row's logits and action are bit for bit
+// those of es_act_kernel for theta = thetas[m], sigma = 0 and the same Philox key.  M is a handful of rows: one CTA each.
+__global__ void __launch_bounds__(128) es_act_rows_kernel(EsActP p) {
+  extern __shared__ float sm_f[];
+  const int m = blockIdx.x;
+  const int A = p.sizes[p.n_layers];
+  if (p.alive && !p.alive[m]) {
+    if (p.discrete) {
+      if (threadIdx.x == 0) static_cast<int64_t*>(p.actions)[m] = 0;
+    } else {
+      for (int j = threadIdx.x; j < A; j += blockDim.x) static_cast<double*>(p.actions)[(size_t)m * A + j] = 0.0;
+    }
+    return;
+  }
+  float* th = sm_f;                                         // [D]
+  float* a0 = th + ((p.D + 3) & ~3);                        // [3][kFwdMaxWidth]: two activation buffers + the logits
+  float* a1 = a0 + kFwdMaxWidth;
+  float* lg = a1 + kFwdMaxWidth;
+  const double* theta = p.theta + (size_t)m * p.D;
+  for (int i = threadIdx.x; i < p.D; i += blockDim.x) th[i] = (float)__ldg(theta + i);
+  __syncthreads();
+  if (threadIdx.x >= 32) return;
+  const int lane = threadIdx.x;
+  for (int i = lane; i < p.sizes[0]; i += 32) a0[i] = __ldg(p.obs + (size_t)m * p.sizes[0] + i);
+  __syncwarp();
+  es_member_walk(p, p.noise, th, a0, a1, lane, [&](int j, int no, float v) {
+    if (p.discrete) lg[j] = v;
+    else static_cast<double*>(p.actions)[(size_t)m * no + j] = (double)tanhf(v);
+  });
+  if (p.discrete && lane == 0) {
+    const uint64_t gen = p.draw ? (uint64_t)*p.draw : 0;
+    uint32_t c[4] = {(uint32_t)m, (uint32_t)p.step, (uint32_t)gen, (uint32_t)(gen >> 32)};
+    philox4x32(c, p.seed);
+    const double u = ((double)(c[0] >> 5) * 67108864.0 + (double)(c[1] >> 6)) * (1.0 / 9007199254740992.0);
+    static_cast<int64_t*>(p.actions)[m] = np_choice(lg, A, u);
+  }
+}
+
 // state[0]: running sum of the blocks' counts, state[1]: ticket word of the last-block detection, state[2]: members still
 // running after this step (written by the last block, which re-arms state[0] and the ticket)
 __global__ void __launch_bounds__(256)
@@ -175,6 +216,28 @@ extern "C" int ppx_es_act(const double* theta, const float* noise, const int64_t
   const unsigned grid = (unsigned)ceil_div(N, 8 * k);
   es_act_kernel<<<grid, 256, smem, (cudaStream_t)stream>>>(p);
   return after_launch("es_act");
+}
+
+extern "C" int ppx_es_act_rows(const double* thetas, const float* noise, int M, const int* layer_sizes, int n_layers, const float* obs,
+                               const uint8_t* alive, int discrete, uint64_t seed, const int64_t* draw_dev, int64_t step, void* actions,
+                               void* stream) {
+  PPX_REQUIRE(thetas && noise && layer_sizes && obs && actions && M >= 1 && step >= 0, "es_act_rows: bad arguments");
+  EsActP p{};
+  p.theta = thetas; p.noise = noise; p.sigma = 0.f; p.P = M;
+  p.obs = obs; p.alive = alive; p.actions = actions; p.discrete = discrete;
+  p.seed = seed; p.draw = draw_dev; p.step = step;
+  static const int64_t table_offset = 0;                    // every row reads the table at offset 0: the layer plan of a table member
+  int rc = es_plan(p, noise, &table_offset, layer_sizes, n_layers, "es_act_rows");
+  if (rc) return rc;
+  const size_t smem = sizeof(float) * ((size_t)((p.D + 3) & ~3) + 3 * kFwdMaxWidth);
+  PPX_REQUIRE(smem <= 227 * 1024, "es_act_rows: %d parameters do not fit in shared memory", p.D);
+  static size_t configured = 0;
+  if (smem > configured) {
+    PPX_CUDA(cudaFuncSetAttribute(es_act_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    configured = smem;
+  }
+  es_act_rows_kernel<<<M, 128, smem, (cudaStream_t)stream>>>(p);
+  return after_launch("es_act_rows");
 }
 
 extern "C" int ppx_es_episode_step(const void* rewards, int rewards_f64, const uint8_t* dones, const double* behavior, int k, int64_t N,

@@ -6,7 +6,8 @@ path: _get_population (:172-182), _get_weights_try (:137-145), _update_weights (
 of episode evaluation (FeedForwardNetwork.predict :48-61) batched over the population
 (`predict_population`, SURVEY §8f.4).  For a batched env that lives on the GPU, `evaluate` runs the episode loop of
 evaluate / get_behavior_char (:153-170) on the device -- fitness, episode lengths and behaviour characterisations -- and
-`run_generation` chains ask -> evaluate -> tell.  For an env on the host, the caller steps it with `predict_population` /
+`run_generation` chains ask -> evaluate -> tell, and `run` is the reference's ES-NSRA loop (:293-384) over a meta-population
+of brains with a device behaviour archive (DESIGN.md §3.15).  For an env on the host, the caller steps it with `predict_population` /
 `discrete_action` and feeds the fitness vector back through `_update_weights` or `tell`.
 
 Build-side design (SURVEY §0.1): the population is a vector of offsets into ONE resident f32 noise
@@ -55,12 +56,16 @@ class EvolutionStrategy(object):
         self._px = False                                                          # PeerExchange for the sharded update | None
         self._graphs = {}
         self.update_mode = "single"
+        self.thetas = None                                                        # the meta-population of run() [M, D] f64
 
     # ---- checkpoints (DESIGN.md §3.14) ----
     def save(self, path):
         """Write theta, the device learning rate, the device draw counter, novelty_param and the constructor configuration
         to `path` (one `torch.save` file, loadable with `weights_only=True`).  The noise table is not stored: `load`
-        regenerates it from its seed.  Under torch.distributed every rank saves its own file: pass a per-rank path."""
+        regenerates it from its seed.  After run(), also the run's state at the generation boundary: `thetas`, the
+        behaviour archive, the brains' last BCs and returns, the f_b window and best, the generation counter, numpy's global
+        RNG state (the brain picks draw from it) and the `state_dict()` of env and brain_env where they have one.  Under
+        torch.distributed every rank saves its own file: pass a per-rank path."""
         from .checkpoint import header
         ck = header(type(self).__name__)
         ck.update(
@@ -71,13 +76,23 @@ class EvolutionStrategy(object):
                         fitness_shaping=self.fitness_shaping),
             K=int(self.K), theta=self.theta.cpu(), lr=self._lr.cpu(), draw=self._draw.cpu(),
             novelty_param=float(self.novelty_param), world_size=D.world_size(), rank=D.rank())
+        if self.thetas is not None:
+            from .checkpoint import np_rng_state
+            env, brain_env = getattr(self, "_run_envs", (None, None))
+            state = {name: e.state_dict() for name, e in (("env", env), ("brain_env", brain_env))
+                     if e is not None and callable(getattr(e, "state_dict", None))}
+            ck["run"] = dict(thetas=self.thetas.cpu(), archive=self.archive.cpu(), bc=self._bc_m.cpu(), f=self._f_m.cpu(),
+                             fb_window=list(self._fb_window), best=float(self._best), generation=int(self._generation),
+                             numpy_rng=np_rng_state(), envs=state)
         torch.save(ck, path)
 
     @classmethod
-    def load(cls, path, device="cuda"):
+    def load(cls, path, device="cuda", env=None, brain_env=None):
         """The strategy saved at `path` by `save()`: the next ask() / evaluate() / tell() / run_generation() compute what the
         saved object would have.  numpy's global RNG is left as it was (the constructor's draw of initial weights is
-        undone).  Captured graphs are captured anew.  ValueError for another format version or world size / rank."""
+        undone) -- unless the file holds a run: then the run's state is restored, numpy's global RNG is set to its state at
+        save(), `env` / `brain_env` (fresh ones, as passed to run()) load their saved `state_dict()`, and the next run()
+        continues the run.  Captured graphs are captured anew.  ValueError for another format version or world size / rank."""
         from .checkpoint import read, tensor_into
         ck = read(path, cls.__name__)
         W, r = D.world_size(), D.rank()
@@ -90,6 +105,22 @@ class EvolutionStrategy(object):
         tensor_into(es.theta, ck["theta"], "ES theta")
         tensor_into(es._lr, ck["lr"], "ES learning rate")
         tensor_into(es._draw, ck["draw"], "ES draw counter")
+        run = ck.get("run")
+        if run is not None:
+            from .checkpoint import np_rng_tuple
+            M, k = run["bc"].shape
+            n = run["archive"].shape[0]
+            es.thetas = run["thetas"].to(es.device)
+            es._run_buffers(M, k, capacity=max(16, 1 << n.bit_length()))
+            es._archive[:n].copy_(run["archive"])
+            es._archive_n = n
+            es._bc_m.copy_(run["bc"])
+            es._f_m.copy_(run["f"])
+            es._fb_window, es._best, es._generation = list(run["fb_window"]), run["best"], run["generation"]
+            for name, e in (("env", env), ("brain_env", brain_env)):
+                if e is not None and name in run["envs"]:
+                    e.load_state_dict(run["envs"][name])
+            np.random.set_state(np_rng_tuple(run["numpy_rng"]))
         return es
 
     # ---- state views ----
@@ -267,6 +298,11 @@ class EvolutionStrategy(object):
         return self._px
 
     # ---- ask / tell: the two device-side halves of one ES iteration, each replayed as ONE CUDA graph ----
+    def _hp_state(self):
+        """Every host scalar the ask / tell graphs bake into kernel arguments: a graph is keyed on these, so a run that
+        adapts novelty_param (or a caller that changes sigma / decay / K) replays a graph captured with the current values."""
+        return (float(self.novelty_param), float(self.SIGMA), float(self.decay), int(self.K), self.fitness_shaping)
+
     def _graph(self, key, fn):
         ent = self._graphs.get(key)
         if ent is None:
@@ -295,7 +331,7 @@ class EvolutionStrategy(object):
             self._ask_off = torch.empty(self.POPULATION_SIZE, dtype=torch.int64, device=self.device)
             self._side = torch.cuda.Stream(device=self.device)
         key = ("ask", archive.data_ptr() if archive is not None else 0, queries.data_ptr() if queries is not None else 0,
-               archive.shape[0] if archive is not None else 0)
+               archive.shape[0] if archive is not None else 0, self._hp_state())
 
         def fn():
             nov = None
@@ -317,7 +353,8 @@ class EvolutionStrategy(object):
         """Second half (:217-239): exchange the fitness of the rank-local members and update the parameters with the
         novelty of meta-population member `brain` computed by the last ask().  `local_rewards` must be a persistent CUDA
         tensor (its address is captured)."""
-        key = ("tell", local_rewards.data_ptr(), int(brain), self._novelty is not None)
+        key = ("tell", local_rewards.data_ptr(), int(brain), self._novelty.data_ptr() if self._novelty is not None else 0,
+               self._hp_state())
 
         def fn():
             r_all = self.gather_fitness(local_rewards)
@@ -364,40 +401,55 @@ class EvolutionStrategy(object):
         P = off.numel() if off is not None else noise.shape[0]
         if P != N:
             raise ValueError(f"the env runs {N} envs but the population has {P} members (one env per member)")
+        discrete, A = self._env_actions(env)
+        if uniforms is not None:
+            L.require_cuda(uniforms, torch.float64, "uniforms")
+            if tuple(uniforms.shape) != (max_steps, N):
+                raise ValueError(f"uniforms must be [{max_steps}, {N}], got {tuple(uniforms.shape)}")
+        sizes = [self.shapes[0][0]] + [sh[1] for sh in self.shapes]
+        import ctypes as C
+        sizes_c = (C.c_int * len(sizes))(*sizes)
+
+        def act(t, o, buf):
+            L.call("ppx_es_act", self.theta.data_ptr(), noise.data_ptr(), off.data_ptr() if off is not None else None, sig, N,
+                   sizes_c, len(sizes) - 1, o.data_ptr(), buf["alive"].data_ptr(), int(discrete), self._noise_seed + 2,
+                   self._draw.data_ptr(), t, int(member_lo or 0), uniforms[t].data_ptr() if uniforms is not None else None,
+                   buf["actions"].data_ptr(), L.stream())
+        return self._episodes(env, "population", A, discrete, max_steps, check_every, act)
+
+    def _env_actions(self, env):
+        """(discrete, number of actions) of env.action_space; ValueError if the network has another number of actions."""
         space = env.action_space
         discrete = getattr(space, "n", None) is not None and not getattr(space, "shape", ())
         A = int(space.n) if discrete else int(space.shape[-1])
         if A != self.shapes[-1][1]:
             raise ValueError(f"the env has {A} actions, the network {self.shapes[-1][1]}")
-        if uniforms is not None:
-            L.require_cuda(uniforms, torch.float64, "uniforms")
-            if tuple(uniforms.shape) != (max_steps, N):
-                raise ValueError(f"uniforms must be [{max_steps}, {N}], got {tuple(uniforms.shape)}")
+        return discrete, A
+
+    def _episodes(self, env, tag, A, discrete, max_steps, check_every, act):
+        """The device episode loop of evaluate() and of run()'s brains: one episode per env, `act(t, obs f32 [N, D0], buffers)`
+        launching the forward that writes buffers["actions"], then env.step and `ppx_es_episode_step`.  `tag` keeps the
+        buffers of the two loops apart."""
+        N = int(env.num_envs)
         obs = env.reset()
         if not (isinstance(obs, torch.Tensor) and obs.is_cuda):
             raise TypeError("evaluate() steps environments that live on the GPU: env.reset() must return a CUDA tensor "
                             f"(got {type(obs).__name__}); for an env returning numpy, loop over predict_population / "
                             "discrete_action on the host")
-        buf = self._eval_buffers(N, A, discrete)
+        buf = self._eval_buffers(tag, N, A, discrete)
         buf["fitness"].zero_()
         buf["lengths"].zero_()
         buf["alive"].fill_(1)
         buf["state"].zero_()
         has_bc = callable(getattr(env, "behavior", None))
         bc_out = None
-        sizes = [self.shapes[0][0]] + [sh[1] for sh in self.shapes]
-        import ctypes as C
-        sizes_c = (C.c_int * len(sizes))(*sizes)
         st = L.stream()
-        acts = buf["actions"]
+        d0 = self.shapes[0][0]
         t = 0
         while t < max_steps:
-            o = self._device_input(obs, torch.float32, (N, sizes[0]), "observations")
-            L.call("ppx_es_act", self.theta.data_ptr(), noise.data_ptr(), off.data_ptr() if off is not None else None, sig, N,
-                   sizes_c, len(sizes) - 1, o.data_ptr(), buf["alive"].data_ptr(), int(discrete), self._noise_seed + 2,
-                   self._draw.data_ptr(), t, int(member_lo or 0), uniforms[t].data_ptr() if uniforms is not None else None,
-                   acts.data_ptr(), st)
-            obs, rew, done, _ = env.step(acts)
+            o = self._device_input(obs, torch.float32, (N, d0), "observations")
+            act(t, o, buf)
+            obs, rew, done, _ = env.step(buf["actions"])
             rew = self._device_input(rew, None, (N,), "rewards")
             done = self._device_input(done, torch.uint8, (N,), "dones")
             bc = None
@@ -407,7 +459,7 @@ class EvolutionStrategy(object):
                     raise TypeError("env.behavior() must return a CUDA tensor [N, k]")
                 bc = bc.reshape(N, -1).to(torch.float64).contiguous()
                 if bc_out is None:
-                    bc_out = self._eval_bc(N, bc.shape[1])
+                    bc_out = self._eval_bc(tag, N, bc.shape[1])
             L.call("ppx_es_episode_step", rew.data_ptr(), int(rew.dtype == torch.float64), done.data_ptr(),
                    bc.data_ptr() if bc is not None else None, bc.shape[1] if bc is not None else 0, N, int(t == max_steps - 1),
                    buf["alive"].data_ptr(), buf["fitness"].data_ptr(), buf["lengths"].data_ptr(),
@@ -423,10 +475,10 @@ class EvolutionStrategy(object):
         self.last_eval_steps = t
         return buf["fitness"], buf["lengths"], bc_out
 
-    def _eval_buffers(self, N, A, discrete):
+    def _eval_buffers(self, tag, N, A, discrete):
         if not hasattr(self, "_eval"):
             self._eval = {}
-        key = (N, A, discrete)
+        key = (tag, N, A, discrete)
         if key not in self._eval:
             dev = self.device
             self._eval[key] = dict(
@@ -437,8 +489,8 @@ class EvolutionStrategy(object):
                 host=torch.zeros(1, dtype=torch.int64).pin_memory(), event=torch.cuda.Event(), polled=False)
         return self._eval[key]
 
-    def _eval_bc(self, N, k):
-        key = ("bc", N, k)
+    def _eval_bc(self, tag, N, k):
+        key = ("bc", tag, N, k)
         if key not in self._eval:
             self._eval[key] = torch.zeros(N, k, dtype=torch.float64, device=self.device)
         return self._eval[key]
@@ -466,6 +518,192 @@ class EvolutionStrategy(object):
         out = self.evaluate(env, max_steps=max_steps, check_every=check_every)
         self.tell(out[0], brain=brain)
         return out
+
+    # ---- the ES-NSRA run loop (evolution_strategies.py:293-384, order of SURVEY §3.4; DESIGN.md §3.15) ----
+    def run(self, env, brain_env, iterations, *, max_steps, meta_population_size=2, reward_target=None, log_interval=1,
+            log_to_file=False, check_every=8):
+        """Train a meta-population of M = meta_population_size parameter vectors (`thetas`, f64 [M, D]) with ES-NSRA for up
+        to `iterations` generations.  `env` runs the population (P envs, P/W per rank when sharded), `brain_env` M envs, one
+        episode per brain at sigma = 0 (identical on every rank: same seed, env_offset=0); both live on the GPU
+        (INTEGRATION.md §4) and brain_env has behavior().  The first run() keeps the constructor's theta as brain 0 and
+        draws brains 1..M-1 from numpy's global RNG as the constructor draws theta, runs the brains once and seeds the
+        behaviour archive with all M characterisations (BCs).  Each generation then
+          1. computes every brain's novelty against the archive (one ppx_knn_novelty launch) and reads it to the host with
+             the previous generation's log row -- the generation's one blocking device->host read;
+          2. picks brain b with pick_brain (numpy's global RNG), copies thetas[b] into theta and runs ask() -> evaluate(env)
+             -> tell() with novelty nu_b and the current novelty_param, then copies theta back into thetas[b];
+          3. runs the brains on brain_env (one ppx_es_act_rows + one ppx_es_episode_step launch per step), appends BC_b to the
+             archive, and -- once f_b, brain b's episode return, is on the host -- adapts novelty_param every 5 generations,
+             logs the row and stops when f_b > reward_target.
+        The adaptation is ppx's rule (the reference stores nsr_plateu / nsr_range / nsr_update; its use of them is not
+        pinned, oracle/es_nsra.py `nsr_adapt`): with R the best f_b of the last 5 generations and B the best before them,
+        novelty_param -= nsr_update (at least nsr_range[0]) if R > B + nsr_plateu, else += nsr_update (at most
+        nsr_range[1]); then B = max(B, R).  A later run() (or one after `load`) continues the run.  Logged through
+        `ppo_exploration_b200.logger` as ("ES", env_id): iteration, total_time, reward (f_b), brain, novelty_param (the
+        weight of the generation's update), learning_rate, fitness_mean, fitness_max, archive_size.  Returns self."""
+        import time
+        from . import logger as ppx_logger
+        M, W = int(meta_population_size), D.world_size()
+        if M < 1 or iterations < 0 or max_steps < 1 or check_every < 1 or log_interval < 1:
+            raise ValueError("run() needs meta_population_size, max_steps, check_every, log_interval >= 1, iterations >= 0")
+        if int(env.num_envs) * W != self.POPULATION_SIZE:
+            raise ValueError(f"env runs {int(env.num_envs)} envs per rank; the population of {self.POPULATION_SIZE} needs "
+                             f"{self.POPULATION_SIZE // W} on each of {W} rank(s)")
+        if int(brain_env.num_envs) != M:
+            raise ValueError(f"brain_env runs {int(brain_env.num_envs)} envs, the meta-population has {M} brains")
+        if not callable(getattr(brain_env, "behavior", None)):
+            raise TypeError("run() characterises the brains by brain_env.behavior() (CUDA f64 [M, k])")
+        if W > 1 and getattr(brain_env, "env_offset", 0) != 0:
+            raise ValueError("every rank must step the same brain_env: build it with env_offset=0")
+        if self.thetas is not None and self.thetas.shape[0] != M:
+            raise ValueError(f"this run has {self.thetas.shape[0]} brains, not meta_population_size={M}")
+        self._env_actions(env)
+        self._env_actions(brain_env)
+        ppx_logger.configure("ES", str(self.env_id), log_to_file)
+        self._run_envs = (env, brain_env)
+        if W > 1:
+            self._check_rng_replicas()
+        if self.thetas is None:
+            self._start_run(brain_env, M, max_steps, check_every)
+        start = time.time()
+        pending = None                                          # (brain, novelty weight) of the generation whose row is on the device
+        for _ in range(iterations):
+            self._knn_into(self._run_dev[:M])
+            vals = self._run_read()
+            if pending is not None and self._finish_generation(pending, vals, M, start, log_interval, reward_target):
+                pending = None
+                break
+            b, _ = self.pick_brain([float(v) for v in vals[:M]])
+            w = float(self.novelty_param)
+            self.theta.copy_(self.thetas[b])
+            self.ask()
+            nu_b = self._run_dev[M + 4:M + 5]                   # tell() mixes in nu_b from a fixed slot: one graph for every brain
+            nu_b.copy_(self._run_dev[b:b + 1])
+            self._novelty = nu_b
+            fit = self.evaluate(env, max_steps=max_steps, check_every=check_every)[0]
+            self.tell(fit)
+            self.thetas[b].copy_(self.theta)
+            bc, f = self._brains(brain_env, max_steps, check_every)
+            self._bc_m.copy_(bc)
+            self._f_m.copy_(f)
+            self._archive_append(bc[b])
+            fit_all = self.gather_fitness(fit)
+            row = self._run_dev
+            row[M].copy_(f[b])
+            row[M + 1].copy_(fit_all.mean())
+            row[M + 2].copy_(fit_all.max())
+            row[M + 3].copy_(self._lr[0])
+            self._generation += 1
+            pending = (b, w)
+        if pending is not None:
+            self._finish_generation(pending, self._run_read(), M, start, log_interval, reward_target)
+        return self
+
+    def _start_run(self, brain_env, M, max_steps, check_every):
+        """Brain 0 = theta, brains 1..M-1 drawn layer by layer from numpy's global RNG (the constructor's order), one brain
+        loop, the archive seeded with every brain's BC."""
+        rest = [np.concatenate([np.random.randn(*s).ravel() for s in self.shapes]) for _ in range(M - 1)]
+        self.thetas = torch.empty(M, self.D, dtype=torch.float64, device=self.device)
+        self.thetas[0].copy_(self.theta)
+        if rest:
+            self.thetas[1:].copy_(torch.as_tensor(np.stack(rest)))
+        bc, f = self._brains(brain_env, max_steps, check_every)
+        self._run_buffers(M, bc.shape[1])
+        self._bc_m.copy_(bc)
+        self._f_m.copy_(f)
+        for m in range(M):
+            self._archive_append(bc[m])
+        self._fb_window, self._best, self._generation = [], -float("inf"), 0
+
+    def _run_buffers(self, M, k, capacity=16):
+        self._archive = torch.empty(capacity, k, dtype=torch.float64, device=self.device)
+        self._archive_n = 0
+        self._bc_m = torch.empty(M, k, dtype=torch.float64, device=self.device)
+        self._f_m = torch.empty(M, dtype=torch.float64, device=self.device)
+        self._knn_sums = torch.empty(M, dtype=torch.float64, device=self.device)
+        # [nu_0 .. nu_M-1, f_b, fitness mean, fitness max, lr | nu_b]: the first M + 4 are the generation's read
+        self._run_dev = torch.zeros(M + 5, dtype=torch.float64, device=self.device)
+        self._run_host = torch.zeros(M + 4, dtype=torch.float64).pin_memory()
+        self._run_event = torch.cuda.Event()
+
+    def _archive_append(self, row):
+        """One BC row onto the device archive; the host keeps the count, and the capacity doubles when it is full."""
+        n = self._archive_n
+        if n == self._archive.shape[0]:
+            grown = torch.empty(2 * n, self._archive.shape[1], dtype=torch.float64, device=self.device)
+            grown[:n].copy_(self._archive)
+            self._archive = grown
+        self._archive[n].copy_(row)
+        self._archive_n = n + 1
+
+    @property
+    def archive(self):
+        """The behaviour archive of run(): f64 CUDA [n, k] (a view), or None before the first run()."""
+        return None if self.thetas is None else self._archive[:self._archive_n]
+
+    def _knn_into(self, nov):
+        """nov [M] = the novelty of every brain's last BC against the archive (one launch)."""
+        L.call("ppx_knn_novelty", self._archive.data_ptr(), self._archive_n, self._bc_m.data_ptr(), self._bc_m.shape[0],
+               self._bc_m.shape[1], int(self.K), self._knn_sums.data_ptr(), nov.data_ptr(), L.stream())
+
+    def _run_read(self):
+        """The generation's one blocking read: the device row [novelties, previous f_b, fitness mean / max, lr] into pinned
+        memory, then an event wait."""
+        self._run_host.copy_(self._run_dev[:self._run_host.numel()], non_blocking=True)
+        self._run_event.record()
+        self._run_event.synchronize()
+        return self._run_host.numpy().copy()
+
+    def _finish_generation(self, pending, vals, M, start, log_interval, reward_target):
+        """Host half of the generation whose row `vals` holds: the f_b window, novelty_param, the log row.  True when f_b
+        exceeds reward_target."""
+        import time
+        from . import logger as ppx_logger
+        b, w = pending
+        fb = float(vals[M])
+        self._fb_window.append(fb)
+        if len(self._fb_window) == 5:                           # ppx's adaptation rule (docstring of run())
+            R = max(self._fb_window)
+            if R > self._best + self.nsr_plateu:
+                self.novelty_param = float(max(self.nsr_range[0], self.novelty_param - self.nsr_update))
+            else:
+                self.novelty_param = float(min(self.nsr_range[1], self.novelty_param + self.nsr_update))
+            self._best = max(self._best, R)
+            self._fb_window = []
+        if self._generation % log_interval == 0:
+            for key, v in (("time/iteration", self._generation), ("time/total_time", time.time() - start), ("es/reward", fb),
+                           ("es/brain", b), ("es/novelty_param", w), ("es/learning_rate", float(vals[M + 3])),
+                           ("es/fitness_mean", float(vals[M + 1])), ("es/fitness_max", float(vals[M + 2])),
+                           ("es/archive_size", self._archive_n)):
+                ppx_logger.record(key, v)
+            ppx_logger.dump(step=self._generation)
+        return reward_target is not None and fb > reward_target
+
+    def _brains(self, brain_env, max_steps, check_every):
+        """One episode per brain on brain_env: row m acts with thetas[m] at sigma = 0 (ppx_es_act_rows; Discrete draws on
+        their own Philox key, noise seed + 3).  Returns (BC f64 [M, k], episode return f64 [M])."""
+        import ctypes as C
+        discrete, A = self._env_actions(brain_env)
+        M = self.thetas.shape[0]
+        sizes = [self.shapes[0][0]] + [sh[1] for sh in self.shapes]
+        sizes_c = (C.c_int * len(sizes))(*sizes)
+        noise = self.noise_table()
+
+        def act(t, o, buf):
+            L.call("ppx_es_act_rows", self.thetas.data_ptr(), noise.data_ptr(), M, sizes_c, len(sizes) - 1, o.data_ptr(),
+                   buf["alive"].data_ptr(), int(discrete), self._noise_seed + 3, self._draw.data_ptr(), t,
+                   buf["actions"].data_ptr(), L.stream())
+        fit, _, bc = self._episodes(brain_env, "brains", A, discrete, max_steps, check_every, act)
+        return bc, fit
+
+    def _check_rng_replicas(self):
+        """Sharded run(): every rank must make the same brain picks, so numpy's global RNG must be in the same state on
+        every rank (the learners' "global" convention)."""
+        digest = D.rng_digest(np.random.get_state())
+        seen = D.all_gather_cat(torch.tensor([digest], dtype=torch.int64, device=self.device)).cpu().numpy().ravel()
+        if not (seen == seen[0]).all():
+            raise RuntimeError("ppx: a sharded ES run() needs numpy's global RNG in the same state on every rank (seed all "
+                               "ranks alike and keep rank-dependent draws off np.random); digests: %s" % seen.tolist())
 
     @property
     def update_skipped(self):

@@ -606,6 +606,26 @@ int ppx_rank_center(const double* r, int P, int64_t* rank_out, double* centred_o
 int ppx_knn_novelty(const double* archive, int64_t M, const double* queries, int Q, int dim, int K,
                     double* sum_out, double* novelty_out, void* stream);
 
+/* ppx_knn_novelty for a population of queries: the same sum_out / novelty_out as ppx_knn_novelty, bit for bit, for any
+ * Q >= 1 (no grid limit, no scratch).  One thread per query keeps a top-K of squared distances; only the S = min(K, M)
+ * winners take a square root (monotone under correct rounding, so the selection is the same).  dim 1..8, K 1..32.
+ * One launch. */
+int ppx_knn_novelty_many(const double* archive, int64_t M, const double* queries, int Q, int dim, int K,
+                         double* sum_out, double* novelty_out, void* stream);
+/* NSRA-ES update with a novelty per member (Conti et al. 2018, Alg. 3; not in the reference):
+ * theta += sum_p c_p eps_p, c_p = lr/(P sigma) * ((1-w) F~_p + w N~_p) / 2 with w = novelty_param, F~ = shape(rewards),
+ * N~ = shape(novelties), both over all P members: z-score (ddof 0; a vector whose std is 0 shapes to 0) or, rank_mode = 1,
+ * ppx_rank_center's centred ranks.  z-score skips the update (theta and lr untouched, status_out[0] = 1) only when BOTH stds
+ * are 0; otherwise, and always in rank mode, *lr_inout *= decay.  W == 1: p_lo = 0, p_n = P, peer arguments NULL, theta
+ * updated in place.  W >= 2: the GEMV over this rank's members [p_lo, p_lo + p_n) and the rank-ordered peer-memory apply
+ * of ppx_es_update_sharded.  Workspace: ppx_es_update_member_workspace(P, D) bytes. */
+int64_t ppx_es_update_member_workspace(int P, int D);
+int ppx_es_update_member(double* theta, const float* noise, const int64_t* offsets, const double* rewards, const double* novelties,
+                         int P, int p_lo, int p_n, int D, double sigma, double novelty_param, int rank_mode, double decay,
+                         double* lr_inout, int* status_out, void* workspace, double* dtheta_local,
+                         const void* const* peer_dtheta_host, void* const* peer_flags_host, int W, int rank, uint32_t* seq_dev,
+                         uint32_t* status_dev, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

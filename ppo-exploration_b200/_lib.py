@@ -156,6 +156,10 @@ SIGNATURES = {
                                     c_p, c_i, c_i, c_p, c_p, c_p]),
     "ppx_rank_center": (c_i, [c_p, c_i, c_p, c_p, c_p]),
     "ppx_knn_novelty": (c_i, [c_p, c_l, c_p, c_i, c_i, c_i, c_p, c_p, c_p]),
+    "ppx_knn_novelty_many": (c_i, [c_p, c_l, c_p, c_i, c_i, c_i, c_p, c_p, c_p]),
+    "ppx_es_update_member_workspace": (c_l, [c_i, c_i]),
+    "ppx_es_update_member": (c_i, [c_p, c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_d, c_d, c_i, c_d, c_p, c_p, c_p, c_p, c_p, c_p,
+                                   c_i, c_i, c_p, c_p, c_p]),
 }
 _STATUS = {n for n, (r, _) in SIGNATURES.items() if r is c_i and n not in ("ppx_version", "ppx_tc_supported", "ppx_mlp3_supported", "ppx_mlp3_tc_supported", "ppx_tc_wgrad_supported", "ppx_mlp3_sumsq_partials", "ppx_mlp3_fused_adam_blocks")}
 

@@ -363,6 +363,115 @@ knn_merge_kernel(const double* __restrict__ cand, int n_cand, int64_t M, int K, 
   }
 }
 
+// ---------------- novelty k-NN for a population of queries ----------------
+// ppx_knn_novelty_many: one THREAD per query, so any Q runs in one launch with no scratch.  Archive rows pass through shared
+// memory in tiles of kKnnTile rows; every thread of the CTA reads the same row (a shared-memory broadcast).  Each thread keeps
+// a sorted top-K of SQUARED distances in registers and takes square roots only of its S = min(K, M) winners at the end.
+// Why this equals ppx_knn_novelty bit for bit: d2 is formed by the same sequence of __dsub_rn / __dmul_rn / __dadd_rn, and a
+// correctly rounded square root is monotone (x <= y -> sqrt(x) <= sqrt(y)).  Sorting the d2 ascending and applying
+// __dsqrt_rn keeps the list sorted, so the first S entries are a valid choice of the S smallest distances -- and the multiset
+// of the S smallest values of a list is unique.  Summing them ascending from 0.0 with __dadd_rn is then the very sum
+// knn_merge_kernel pops (equal values in either order add identically).  A row whose d2 is not below the current K-th best
+// cannot change that multiset and is rejected with one compare.
+constexpr int kKnnTile = 256, kKnnManyMaxDim = 8, kKnnManyThreads = 64;
+
+template <int KMAX>
+__global__ void __launch_bounds__(kKnnManyThreads)
+knn_many_kernel(const double* __restrict__ archive, int64_t M, const double* __restrict__ queries, int Q, int dim, int K,
+                double* __restrict__ sum_out, double* __restrict__ nov_out) {
+  __shared__ double tile[kKnnTile * kKnnManyMaxDim];
+  const int q = blockIdx.x * kKnnManyThreads + threadIdx.x;
+  const bool live = q < Q;
+  double qv[kKnnManyMaxDim];
+#pragma unroll
+  for (int d = 0; d < kKnnManyMaxDim; ++d) qv[d] = (live && d < dim) ? queries[(int64_t)q * dim + d] : 0.0;
+  // the top K sit right-aligned in best[KMAX - K .. KMAX): -inf below them keeps the array sorted, so sorted_insert works
+  // unchanged and the K-th best is always best[KMAX - 1], a fixed register
+  double best[KMAX];
+#pragma unroll
+  for (int i = 0; i < KMAX; ++i) best[i] = i < KMAX - K ? -INFINITY : INFINITY;
+  for (int64_t base = 0; base < M; base += kKnnTile) {
+    const int rows = (int)min((int64_t)kKnnTile, M - base);
+    __syncthreads();
+    for (int i = threadIdx.x; i < rows * dim; i += kKnnManyThreads) tile[i] = archive[base * dim + i];
+    __syncthreads();
+    if (!live) continue;
+    for (int r = 0; r < rows; ++r) {
+      const double* a = tile + r * dim;
+      double d2 = 0.0;
+#pragma unroll
+      for (int d = 0; d < kKnnManyMaxDim; ++d) {
+        if (d < dim) {
+          const double diff = __dsub_rn(a[d], qv[d]);
+          d2 = __dadd_rn(d2, __dmul_rn(diff, diff));                   // no FMA contraction: the existing kernel's distance
+        }
+      }
+      if (d2 < best[KMAX - 1]) sorted_insert<KMAX>(best, d2);
+    }
+  }
+  if (!live) return;
+  const int S = (int)min((int64_t)K, M);
+  double sum = 0.0;
+#pragma unroll
+  for (int i = 0; i < KMAX; ++i)
+    if (i >= KMAX - K && i < KMAX - K + S) sum = __dadd_rn(sum, __dsqrt_rn(best[i]));
+  if (sum_out) sum_out[q] = sum;
+  if (nov_out) {
+    double nu = sum / (double)S;
+    if (nu <= 1e-3) nu = 5e-3;                                         // :323-324
+    nov_out[q] = nu;
+  }
+}
+
+// ---------------- update with a novelty per member (NSRA-ES, Conti et al. 2018, Alg. 3) ----------------
+// mean and ddof-0 variance of v[0..P) by the block reduction of es_stats_coef_kernel (same summation order)
+__device__ __forceinline__ void block_mean_var(const double* __restrict__ v, int P, double* s_red, double& mean, double& var) {
+  double a = 0.0;
+  for (int i = threadIdx.x; i < P; i += blockDim.x) a += v[i];
+  mean = block_sum(a, s_red) / (double)P;
+  a = 0.0;
+  for (int i = threadIdx.x; i < P; i += blockDim.x) { const double d = v[i] - mean; a += d * d; }
+  var = block_sum(a, s_red) / (double)P;
+}
+
+// z-score path in ONE launch: both vectors shaped (a zero-std vector shapes to 0), skip only when both stds are 0,
+// coef[p] = lr/(P sigma) * ((1-w) F~_p + w N~_p) / 2
+__global__ void __launch_bounds__(1024)
+es_member_stats_coef_kernel(const double* __restrict__ r, const double* __restrict__ nov, int P, double* stats, int* status,
+                            const double* __restrict__ lr, double sigma, double nw, double* __restrict__ coef) {
+  __shared__ double s_red[32];
+  double mr, vr, mn, vn;
+  block_mean_var(r, P, s_red, mr, vr);
+  block_mean_var(nov, P, s_red, mn, vn);
+  const double sr = __dsqrt_rn(vr), sn = __dsqrt_rn(vn);
+  const bool skip = (sr == 0.0) && (sn == 0.0);
+  if (threadIdx.x == 0) {
+    stats[0] = mr; stats[1] = sr; stats[2] = skip ? 1.0 : 0.0; stats[3] = mn; stats[4] = sn;
+    if (status) *status = skip ? 1 : 0;
+  }
+  const double f = *lr / ((double)P * sigma);
+  // F~ first, then N~ and the mix: each pass keeps few values live across the division's slow-path call (no spills)
+  for (int p = threadIdx.x; p < P; p += blockDim.x) coef[p] = sr == 0.0 ? 0.0 : (r[p] - mr) / sr;
+  for (int p = threadIdx.x; p < P; p += blockDim.x) {
+    const double N = sn == 0.0 ? 0.0 : (nov[p] - mn) / sn;
+    coef[p] = skip ? 0.0 : f * (((1.0 - nw) * coef[p] + nw * N) / 2.0);
+  }
+}
+
+// centred-rank path, after rank_kernel on each vector: never skips
+__global__ void __launch_bounds__(256)
+es_member_rank_coef_kernel(const double* __restrict__ cf, const double* __restrict__ cn, int P, double* stats, int* status,
+                           const double* __restrict__ lr, double sigma, double nw, double* __restrict__ coef) {
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p == 0) {
+    stats[2] = 0.0;
+    if (status) *status = 0;
+  }
+  if (p >= P) return;
+  const double f = *lr / ((double)P * sigma);
+  coef[p] = f * (((1.0 - nw) * cf[p] + nw * cn[p]) / 2.0);
+}
+
 int gemv_splits(int P, int D) {
   const int64_t colblocks = ceil_div(D, 512);
   int64_t s = ceil_div(16 * (int64_t)sm_count(), colblocks);      // measured at C5: 35 us with 16 CTAs per SM, 63 us with 4
@@ -444,19 +553,11 @@ extern "C" int ppx_es_offsets(uint64_t seed, int64_t* draw_dev, int P, int64_t t
 }
 
 namespace {
-// stats + coefficients over ALL P rewards (replicated: every rank computes the identical z-scores), then the GEMV over
-// members [p_lo, p_lo + p_n) with the column-sum tail
-int es_update_core(double* theta, const float* noise, const int64_t* offsets, const double* rewards, int P, int p_lo, int p_n, int D,
-                   double sigma, double novelty_param, double novelty, const double* novelty_dev, int use_novelty, double decay,
-                   double* lr_inout, int* status_out, void* workspace, double* dtheta_out, cudaStream_t st) {
-  double* stats = (double*)workspace;
-  double* coef = stats + 8;
-  double* partial = coef + 2 * (int64_t)P;
+// the GEMV over members [p_lo, p_lo + p_n) of coef[0..P) with the column-sum tail: theta += update and lr *= decay
+// (dtheta_out NULL), or this rank's partial update -> dtheta_out
+int es_gemv_tail(double* theta, const float* noise, const int64_t* offsets, const double* coef, int P, int p_lo, int p_n, int D,
+                 const double* stats, double decay, double* lr_inout, double* partial, double* dtheta_out, cudaStream_t st) {
   const int splits = gemv_splits(P, D);
-  es_stats_coef_kernel<<<1, 1024, 0, st>>>(rewards, P, stats, status_out, lr_inout, sigma, novelty_param, novelty, novelty_dev,
-                                           use_novelty, coef);
-  int rc = after_launch("es_update(stats+coef)");
-  if (rc) return rc;
   const int p_chunk = (int)ceil_div(p_n, splits);
   dim3 grid((unsigned)ceil_div(D, 512), (unsigned)splits);
   const bool vec = (D % 4 == 0) && ((uintptr_t)noise % 16 == 0);
@@ -465,10 +566,25 @@ int es_update_core(double* theta, const float* noise, const int64_t* offsets, co
   const float* nz = offsets ? noise : noise + (int64_t)p_lo * D;
   if (vec) es_gemv_kernel<true><<<grid, 128, 0, st>>>(nz, offsets ? offsets + p_lo : nullptr, coef + p_lo, p_n, D, p_chunk, partial);
   else es_gemv_kernel<false><<<grid, 128, 0, st>>>(nz, offsets ? offsets + p_lo : nullptr, coef + p_lo, p_n, D, p_chunk, partial);
-  rc = after_launch("es_update(gemv)");
+  int rc = after_launch("es_update(gemv)");
   if (rc) return rc;
   es_colsum_kernel<<<(unsigned)ceil_div(D, 32), 256, 0, st>>>(partial, splits, D, stats, theta, dtheta_out, decay, lr_inout);
   return after_launch("es_update(column sums)");
+}
+
+// stats + coefficients over ALL P rewards (replicated: every rank computes the identical z-scores), then the GEMV over
+// members [p_lo, p_lo + p_n) with the column-sum tail
+int es_update_core(double* theta, const float* noise, const int64_t* offsets, const double* rewards, int P, int p_lo, int p_n, int D,
+                   double sigma, double novelty_param, double novelty, const double* novelty_dev, int use_novelty, double decay,
+                   double* lr_inout, int* status_out, void* workspace, double* dtheta_out, cudaStream_t st) {
+  double* stats = (double*)workspace;
+  double* coef = stats + 8;
+  double* partial = coef + 2 * (int64_t)P;
+  es_stats_coef_kernel<<<1, 1024, 0, st>>>(rewards, P, stats, status_out, lr_inout, sigma, novelty_param, novelty, novelty_dev,
+                                           use_novelty, coef);
+  int rc = after_launch("es_update(stats+coef)");
+  if (rc) return rc;
+  return es_gemv_tail(theta, noise, offsets, coef, P, p_lo, p_n, D, stats, decay, lr_inout, partial, dtheta_out, st);
 }
 }  // namespace
 
@@ -532,6 +648,52 @@ extern "C" int ppx_es_update(double* theta, const float* noise, const int64_t* o
   return after_launch("es_update(apply)");
 }
 
+extern "C" int64_t ppx_es_update_member_workspace(int P, int D) {
+  return (int64_t)sizeof(double) * (8 + 3 * (int64_t)P + (int64_t)gemv_splits(P, D) * D);
+}
+
+extern "C" int ppx_es_update_member(double* theta, const float* noise, const int64_t* offsets, const double* rewards,
+                                    const double* novelties, int P, int p_lo, int p_n, int D, double sigma, double novelty_param,
+                                    int rank_mode, double decay, double* lr_inout, int* status_out, void* workspace,
+                                    double* dtheta_local, const void* const* peer_dtheta_host, void* const* peer_flags_host, int W,
+                                    int rank, uint32_t* seq_dev, uint32_t* status_dev, void* stream) {
+  PPX_REQUIRE(theta && noise && rewards && novelties && lr_inout && workspace, "es_update_member: null pointer");
+  PPX_REQUIRE(P >= 2 && D >= 1 && sigma != 0.0 && W >= 1 && p_lo >= 0 && p_n >= 1 && p_lo + p_n <= P,
+              "es_update_member: P=%d p_lo=%d p_n=%d D=%d W=%d", P, p_lo, p_n, D, W);
+  PPX_REQUIRE(W >= 2 || (p_lo == 0 && p_n == P), "es_update_member: one rank updates all P members (p_lo=%d p_n=%d)", p_lo, p_n);
+  p2p::Peers PP;
+  if (W >= 2) {
+    PPX_REQUIRE(dtheta_local, "es_update_member: W=%d needs dtheta_local", W);
+    int rc = p2p::fill(&PP, peer_dtheta_host, peer_flags_host, W, rank, seq_dev, status_dev);
+    if (rc) return rc;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  double* stats = (double*)workspace;
+  double* coef = stats + 8;
+  double* cf = coef + P;
+  double* cn = cf + P;
+  double* partial = cn + P;
+  int rc;
+  if (rank_mode) {
+    rank_kernel<<<(unsigned)ceil_div(P, 256), 256, 0, st>>>(rewards, P, nullptr, cf);
+    rc = after_launch("es_update_member(rank fitness)");
+    if (rc) return rc;
+    rank_kernel<<<(unsigned)ceil_div(P, 256), 256, 0, st>>>(novelties, P, nullptr, cn);
+    rc = after_launch("es_update_member(rank novelty)");
+    if (rc) return rc;
+    es_member_rank_coef_kernel<<<(unsigned)ceil_div(P, 256), 256, 0, st>>>(cf, cn, P, stats, status_out, lr_inout, sigma,
+                                                                           novelty_param, coef);
+  } else {
+    es_member_stats_coef_kernel<<<1, 1024, 0, st>>>(rewards, novelties, P, stats, status_out, lr_inout, sigma, novelty_param, coef);
+  }
+  rc = after_launch("es_update_member(coef)");
+  if (rc) return rc;
+  rc = es_gemv_tail(theta, noise, offsets, coef, P, p_lo, p_n, D, stats, decay, lr_inout, partial, W >= 2 ? dtheta_local : nullptr, st);
+  if (rc || W == 1) return rc;
+  es_apply_p2p_kernel<<<1, 1024, 0, st>>>(PP, theta, D, stats, decay, lr_inout);
+  return after_launch("es_update_member(p2p apply)");
+}
+
 extern "C" int ppx_rank_center(const double* r, int P, int64_t* rank_out, double* centred_out, void* stream) {
   PPX_REQUIRE(r && P >= 2 && (rank_out || centred_out), "rank_center: bad arguments");
   rank_kernel<<<(unsigned)ceil_div(P, 256), 256, 0, (cudaStream_t)stream>>>(r, P, rank_out, centred_out);
@@ -569,4 +731,15 @@ extern "C" int ppx_knn_novelty(const double* archive, int64_t M, const double* q
     knn_merge_kernel<32><<<(unsigned)Q, 32, 0, (cudaStream_t)stream>>>(cand, splits * K, M, K, sum_out, novelty_out);
   }
   return after_launch("knn_novelty");
+}
+
+extern "C" int ppx_knn_novelty_many(const double* archive, int64_t M, const double* queries, int Q, int dim, int K, double* sum_out,
+                                    double* novelty_out, void* stream) {
+  PPX_REQUIRE(archive && queries && M >= 1 && Q >= 1 && (sum_out || novelty_out), "knn_novelty_many: bad arguments");
+  PPX_REQUIRE(dim >= 1 && dim <= kKnnManyMaxDim, "knn_novelty_many: dim=%d (1..%d)", dim, kKnnManyMaxDim);
+  PPX_REQUIRE(K >= 1 && K <= 32, "knn_novelty_many: K=%d (1..32)", K);
+  const unsigned grid = (unsigned)ceil_div(Q, kKnnManyThreads);
+  if (K <= 16) knn_many_kernel<16><<<grid, kKnnManyThreads, 0, (cudaStream_t)stream>>>(archive, M, queries, Q, dim, K, sum_out, novelty_out);
+  else knn_many_kernel<32><<<grid, kKnnManyThreads, 0, (cudaStream_t)stream>>>(archive, M, queries, Q, dim, K, sum_out, novelty_out);
+  return after_launch("knn_novelty_many");
 }

@@ -26,7 +26,9 @@ class EvolutionStrategy(object):
     def __init__(self, env_id=None, hidden_sizes=(64, 64), nsr_plateu=1.5, nsr_range=(0, 1), nsr_update=0.05,
                  population_size=50, sigma=0.1, learning_rate=0.01, decay=0.9995, novelty_param=0.5, num_threads=1,
                  obs_dim=None, n_actions=None, device="cuda", noise_table_size=1 << 24, noise_seed=0,
-                 fitness_shaping="zscore"):
+                 fitness_shaping="zscore", novelty_mode="brain"):
+        if novelty_mode not in ("brain", "member"):
+            raise ValueError(f"novelty_mode must be 'brain' or 'member', got {novelty_mode!r}")
         if obs_dim is None or n_actions is None:
             raise ValueError("pass obs_dim= and n_actions= (the reference reads them from gym.make(env_id), "
                              "evolution_strategies.py:121; the env layer is out of scope here)")
@@ -48,6 +50,9 @@ class EvolutionStrategy(object):
         self.K = 10
         self.nsr_plateu, self.nsr_range, self.nsr_update = nsr_plateu, list(nsr_range), nsr_update
         self.fitness_shaping = fitness_shaping
+        # "brain": the reference's update, brain b's novelty broadcast over the population; "member": NSRA-ES (Conti et al.
+        # 2018, Alg. 3), every member's own novelty shaped next to its fitness (DESIGN.md §3.16)
+        self.novelty_mode = novelty_mode
         self._status = torch.zeros(1, dtype=torch.int32, device=self.device)
         self._ws = None
         self._noise = None
@@ -73,7 +78,7 @@ class EvolutionStrategy(object):
                         nsr_range=list(self.nsr_range), nsr_update=self.nsr_update, population_size=int(self.POPULATION_SIZE),
                         sigma=float(self.SIGMA), decay=self.decay, obs_dim=int(self.shapes[0][0]),
                         n_actions=int(self.shapes[-1][1]), noise_table_size=self._noise_size, noise_seed=self._noise_seed,
-                        fitness_shaping=self.fitness_shaping),
+                        fitness_shaping=self.fitness_shaping, novelty_mode=self.novelty_mode),
             K=int(self.K), theta=self.theta.cpu(), lr=self._lr.cpu(), draw=self._draw.cpu(),
             novelty_param=float(self.novelty_param), world_size=D.world_size(), rank=D.rank())
         if self.thetas is not None:
@@ -258,11 +263,16 @@ class EvolutionStrategy(object):
     def _update_weights(self, rewards, population, novelty=None):
         """:217-239.  Asynchronous; `self.update_skipped` reads back the std==0 flag.  `novelty` may be a python float
         (as in the reference) or a 1-element f64 CUDA tensor (e.g. `novelty_batch(...)[1][m:m+1]`), which keeps the
-        k-NN result on the device -- no host round trip in the step."""
+        k-NN result on the device -- no host round trip in the step.
+        novelty_mode="member": `novelty` is required, the novelty of every member (f64 [P], global member order, e.g.
+        `member_novelty(...)`), and the update is ppx_es_update_member: fitness and novelty each shaped over the P members,
+        mixed with novelty_param; z-score skips only when both stds are 0."""
         noise, off = self._as_eps(population)
         P = off.numel() if off is not None else noise.shape[0]
         r = torch.as_tensor(np.asarray(rewards, dtype=np.float64)).to(self.device) if not isinstance(rewards, torch.Tensor) \
             else rewards.to(self.device, torch.float64)
+        if self.novelty_mode == "member":
+            return self._update_weights_member(r, noise, off, P, novelty)
         need = L.call("ppx_es_update_workspace", P, self.D)
         if self._ws is None or self._ws.numel() * 8 < need:
             self._ws = torch.zeros(need // 8 + 1, dtype=torch.float64, device=self.device)     # holds self re-arming tickets
@@ -290,6 +300,32 @@ class EvolutionStrategy(object):
                int(self.fitness_shaping == "centered_rank"), float(self.decay), self._lr.data_ptr(),
                self._status.data_ptr(), self._ws.data_ptr(), L.stream())
 
+    def _update_weights_member(self, r, noise, off, P, novelty):
+        if novelty is None:
+            raise ValueError("novelty_mode='member' updates with the novelty of every member: pass novelty= (f64 [P])")
+        nov = torch.as_tensor(np.asarray(novelty, dtype=np.float64)).to(self.device) if not isinstance(novelty, torch.Tensor) \
+            else novelty.to(self.device, torch.float64)
+        nov = nov.reshape(-1).contiguous()
+        if nov.numel() != P or r.numel() != P:
+            raise ValueError(f"member mode needs {P} rewards and {P} novelties, got {r.numel()} and {nov.numel()}")
+        need = L.call("ppx_es_update_member_workspace", P, self.D)
+        if self._ws is None or self._ws.numel() * 8 < need:
+            self._ws = torch.zeros(need // 8 + 1, dtype=torch.float64, device=self.device)
+        W, rk = D.world_size(), D.rank()
+        rank_mode = int(self.fitness_shaping == "centered_rank")
+        px = self._peer_exchange() if (W > 1 and not rank_mode and P % W == 0) else None
+        common = (self.theta.data_ptr(), noise.data_ptr(), off.data_ptr() if off is not None else None, r.data_ptr(),
+                  nov.data_ptr(), P)
+        tail = (float(self.SIGMA), float(self.novelty_param), rank_mode, float(self.decay), self._lr.data_ptr(),
+                self._status.data_ptr(), self._ws.data_ptr())
+        if px is not None:
+            self.update_mode = "sharded: partial GEMV over P/W members + fused peer-memory all-reduce of the update"
+            L.call("ppx_es_update_member", *common, rk * (P // W), P // W, self.D, *tail, self._dtheta.data_ptr(), px.peer_grad,
+                   px.peer_flags[2], px.W, px.rank, px.seq[2], px.status_ptr, L.stream())
+            return
+        self.update_mode = "single" if W == 1 else "replicated"
+        L.call("ppx_es_update_member", *common, 0, P, self.D, *tail, None, None, None, 1, 0, None, None, L.stream())
+
     def _peer_exchange(self):
         if self._px is False:
             self._px = D.peer_exchange_or_none(2 * self.D, self.device, L.call("ppx_p2p_max_params"))
@@ -301,7 +337,8 @@ class EvolutionStrategy(object):
     def _hp_state(self):
         """Every host scalar the ask / tell graphs bake into kernel arguments: a graph is keyed on these, so a run that
         adapts novelty_param (or a caller that changes sigma / decay / K) replays a graph captured with the current values."""
-        return (float(self.novelty_param), float(self.SIGMA), float(self.decay), int(self.K), self.fitness_shaping)
+        return (float(self.novelty_param), float(self.SIGMA), float(self.decay), int(self.K), self.fitness_shaping,
+                self.novelty_mode)
 
     def _graph(self, key, fn):
         ent = self._graphs.get(key)
@@ -349,15 +386,27 @@ class EvolutionStrategy(object):
         self._novelty = out[2]
         return out
 
-    def tell(self, local_rewards, brain=0):
+    def tell(self, local_rewards, brain=0, local_novelty=None):
         """Second half (:217-239): exchange the fitness of the rank-local members and update the parameters with the
         novelty of meta-population member `brain` computed by the last ask().  `local_rewards` must be a persistent CUDA
-        tensor (its address is captured)."""
-        key = ("tell", local_rewards.data_ptr(), int(brain), self._novelty.data_ptr() if self._novelty is not None else 0,
-               self._hp_state())
+        tensor (its address is captured).  novelty_mode="member": `local_novelty` (required; a persistent CUDA f64 tensor
+        [P/W], this rank's members, e.g. `member_novelty(archive, bc)`) goes through the same all-gather as the fitness and
+        the update is ppx_es_update_member."""
+        member = self.novelty_mode == "member"
+        if member != (local_novelty is not None):
+            raise ValueError("tell(local_novelty=) is required with novelty_mode='member' and rejected with 'brain'")
+        if member:
+            L.require_cuda(local_novelty, torch.float64, "local_novelty")
+            key = ("tell", local_rewards.data_ptr(), local_novelty.data_ptr(), self._hp_state())
+        else:
+            key = ("tell", local_rewards.data_ptr(), int(brain), self._novelty.data_ptr() if self._novelty is not None else 0,
+                   self._hp_state())
 
         def fn():
             r_all = self.gather_fitness(local_rewards)
+            if member:
+                self._update_weights(r_all, self._ask_off, novelty=self.gather_fitness(local_novelty))
+                return
             nov = self._novelty[brain:brain + 1] if self._novelty is not None else None
             self._update_weights(r_all, self._ask_off, novelty=nov)
         return self._graph(key, fn)
@@ -513,11 +562,31 @@ class EvolutionStrategy(object):
 
     def run_generation(self, env, *, max_steps, archive=None, queries=None, brain=0, check_every=8):
         """One ES generation on an env that lives on the GPU: ask() -> evaluate() of this rank's members -> tell().  Sharded,
-        every rank evaluates its P/W envs and tell() gathers the fitness.  Returns what evaluate() returned."""
+        every rank evaluates its P/W envs and tell() gathers the fitness.  Returns what evaluate() returned.
+        novelty_mode="member": ask() -> evaluate() (the env must have behavior()) -> member_novelty(archive, BCs) -> tell();
+        `archive` (f64 CUDA [n, k]) is required and `queries` / `brain` are not used."""
+        if self.novelty_mode == "member":
+            if archive is None:
+                raise ValueError("run_generation() with novelty_mode='member' scores the members against archive=")
+            self.ask()
+            out = self.evaluate(env, max_steps=max_steps, check_every=check_every)
+            if out[2] is None:
+                raise TypeError("novelty_mode='member' characterises the members by env.behavior() (CUDA f64 [N, k])")
+            nov = self._member_nov_buffer(out[2].shape[0])
+            self.member_novelty(archive, out[2], out=nov)
+            self.tell(out[0], local_novelty=nov)
+            return out
         self.ask(archive, queries)
         out = self.evaluate(env, max_steps=max_steps, check_every=check_every)
         self.tell(out[0], brain=brain)
         return out
+
+    def _member_nov_buffer(self, n):
+        """The persistent [n] f64 buffer of this rank's member novelties that the captured tell() graph reads."""
+        buf = getattr(self, "_member_nov", None)
+        if buf is None or buf.numel() != n:
+            buf = self._member_nov = torch.zeros(n, dtype=torch.float64, device=self.device)
+        return buf
 
     # ---- the ES-NSRA run loop (evolution_strategies.py:293-384, order of SURVEY §3.4; DESIGN.md §3.15) ----
     def run(self, env, brain_env, iterations, *, max_steps, meta_population_size=2, reward_target=None, log_interval=1,
@@ -540,7 +609,11 @@ class EvolutionStrategy(object):
         novelty_param -= nsr_update (at least nsr_range[0]) if R > B + nsr_plateu, else += nsr_update (at most
         nsr_range[1]); then B = max(B, R).  A later run() (or one after `load`) continues the run.  Logged through
         `ppo_exploration_b200.logger` as ("ES", env_id): iteration, total_time, reward (f_b), brain, novelty_param (the
-        weight of the generation's update), learning_rate, fitness_mean, fitness_max, archive_size.  Returns self."""
+        weight of the generation's update), learning_rate, fitness_mean, fitness_max, archive_size.
+        novelty_mode="member" (NSRA-ES, DESIGN.md §3.16): `env` must have behavior() too.  After evaluate(env), one
+        ppx_knn_novelty_many launch scores this rank's members' BCs against the archive as it stands before BC_b is appended
+        (M passed by value, so the tell graph is never recaptured as the archive grows), and tell() updates brain b with the
+        members' own novelties.  The log gains novelty_mean, the population's mean novelty.  Returns self."""
         import time
         from . import logger as ppx_logger
         M, W = int(meta_population_size), D.world_size()
@@ -553,6 +626,9 @@ class EvolutionStrategy(object):
             raise ValueError(f"brain_env runs {int(brain_env.num_envs)} envs, the meta-population has {M} brains")
         if not callable(getattr(brain_env, "behavior", None)):
             raise TypeError("run() characterises the brains by brain_env.behavior() (CUDA f64 [M, k])")
+        member = self.novelty_mode == "member"
+        if member and not callable(getattr(env, "behavior", None)):
+            raise TypeError("run() with novelty_mode='member' characterises the members by env.behavior() (CUDA f64 [N, k])")
         if W > 1 and getattr(brain_env, "env_offset", 0) != 0:
             raise ValueError("every rank must step the same brain_env: build it with env_offset=0")
         if self.thetas is not None and self.thetas.shape[0] != M:
@@ -577,11 +653,18 @@ class EvolutionStrategy(object):
             w = float(self.novelty_param)
             self.theta.copy_(self.thetas[b])
             self.ask()
-            nu_b = self._run_dev[M + 4:M + 5]                   # tell() mixes in nu_b from a fixed slot: one graph for every brain
-            nu_b.copy_(self._run_dev[b:b + 1])
-            self._novelty = nu_b
-            fit = self.evaluate(env, max_steps=max_steps, check_every=check_every)[0]
-            self.tell(fit)
+            if member:
+                fit, _, bc_p = self.evaluate(env, max_steps=max_steps, check_every=check_every)
+                nov_p = self._member_nov_buffer(bc_p.shape[0])
+                L.call("ppx_knn_novelty_many", self._archive.data_ptr(), self._archive_n, bc_p.data_ptr(), bc_p.shape[0],
+                       bc_p.shape[1], int(self.K), None, nov_p.data_ptr(), L.stream())
+                self.tell(fit, local_novelty=nov_p)
+            else:
+                nu_b = self._run_dev[M + 4:M + 5]               # tell() mixes in nu_b from a fixed slot: one graph for every brain
+                nu_b.copy_(self._run_dev[b:b + 1])
+                self._novelty = nu_b
+                fit = self.evaluate(env, max_steps=max_steps, check_every=check_every)[0]
+                self.tell(fit)
             self.thetas[b].copy_(self.theta)
             bc, f = self._brains(brain_env, max_steps, check_every)
             self._bc_m.copy_(bc)
@@ -593,6 +676,8 @@ class EvolutionStrategy(object):
             row[M + 1].copy_(fit_all.mean())
             row[M + 2].copy_(fit_all.max())
             row[M + 3].copy_(self._lr[0])
+            if member:
+                row[M + 4].copy_(self.gather_fitness(nov_p).mean())
             self._generation += 1
             pending = (b, w)
         if pending is not None:
@@ -621,9 +706,10 @@ class EvolutionStrategy(object):
         self._bc_m = torch.empty(M, k, dtype=torch.float64, device=self.device)
         self._f_m = torch.empty(M, dtype=torch.float64, device=self.device)
         self._knn_sums = torch.empty(M, dtype=torch.float64, device=self.device)
-        # [nu_0 .. nu_M-1, f_b, fitness mean, fitness max, lr | nu_b]: the first M + 4 are the generation's read
+        # [nu_0 .. nu_M-1, f_b, fitness mean, fitness max, lr | nu_b]: the first M + 4 are the generation's read; member
+        # mode reads one more slot, M + 4 = the population's mean novelty (it has no nu_b)
         self._run_dev = torch.zeros(M + 5, dtype=torch.float64, device=self.device)
-        self._run_host = torch.zeros(M + 4, dtype=torch.float64).pin_memory()
+        self._run_host = torch.zeros(M + 4 + (self.novelty_mode == "member"), dtype=torch.float64).pin_memory()
         self._run_event = torch.cuda.Event()
 
     def _archive_append(self, row):
@@ -674,7 +760,8 @@ class EvolutionStrategy(object):
             for key, v in (("time/iteration", self._generation), ("time/total_time", time.time() - start), ("es/reward", fb),
                            ("es/brain", b), ("es/novelty_param", w), ("es/learning_rate", float(vals[M + 3])),
                            ("es/fitness_mean", float(vals[M + 1])), ("es/fitness_max", float(vals[M + 2])),
-                           ("es/archive_size", self._archive_n)):
+                           ("es/archive_size", self._archive_n)) + ((("es/novelty_mean", float(vals[M + 4])),)
+                                                                    if self.novelty_mode == "member" else ()):
                 ppx_logger.record(key, v)
             ppx_logger.dump(step=self._generation)
         return reward_target is not None and fb > reward_target
@@ -730,6 +817,23 @@ class EvolutionStrategy(object):
         L.call("ppx_knn_novelty", a.data_ptr(), a.shape[0], q.data_ptr(), q.shape[0], a.shape[1], int(K), s.data_ptr(),
                nov.data_ptr(), L.stream())
         return s, nov
+
+    def member_novelty(self, archive, behaviors, out=None):
+        """The novelty of every row of `behaviors` [n, k] against `archive` [M, k] (both f64 CUDA, or array-likes): f64 CUDA
+        [n], with ppx_knn_novelty's values bit for bit, one thread per query (ppx_knn_novelty_many; k <= 8).  `out`: an f64
+        CUDA [n] buffer to write into."""
+        a = archive if isinstance(archive, torch.Tensor) else torch.as_tensor(np.asarray(archive, np.float64))
+        a = a.to(self.device, torch.float64).contiguous()
+        q = behaviors if isinstance(behaviors, torch.Tensor) else torch.as_tensor(np.asarray(behaviors, np.float64))
+        q = q.to(self.device, torch.float64).reshape(-1, a.shape[1]).contiguous()
+        if out is None:
+            out = torch.empty(q.shape[0], dtype=torch.float64, device=self.device)
+        L.require_cuda(out, torch.float64, "out")
+        if out.numel() != q.shape[0]:
+            raise ValueError(f"out has {out.numel()} entries for {q.shape[0]} behaviours")
+        L.call("ppx_knn_novelty_many", a.data_ptr(), a.shape[0], q.data_ptr(), q.shape[0], a.shape[1],
+               int(self.K), None, out.data_ptr(), L.stream())
+        return out
 
     def get_kNN(self, archive, bc, n_neighbors):
         """:264-281: summed distance to the n_neighbors nearest archive entries (python float)."""

@@ -140,35 +140,25 @@ int ppx_mean_std(const float* x, int64_t n, double* out2, void* stream);
 
 /* Host-side (no GPU): bit-exact replay of numpy's legacy `np.random.permutation(n)` (the draw of
  * buffer.py:239) from numpy's own MT19937 state (np.random.get_state(): key[624], pos); the advanced
- * state is written back so the caller can np.random.set_state it.  `_draws` + `_apply` are the same
- * computation split into its RNG-bound and its memory-bound half so two host threads can pipeline
- * consecutive epochs. */
+ * state is written back so the caller can np.random.set_state it. */
 int ppx_np_permutation(uint32_t* key624_host, int* pos_host, int64_t n, int64_t* out_host);
-int ppx_np_shuffle_draws(uint32_t* key624_host, int* pos_host, int64_t n, int64_t* j_out_host);
-int ppx_np_shuffle_apply(const int64_t* j_host, int64_t n, int64_t* out_host);
-/* n <= 2^31 - 1: int32 partner list / scratch (constant-mask draw loop, cache-resident swaps); same stream. */
+/* Only the draws of the same stream, n <= 2^31 - 1, as an int32 Fisher-Yates partner list: _draws32 indexed by position
+ * (j_out[i] = partner of position i, constant-mask scalar loop), _draws32_stream in acceptance order (acc[r] belongs to
+ * position n-1-r; AVX-512 block rejection when available). */
 int ppx_np_shuffle_draws32(uint32_t* key624_host, int* pos_host, int64_t n, int32_t* j_out_host);
-int ppx_np_shuffle_apply32(const int32_t* j_host, int64_t n, int32_t* scratch_host, int64_t* out_host);
-/* Streaming pair for two host threads working on the SAME permutation: _draws32_stream writes the accepted
- * partners in acceptance order (acc[r] belongs to position n-1-r; AVX-512 block rejection when available) and
- * publishes the count of final entries through *progress_host (start it at 0); _apply32_stream consumes them as
- * they appear, so the permutation is ready ~max(stage) instead of sum(stages) after the call. */
-int ppx_np_shuffle_draws32_stream(uint32_t* key624_host, int* pos_host, int64_t n, int32_t* acc_host,
-                                  int64_t* progress_host);
-int ppx_np_shuffle_apply32_stream(const int32_t* acc_host, int64_t n, const int64_t* progress_host,
-                                  int32_t* scratch_host, int64_t* out_host);
-/* The same swaps applied ON THE DEVICE, in parallel and bit-exactly (shuffle_dev.cu): j_dev is the uploaded partner
+int ppx_np_shuffle_draws32_stream(uint32_t* key624_host, int* pos_host, int64_t n, int32_t* acc_host);
+/* The swaps applied ON THE DEVICE, in parallel and bit-exactly (shuffle_dev.cu): j_dev is the uploaded partner
  * list, either indexed by position (acceptance_order = 0: j_dev[i], i = 1 .. n-1, from ppx_np_shuffle_draws32) or in
- * acceptance order (1: entry r belongs to position n-1-r, from ppx_np_shuffle_draws32_stream, the AVX-512 draw loop);
- * out_dev [n] int64 is arange(n) after the swaps = np.random.permutation(n).  For hosts whose cores are shared by many ranks (the draws stay on the host: they ARE the
- * RNG stream).  n <= 2^24; workspace of ppx_np_shuffle_apply_device_workspace(n) bytes; asynchronous on `stream`. */
+ * acceptance order (1: entry r belongs to position n-1-r, from ppx_np_shuffle_draws32_stream);
+ * out_dev [n] int64 is arange(n) after the swaps = np.random.permutation(n).  n < 2^31; workspace of
+ * ppx_np_shuffle_apply_device_workspace(n) bytes (24 per index; -1 for an unsupported n); asynchronous on `stream`. */
 int64_t ppx_np_shuffle_apply_device_workspace(int64_t n);
 int ppx_np_shuffle_apply_device(const int32_t* j_dev, int64_t n, int acceptance_order, void* workspace, int64_t* out_dev,
                                 void* stream);
 /* One staging step of a permutation, callable from the host thread that drew it: H2D of the pinned partner list (acceptance
  * order) into j_dev, ppx_np_shuffle_apply_device into out_dev, and cudaEventRecord of `copied_event` (after the copy) and
  * `ready_event` (after the swaps) when given (cudaEvent_t; NULL = skip).  Makes the device owning j_dev current for the
- * calling thread.  2 <= n <= 2^24. */
+ * calling thread.  1 <= n < 2^31. */
 int ppx_np_shuffle_stage(const int32_t* j_host_pinned, int64_t n, int32_t* j_dev, void* workspace, int64_t* out_dev,
                          void* stream, void* copied_event, void* ready_event);
 

@@ -71,12 +71,8 @@ SIGNATURES = {
     "ppx_loss_row_commit": (c_i, [c_p, c_p, c_p, c_i, c_i, c_p]),
     "ppx_mean_std": (c_i, [c_p, c_l, c_p, c_p]),
     "ppx_np_permutation": (c_i, [c_p, C.POINTER(c_i), c_l, c_p]),
-    "ppx_np_shuffle_draws": (c_i, [c_p, C.POINTER(c_i), c_l, c_p]),
-    "ppx_np_shuffle_apply": (c_i, [c_p, c_l, c_p]),
     "ppx_np_shuffle_draws32": (c_i, [c_p, C.POINTER(c_i), c_l, c_p]),
-    "ppx_np_shuffle_apply32": (c_i, [c_p, c_l, c_p, c_p]),
-    "ppx_np_shuffle_draws32_stream": (c_i, [c_p, C.POINTER(c_i), c_l, c_p, c_p]),
-    "ppx_np_shuffle_apply32_stream": (c_i, [c_p, c_l, c_p, c_p, c_p]),
+    "ppx_np_shuffle_draws32_stream": (c_i, [c_p, C.POINTER(c_i), c_l, c_p]),
     "ppx_np_shuffle_apply_device_workspace": (c_l, [c_l]),
     "ppx_np_shuffle_apply_device": (c_i, [c_p, c_l, c_i, c_p, c_p, c_p]),
     "ppx_np_shuffle_stage": (c_i, [c_p, c_l, c_p, c_p, c_p, c_p, c_p, c_p]),

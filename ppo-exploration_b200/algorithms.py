@@ -24,8 +24,7 @@ import torch
 
 from . import _lib as L
 from . import dist as D
-from .buffer import (RolloutStorage, IntrinsicStorage, HostRngStream, DevicePartners, device_shuffle_default,
-                     rng_states_equal, _dev)
+from .buffer import RolloutStorage, IntrinsicStorage, HostRngStream, rng_states_equal, _dev
 from .models import Policy, RndNetwork, IntrinsicCuriosityModule, ActionConverter, _Scratch
 from .util import RunningMeanStd, normalize_obs
 
@@ -79,13 +78,12 @@ class BaseAlgorithm(object):
         self._cursor = torch.zeros(1, dtype=torch.int64, device=self.device)    # optimiser step of the running train() call
         self._losses_buf = None                # [steps, 8] f64, persistent (graphs keep its address)
         self._readback = None                  # pinned host copy of the loss log (+ sharded status words)
-        self._perm_all, self._perm_events, self._perm_keep, self._copy_stream = None, [], [], None
+        self._perm_all, self._perm_events, self._copy_stream = None, [], None
         self._perm_gen = 0
         self._perm_sets, self._next_set = None, 0               # two staging sets: the speculative stream of the NEXT pass fills the other one
         self._perm_j, self._perm_ws = None, None
         self._glob = None                      # sharded "global": the all-gathered rollout [W, T, N, ...] per field
         self.rng_wait_s = 0.0                  # cumulative host time train() spent waiting for permutations
-        self.device_shuffle = device_shuffle_default()         # swaps of the epoch shuffle applied on the GPU (shuffle_dev.cu)
 
     def __new__(cls, *args, **kwargs):
         obj = super().__new__(cls)
@@ -510,7 +508,7 @@ class BaseAlgorithm(object):
         if sp is not None:
             stream, snapshot = sp
             if (stream.script == list(script) and rng_states_equal(cur, snapshot) and stream.err is None
-                    and stream.device_apply == self._device_apply() and stream.generation == self._perm_gen):
+                    and stream.generation == self._perm_gen):
                 return stream
             stream.cancel()
             stream.t1.join()                                    # its uploader must not queue anything after the new stream's
@@ -521,26 +519,24 @@ class BaseAlgorithm(object):
         the partner list + the parallel swaps, on the copy stream) into the staging set this stream owns."""
         set_idx, self._next_set = self._next_set, self._next_set ^ 1
         total = next((int(op[1]) for op in script if op[0] == 'perm'), 0)
-        up = None
-        if self._device_apply() and self._perm_j is not None and 2 <= total <= (1 << 24):
-            dst_all, js, ws, cs = self._perm_sets[set_idx], self._perm_j, self._perm_ws, self._copy_stream
-            evs = self._stage_events[set_idx]
+        dst_all, js, ws, cs = self._perm_sets[set_idx], self._perm_j, self._perm_ws, self._copy_stream
+        evs = self._stage_events[set_idx]
 
-            def up(k, dp):                                      # runs on the draw thread: one GIL-free C call
-                copied, ready = evs[k]
-                L.call("ppx_np_shuffle_stage", dp.j.data_ptr(), total, js[k & 1].data_ptr(), ws.data_ptr(),
-                       dst_all.data_ptr() + 8 * k * total, cs.cuda_stream, copied.cuda_event, ready.cuda_event)
-                dp.ready = ready
-                dp.release(copied)                              # the pinned partner buffer is free once the copy has run
-                return copied
-        stream = HostRngStream(script, state=state, device_apply=self._device_apply(), uploader=up)
+        def up(k, dp):                                          # runs on the draw thread: one GIL-free C call
+            copied, ready = evs[k]
+            L.call("ppx_np_shuffle_stage", dp.j.data_ptr(), total, js[k & 1].data_ptr(), ws.data_ptr(),
+                   dst_all.data_ptr() + 8 * k * total, cs.cuda_stream, copied.cuda_event, ready.cuda_event)
+            dp.ready = ready
+            dp.release(copied)                                  # the pinned partner buffer is free once the copy has run
+            return copied
+        stream = HostRngStream(script, state=state, uploader=up)
         stream.set_idx, stream.generation = set_idx, self._perm_gen
         return stream
 
     def _device_apply(self):
-        """The swaps of the shuffle run on the GPU (only the draws ARE the RNG stream); the permutation is only ever
-        needed on the device."""
-        return bool(self.device_shuffle)
+        """The swaps of the epoch shuffle run on the GPU; only the draws, which are the RNG stream, stay on the host.
+        Always true; bench.py reads it."""
+        return True
 
     def _rng_close(self, rng, speculate=True):
         """Commit the consumed draws to the global numpy RNG and pre-draw the next call's stream from there."""
@@ -571,10 +567,11 @@ class BaseAlgorithm(object):
         if self._perm_sets is None or self._perm_sets[0].numel() != self.n_epochs * total:
             self._perm_sets = [torch.empty(self.n_epochs * total, dtype=torch.int64, device=self.device) for _ in range(2)]
             self._copy_stream = self._copy_stream or torch.cuda.Stream(device=self.device)
-            self._perm_j = None
-            if self._device_apply() and 2 <= total <= (1 << 24):
-                self._perm_j = [torch.empty(total, dtype=torch.int32, device=self.device) for _ in range(2)]
-                self._perm_ws = torch.empty(L.call("ppx_np_shuffle_apply_device_workspace", total), dtype=torch.uint8, device=self.device)
+            ws_bytes = L.call("ppx_np_shuffle_apply_device_workspace", total)
+            if ws_bytes < 0:
+                raise ValueError(f"ppx: {total} shuffle indices per epoch; the device shuffle takes fewer than 2^31")
+            self._perm_j = [torch.empty(total, dtype=torch.int32, device=self.device) for _ in range(2)]
+            self._perm_ws = torch.empty(ws_bytes, dtype=torch.uint8, device=self.device)
             # events of the staging steps (copy done, permutation ready), recorded once so that their handles exist
             self._stage_events = [[(torch.cuda.Event(), torch.cuda.Event()) for _ in range(self.n_epochs)] for _ in range(2)]
             for evs in self._stage_events:
@@ -583,12 +580,10 @@ class BaseAlgorithm(object):
                         e.record(self._copy_stream)
             _Scratch.generation += 1
             self._perm_gen += 1                                 # retires a speculative stream that stages into the old sets
-        self._perm_events, self._perm_keep = [None] * self.n_epochs, []
+        self._perm_events = [None] * self.n_epochs
         rng = self._rng_open(self._rng_script(ro, randn_per_minibatch))
         self._perm_set = rng.set_idx
         self._perm_all = self._perm_sets[rng.set_idx]
-        if rng.uploader is None:                                # uploads issued by this thread: after the previous readers of the set
-            self._copy_stream.wait_stream(torch.cuda.current_stream())
         self._rng_check = None
         if D.world_size() > 1 and self.shard_shuffle == "global":
             # every rank must draw the SAME permutation: exchange a digest of the numpy state the stream starts from
@@ -610,30 +605,13 @@ class BaseAlgorithm(object):
         for k in srcs:
             D.all_gather_into(self._glob[k], getattr(ro, k))
 
-    def _perm_upload(self, rng, epoch, total):
-        """Stage epoch `epoch`'s permutation in its slice of the all-epoch device buffer, on the copy stream (the H2D
-        copy and the device-side swaps overlap the previous epoch's kernels)."""
+    def _perm_upload(self, rng, epoch):
+        """Epoch `epoch`'s permutation: the stream's draw thread has staged it (or is staging it) in its slice of the
+        all-epoch device buffer on the copy stream; this takes the event that marks it ready."""
         t0 = time.perf_counter()
-        perm = rng.next()                                       # pinned int64 [total], or the partner list (DevicePartners)
+        perm = rng.next()                                       # the partner list (DevicePartners), staged by the uploader
         self.rng_wait_s += time.perf_counter() - t0             # host time blocked on the (sequential) numpy RNG stream
-        on_device = isinstance(perm, DevicePartners)
-        if on_device and perm.ready is not None:                # already staged by the stream's draw thread
-            self._perm_events[epoch] = perm.ready
-            return
-        dst = self._perm_all[epoch * total:(epoch + 1) * total]
-        with torch.cuda.stream(self._copy_stream):
-            if on_device:                                       # 4 bytes per index up instead of 8, swaps resolved in parallel on the copy stream
-                j = self._perm_j[epoch & 1]
-                j.copy_(perm.j, non_blocking=True)
-                L.call("ppx_np_shuffle_apply_device", j.data_ptr(), total, 1, self._perm_ws.data_ptr(), dst.data_ptr(), L.stream())
-            else:
-                dst.copy_(perm, non_blocking=True)
-            ev = torch.cuda.Event()
-            ev.record(self._copy_stream)
-        if on_device:
-            perm.release(ev)                                    # the pinned partner buffer is free once the copy has run
-        self._perm_events[epoch] = ev
-        self._perm_keep.append(perm)                            # keep the pinned source alive until train() has synchronised
+        self._perm_events[epoch] = perm.ready
 
     def _epoch_minibatches(self, ro, rng, epoch=0, n_epochs=1):
         """Yields (gather options, B_local, B_total, graph key, sources) for one epoch.  The indices are the reference's
@@ -646,7 +624,7 @@ class BaseAlgorithm(object):
         glob = W > 1 and self.shard_shuffle == "global"
         total, Bg, n_mb = self._train_geometry(ro)
         if self._perm_events[epoch] is None:
-            self._perm_upload(rng, epoch, total)
+            self._perm_upload(rng, epoch)
         torch.cuda.current_stream().wait_event(self._perm_events[epoch])
         for k in range(n_mb):
             bg = min(Bg, total - k * Bg)
@@ -660,7 +638,7 @@ class BaseAlgorithm(object):
                 opts = L.GatherOpts(0, 0, 0, self._cursor.data_ptr(), n_mb, total, Bg)
                 yield opts, 0, bg, (bg * W if W > 1 else 0), ("l", bg, self._perm_set), None
         if epoch + 1 < n_epochs:                                # after this epoch's randn()s were consumed (RND)
-            self._perm_upload(rng, epoch + 1, total)
+            self._perm_upload(rng, epoch + 1)
 
     def _sync_grads(self, bank):
         if D.world_size() > 1:
@@ -722,7 +700,6 @@ class BaseAlgorithm(object):
             if not (seen == seen[0]).all():
                 raise RuntimeError("ppx: shard_shuffle='global' needs the numpy global RNG in the same state on every rank "
                                    "(seed all ranks alike and keep rank-dependent draws off np.random); digests: %s" % seen.tolist())
-        self._perm_keep = []
         if self._px and int(rb[steps * 8 + W].item()) != 0:
             raise RuntimeError("ppx: a peer-memory barrier timed out (a rank fell out of the sharded update)")
         self.last_losses = losses

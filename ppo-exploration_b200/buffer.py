@@ -16,7 +16,6 @@ The shuffle indices come from the same `np.random.permutation(T*N)` draw as the 
 """
 import atexit
 import ctypes as C
-import os
 import queue
 import threading
 import time
@@ -66,7 +65,7 @@ class _Task:
 
 class _WorkerPool:
     """Host worker threads that outlive the streams they serve.  A learner opens one HostRngStream per train() call (and
-    one speculative stream per call); starting and retiring three OS threads each time is not free for the GPU -- the
+    one speculative stream per call); starting and retiring an OS thread each time is not free for the GPU -- the
     address-space changes of thread stacks (mmap / madvise in a process with pinned CUDA mappings) showed up as one
     ~0.3 ms stall of the running kernels per pass on the bench host (tools/trace_sharded.py).  Idle workers are re-used;
     the pool only grows when every worker is busy (e.g. two learners with parked speculative streams)."""
@@ -105,8 +104,6 @@ def _stop_streams_at_exit():
         st.cancel()
     for st in list(_live_streams):
         st.t1.join(timeout=2.0)
-        for t in st.t2:
-            t.join(timeout=2.0)
 
 
 atexit.register(_stop_streams_at_exit)
@@ -174,46 +171,21 @@ class _PartnerPool:
 _partner_pool = _PartnerPool()
 
 
-def device_shuffle_default():
-    """Apply the shuffle's swaps on the GPU (shuffle_dev.cu: 58 us per 524 288 on the copy stream, against 0.9 ms on a host
-    core)?  Yes unless PPX_SHUFFLE_DEVICE=0: the host then only draws (0.3 ms per permutation), so a pass no longer depends
-    on how many cores the ranks of a node have to share (8 ranks on 16 cores) or on a noisy host.  The host-side swaps
-    remain for the sharded "global" shuffle (which needs the permutation on the host) and for n > 2^24."""
-    return os.environ.get("PPX_SHUFFLE_DEVICE", "1") != "0"
-
-
-def _apply_workers():
-    """Stage-2 threads of a HostRngStream: 2 (measured on the bench host: 50 -> 66M transitions/s at C2; 3-4 workers gain
-    nothing more, the draw stage and the GIL hand-offs then pace the stream), 1 when the ranks of this node have to share
-    the host cores.  PPX_SHUFFLE_WORKERS overrides."""
-    env = os.environ.get("PPX_SHUFFLE_WORKERS")
-    if env:
-        return max(1, int(env))
-    try:
-        cores = len(os.sched_getaffinity(0))
-    except AttributeError:
-        cores = os.cpu_count() or 4
-    ranks = max(1, int(os.environ.get("LOCAL_WORLD_SIZE", "1")))
-    return max(1, min(2, cores // ranks - 2))
-
-
 class HostRngStream:
-    """Replays a fixed script of draws of the numpy legacy RNG in worker threads, in order, so the host shuffle
+    """Replays a fixed script of draws of the numpy legacy RNG on a worker thread, in order, so the epoch shuffle
     (buffer.py:239) and RND's per-minibatch randn() (algorithms.py:468) overlap the GPU work while consuming exactly
-    the reference's random stream.  script items: ('perm', n) | ('randn',).
+    the reference's random stream.  script items: ('perm', n) | ('randn',).  A 'perm' item comes out as its
+    Fisher-Yates partner list (`DevicePartners`): the host draws, the device applies the swaps (shuffle_dev.cu: 58 us per
+    524 288 on the copy stream, against 0.9 ms on a host core).
 
     The stream works on a PRIVATE RandomState seeded with `state` (default: a snapshot of the global np.random state)
     and never touches the global one; the caller commits `final_state()` with np.random.set_state once the script has
     been consumed.  That makes a stream safe to start speculatively (before the caller knows it will be needed) and to
-    cancel.  Two pipelined stages (both release the GIL inside libppx): stage 1 (one thread) owns the RNG -- it draws
-    the Fisher-Yates partner sequence of each permutation and the scalar randn()s; stage 2 (`workers` threads, dealt the
-    permutations round-robin: only the DRAWS of successive permutations are sequential, their swaps are independent)
-    applies the swaps into a pinned buffer, running behind stage 1's published progress inside the permutation being
-    drawn.  Results come out in script order; at most `ahead` items are in flight or waiting."""
+    cancel.  The draw thread releases the GIL inside libppx.  Results come out in script order; at most `ahead` items
+    are in flight or waiting."""
 
-    def __init__(self, script, state=None, ahead=None, workers=None, device_apply=False, uploader=None):
+    def __init__(self, script, state=None, ahead=None, uploader=None):
         self.script = list(script)
-        self.device_apply = bool(device_apply)                  # 'perm' items come out as DevicePartners (n <= 2^24)
         # uploader(k, partners) -> CUDA event or None: called ON THE DRAW THREAD for the k-th permutation of the script as
         # soon as it is drawn; it queues the H2D copy + the device-side swaps, sets partners.ready and returns the event
         # that marks the end of the copy.  Before the draw thread would go idle (queue full, script done) it waits on the
@@ -222,44 +194,33 @@ class HostRngStream:
         # once per pass, after the last permutation).
         self.uploader = uploader
         self.profile, self.t_birth = [], time.perf_counter()    # per staged permutation: (start, wait+setup, draw, publish+stage) seconds
-        nw = int(workers) if workers is not None else _apply_workers()
-        self.nw = max(1, nw)
         if ahead is None:
             # a stream that stages its permutations itself may run through its whole script (the staging set holds every
-            # epoch; a speculative stream then prepares the whole next pass while this one computes); device_apply without
-            # an uploader has no stage 2: two finished permutations in hand are enough
-            ahead = max(2, len(self.script)) if uploader is not None else (2 if self.device_apply else self.nw + 2)
-        # results are delivered in script order through `q`: stage 1 enqueues one slot [event, value] per item BEFORE
-        # it dispatches the work, the stage-2 worker that owns the item fills it
+            # epoch; a speculative stream then prepares the whole next pass while this one computes); without an
+            # uploader two finished permutations in hand are enough
+            ahead = max(2, len(self.script)) if uploader is not None else 2
+        # results are delivered in script order through `q`: the draw thread enqueues one slot [event, value] per item
+        # BEFORE it draws the item, and fills it
         self.q = queue.Queue(maxsize=max(1, int(ahead)))
-        self.mids = [queue.Queue(maxsize=2) for _ in range(self.nw)]
         self.err = None
         self.cancelled = False
         self._final = None
         self.rs = np.random.RandomState()
         self.rs.set_state(np.random.get_state() if state is None else state)
-        script = self.script
-        self._jbufs = {}                                        # rotating partner buffers (<= ahead + 1 in flight per size)
         _live_streams.add(self)
-        # stage 2 is only needed when some permutation of the script is applied on the host
-        need2 = any(op[0] == 'perm' and not (self.device_apply and 2 <= int(op[1]) <= (1 << 24)) for op in script)
-        self.nw2 = self.nw if need2 else 0
-        self.t2 = [_workers.submit(self._apply, w) for w in range(self.nw2)]
-        self.t1 = _workers.submit(self._draw, list(script))
+        self.t1 = _workers.submit(self._draw, list(self.script))
 
-    def _put(self, qq, item):
+    def _put(self, item):
         while not self.cancelled:
             try:
-                qq.put(item, timeout=0.05)
+                self.q.put(item, timeout=0.05)
                 return True
             except queue.Full:
                 continue
         return False
 
     def _draw(self, script):
-        """Stage 1 (one thread, owns the RNG): draws in script order; permutations are handed round-robin to the
-        stage-2 workers -- the swaps of different permutations are independent, only the draws are sequential."""
-        k = 0
+        """The draw thread (owns the RNG): the partner list of each permutation and the scalar randn()s, in script order."""
         kperm = -1
         pending = None
         try:
@@ -271,7 +232,7 @@ class HostRngStream:
                 if pending is not None and self.q.full():       # about to block: see `uploader`
                     pending.synchronize()
                     pending = None
-                if not self._put(self.q, slot):
+                if not self._put(slot):
                     break
                 if op[0] == 'perm':
                     n = int(op[1])
@@ -279,45 +240,16 @@ class HostRngStream:
                     st = self.rs.get_state()
                     key = np.ascontiguousarray(st[1], dtype=np.uint32).copy()
                     pos = C.c_int(int(st[2]))
-                    if self.device_apply and 2 <= n <= (1 << 24):
-                        # draws only: the partner list goes to the device, which applies the swaps (shuffle_dev.cu)
-                        dp = _partner_pool.take(n)
-                        prog = np.zeros(1, np.int64)
-                        t0 = time.perf_counter()
-                        L.call("ppx_np_shuffle_draws32_stream", key.ctypes.data, C.byref(pos), n, dp.j.data_ptr(), prog.ctypes.data)
-                        t1 = time.perf_counter()
-                        self.rs.set_state((st[0], key, pos.value, st[3], st[4]))
-                        if self.uploader is not None and not self.cancelled:
-                            pending = self.uploader(kperm, dp)
-                        slot[1] = dp
-                        slot[0].set()
-                        t2 = time.perf_counter()
-                        self.profile.append((t_item - self.t_birth, t0 - t_item, t1 - t0, t2 - t1))
-                        continue
-                    small = n <= 0x7fffffff
-                    nbuf = self.q.maxsize + 2
-                    pool = self._jbufs.setdefault(n, [[(np.empty(max(n, 1), np.int32 if small else np.int64),
-                                                        np.zeros(1, np.int64)) for _ in range(nbuf)], 0])
-                    j, prog = pool[0][pool[1] % nbuf]
-                    pool[1] += 1
-                    mid = self.mids[k % self.nw]
-                    k += 1
-                    if small:
-                        # streaming: hand the buffer to stage 2 first, it runs behind the published progress counter
-                        prog[0] = 0
-                        if not self._put(mid, ('perm', j, n, prog, slot)):
-                            break
-                        try:
-                            L.call("ppx_np_shuffle_draws32_stream", key.ctypes.data, C.byref(pos), n, j.ctypes.data,
-                                   prog.ctypes.data)
-                        except Exception:
-                            prog[0] = 1 << 62                   # never leave stage 2 spinning on a failed draw
-                            raise
-                    else:
-                        L.call("ppx_np_shuffle_draws", key.ctypes.data, C.byref(pos), n, j.ctypes.data)
-                        if not self._put(mid, ('perm', j, n, None, slot)):
-                            break
+                    dp = _partner_pool.take(n)
+                    t0 = time.perf_counter()
+                    L.call("ppx_np_shuffle_draws32_stream", key.ctypes.data, C.byref(pos), n, dp.j.data_ptr())
+                    t1 = time.perf_counter()
                     self.rs.set_state((st[0], key, pos.value, st[3], st[4]))
+                    if self.uploader is not None and not self.cancelled:
+                        pending = self.uploader(kperm, dp)
+                    slot[1] = dp
+                    slot[0].set()
+                    self.profile.append((t_item - self.t_birth, t0 - t_item, t1 - t0, time.perf_counter() - t1))
                 else:
                     slot[1] = float(self.rs.randn())
                     slot[0].set()
@@ -325,38 +257,9 @@ class HostRngStream:
                 self._final = self.rs.get_state()
         except Exception as e:
             self.err = e
-        self._put(self.q, None)
-        for mid in self.mids:
-            self._put(mid, None)
+        self._put(None)
         if pending is not None:
             pending.synchronize()
-
-    def _apply(self, w):
-        """Stage 2 worker w: applies the swaps of the permutations dealt to it into a pinned buffer."""
-        scratch32 = None
-        mid = self.mids[w]
-        try:
-            while not self.cancelled:
-                try:
-                    item = mid.get(timeout=0.05)
-                except queue.Empty:
-                    continue
-                if item is None:
-                    break
-                _, j, n, prog, slot = item
-                out = torch.empty(n, dtype=torch.int64, pin_memory=torch.cuda.is_available())
-                if prog is not None:
-                    if scratch32 is None or scratch32.size < n:
-                        scratch32 = np.empty(max(n, 1), np.int32)
-                    L.call("ppx_np_shuffle_apply32_stream", j.ctypes.data, n, prog.ctypes.data,
-                           scratch32.ctypes.data, out.data_ptr())
-                else:
-                    L.call("ppx_np_shuffle_apply", j.ctypes.data, n, out.data_ptr())
-                slot[1] = out
-                slot[0].set()
-        except Exception as e:
-            self.err = e
-            self.cancelled = True                               # unblock everything; next() reports the error
 
     def next(self):
         slot = self.q.get()
@@ -368,7 +271,7 @@ class HostRngStream:
         return slot[1]
 
     def final_state(self):
-        """RNG state after the whole script (blocks until stage 1 has drawn everything)."""
+        """RNG state after the whole script (blocks until the draw thread has drawn everything)."""
         self.t1.join()
         if self.err is not None:
             raise self.err
@@ -380,8 +283,6 @@ class HostRngStream:
 
     def drain(self):
         self.t1.join()
-        for t in self.t2:
-            t.join()
 
 
 class BaseBuffer(object):

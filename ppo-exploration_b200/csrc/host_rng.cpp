@@ -10,16 +10,12 @@
 //   next_uint32:                MT19937 genrand with the standard tempering
 // The caller passes numpy's own state (np.random.get_state(): key[624], pos) and writes the advanced
 // state back with np.random.set_state, so interleaved numpy calls (e.g. RND's randn()) stay in sequence.
-// Two stages so they can pipeline across epochs AND inside one permutation: stage 1 draws the partner
-// sequence (RNG-bound; AVX-512 block rejection with compress-store when the CPU has it), stage 2 applies the
-// swaps (cache-miss-bound) and, in the streaming variant, starts as soon as the first partners are published.
+// The learner's shuffle only draws here -- the partner sequence (RNG-bound; AVX-512 block rejection with compress-store
+// when the CPU has it) -- and applies the swaps on the device (shuffle_dev.cu); ppx_np_permutation does both on the host.
 // Compiled by g++ (not nvcc): it uses target attributes / immintrin.
 #include <stdlib.h>
 #include <immintrin.h>
-#include <time.h>
 #include "common.cuh"
-
-extern "C" int ppx_np_shuffle_apply(const int64_t* j_host, int64_t n, int64_t* out_host);
 
 namespace {
 constexpr int MT_N = 624, MT_M = 397;
@@ -147,7 +143,7 @@ static inline void draw_partners(Mt& mt, int64_t n, int64_t* j_out) {
 
 // 32-bit variant of draw_partners for n <= 2^31: the mask only changes when i crosses a power of two, so the
 // inner loop runs with a constant mask straight over the tempered block (no per-draw clz, no call per word),
-// and the partner list is int32 (half the cache footprint for stage 2).  Same draw sequence.
+// and the partner list is int32.  Same draw sequence.
 static inline void draw_partners32(Mt& mt, int64_t n, int32_t* j_out) {
   int64_t i = n - 1;
   while (i >= 1) {
@@ -167,16 +163,8 @@ static inline void draw_partners32(Mt& mt, int64_t n, int32_t* j_out) {
   }
 }
 
-// stage 1: the swap partners j_i for i = n-1 .. 1 (j_out[i] = partner of position i; j_out[0] unused)
-extern "C" int ppx_np_shuffle_draws(uint32_t* key624_host, int* pos_host, int64_t n, int64_t* j_out_host) {
-  PPX_REQUIRE(key624_host && pos_host && j_out_host && n >= 0, "np_shuffle_draws: bad arguments");
-  PPX_REQUIRE(*pos_host >= 0 && *pos_host <= MT_N, "np_shuffle_draws: MT19937 pos=%d out of range", *pos_host);
-  Mt mt(key624_host, *pos_host);
-  draw_partners(mt, n, j_out_host);
-  *pos_host = mt.pos;
-  return PPX_OK;
-}
-
+// the swap partners j_i for i = n-1 .. 1 (j_out[i] = partner of position i; j_out[0] unused): the scalar reference
+// of the acceptance-order draw loop below
 extern "C" int ppx_np_shuffle_draws32(uint32_t* key624_host, int* pos_host, int64_t n, int32_t* j_out_host) {
   PPX_REQUIRE(key624_host && pos_host && j_out_host && n >= 0 && n <= 0x7fffffffll, "np_shuffle_draws32: bad arguments");
   PPX_REQUIRE(*pos_host >= 0 && *pos_host <= MT_N, "np_shuffle_draws32: MT19937 pos=%d out of range", *pos_host);
@@ -186,25 +174,8 @@ extern "C" int ppx_np_shuffle_draws32(uint32_t* key624_host, int* pos_host, int6
   return PPX_OK;
 }
 
-// stage 2 for the int32 partner list: swaps on an int32 scratch array (n*4 bytes: cache resident), widened into
-// the int64 output at the end
-extern "C" int ppx_np_shuffle_apply32(const int32_t* j_host, int64_t n, int32_t* scratch_host, int64_t* out_host) {
-  PPX_REQUIRE(j_host && scratch_host && out_host && n >= 0 && n <= 0x7fffffffll, "np_shuffle_apply32: bad arguments");
-  int32_t* __restrict__ a = scratch_host;
-  for (int64_t i = 0; i < n; ++i) a[i] = (int32_t)i;
-  for (int64_t i = n - 1; i >= 1; --i) {
-    const int32_t j = j_host[i];
-    const int32_t t = a[j];
-    a[j] = a[i];
-    a[i] = t;
-  }
-  for (int64_t i = 0; i < n; ++i) out_host[i] = (int64_t)a[i];
-  return PPX_OK;
-}
-
-// stage 2: arange(n) with the swaps applied
-extern "C" int ppx_np_shuffle_apply(const int64_t* j_host, int64_t n, int64_t* out_host) {
-  PPX_REQUIRE(j_host && out_host && n >= 0, "np_shuffle_apply: bad arguments");
+// arange(n) with the swaps applied
+static void np_shuffle_apply(const int64_t* j_host, int64_t n, int64_t* out_host) {
   for (int64_t i = 0; i < n; ++i) out_host[i] = i;
   for (int64_t i = n - 1; i >= 1; --i) {
     const int64_t j = j_host[i];
@@ -212,10 +183,9 @@ extern "C" int ppx_np_shuffle_apply(const int64_t* j_host, int64_t n, int64_t* o
     out_host[j] = out_host[i];
     out_host[i] = t;
   }
-  return PPX_OK;
 }
 
-// both stages back to back (single-threaded callers); out_host doubles as the partner buffer
+// draws and swaps back to back, on the host
 extern "C" int ppx_np_permutation(uint32_t* key624_host, int* pos_host, int64_t n, int64_t* out_host) {
   PPX_REQUIRE(key624_host && pos_host && out_host && n >= 0, "np_permutation: bad arguments");
   PPX_REQUIRE(*pos_host >= 0 && *pos_host <= MT_N, "np_permutation: MT19937 pos=%d out of range", *pos_host);
@@ -224,18 +194,15 @@ extern "C" int ppx_np_permutation(uint32_t* key624_host, int* pos_host, int64_t 
   if (!j) return ppx::fail(PPX_ERR_ARG, "np_permutation: out of host memory");
   draw_partners(mt, n, j);
   *pos_host = mt.pos;
-  const int rc = ppx_np_shuffle_apply(j, n, out_host);
+  np_shuffle_apply(j, n, out_host);
   free(j);
-  return rc;
+  return PPX_OK;
 }
 
 // ------------------------------------------------------------------------------------------------
-// Streaming pair: stage 1 writes the accepted partners in ACCEPTANCE order (acc[r] is the partner of position
-// i = n-1-r) and publishes how many are final through *progress (release); stage 2 runs behind it (acquire).
+// The learner's draw loop: the accepted partners in ACCEPTANCE order (acc[r] is the partner of position i = n-1-r).
 // ------------------------------------------------------------------------------------------------
 namespace {
-inline void publish(volatile int64_t* progress, int64_t r) { __atomic_store_n(progress, r, __ATOMIC_RELEASE); }
-
 #define PPX_DRAW_SCALAR_STEP()                                   \
   {                                                              \
     const uint32_t v = o[p++] & mask;                            \
@@ -245,8 +212,8 @@ inline void publish(volatile int64_t* progress, int64_t r) { __atomic_store_n(pr
     i -= ok;                                                     \
   }
 
-void draw_acc_base(Mt& mt, int64_t n, int32_t* acc, volatile int64_t* progress) {
-  int64_t i = n - 1, r = 0, last_pub = 0;
+void draw_acc_base(Mt& mt, int64_t n, int32_t* acc) {
+  int64_t i = n - 1, r = 0;
   while (i >= 1) {
     const uint32_t mask = 0xffffffffu >> __builtin_clz((uint32_t)i);
     const int64_t lo = (int64_t)(mask >> 1) + 1;
@@ -256,10 +223,8 @@ void draw_acc_base(Mt& mt, int64_t n, int32_t* acc, volatile int64_t* progress) 
       int p = mt.pos;
       while (p < MT_N && i >= lo) PPX_DRAW_SCALAR_STEP()
       mt.pos = p;
-      if (r - last_pub >= 8192) { publish(progress, r); last_pub = r; }
     }
   }
-  publish(progress, r);
 }
 
 // 64 (then 16) draws per step: with i the position at the start of the step, a draw v is certainly accepted if
@@ -268,8 +233,8 @@ void draw_acc_base(Mt& mt, int64_t n, int32_t* acc, volatile int64_t* progress) 
 // a register compress and a full-width store: the lanes past the packed ones land on entries a later step rewrites
 // (r + 16 <= n - 1 because the vector paths stop 16 positions above the end of the mask's range).
 __attribute__((target("avx512f,avx512bw,avx512vl,avx512dq,popcnt")))
-void draw_acc_avx512(Mt& mt, int64_t n, int32_t* acc, volatile int64_t* progress) {
-  int64_t i = n - 1, r = 0, last_pub = 0;
+void draw_acc_avx512(Mt& mt, int64_t n, int32_t* acc) {
+  int64_t i = n - 1, r = 0;
   while (i >= 1) {
     const uint32_t mask = 0xffffffffu >> __builtin_clz((uint32_t)i);
     const int64_t lo = (int64_t)(mask >> 1) + 1;
@@ -318,45 +283,17 @@ void draw_acc_avx512(Mt& mt, int64_t n, int32_t* acc, volatile int64_t* progress
       }
       while (p < MT_N && i >= lo && (p + 16 > MT_N || i - 16 < lo)) PPX_DRAW_SCALAR_STEP()
       mt.pos = p;
-      if (r - last_pub >= 8192) { publish(progress, r); last_pub = r; }
     }
   }
-  publish(progress, r);
 }
 }  // namespace
 
-extern "C" int ppx_np_shuffle_draws32_stream(uint32_t* key624_host, int* pos_host, int64_t n, int32_t* acc_host,
-                                             int64_t* progress_host) {
-  PPX_REQUIRE(key624_host && pos_host && acc_host && progress_host && n >= 0 && n <= 0x7fffffffll, "np_shuffle_draws32_stream: bad arguments");
+extern "C" int ppx_np_shuffle_draws32_stream(uint32_t* key624_host, int* pos_host, int64_t n, int32_t* acc_host) {
+  PPX_REQUIRE(key624_host && pos_host && acc_host && n >= 0 && n <= 0x7fffffffll, "np_shuffle_draws32_stream: bad arguments");
   PPX_REQUIRE(*pos_host >= 0 && *pos_host <= MT_N, "np_shuffle_draws32_stream: MT19937 pos=%d out of range", *pos_host);
   Mt mt(key624_host, *pos_host);
-  if (has_avx512()) draw_acc_avx512(mt, n, acc_host, progress_host);
-  else draw_acc_base(mt, n, acc_host, progress_host);
+  if (has_avx512()) draw_acc_avx512(mt, n, acc_host);
+  else draw_acc_base(mt, n, acc_host);
   *pos_host = mt.pos;
-  return PPX_OK;
-}
-
-extern "C" int ppx_np_shuffle_apply32_stream(const int32_t* acc_host, int64_t n, const int64_t* progress_host,
-                                             int32_t* scratch_host, int64_t* out_host) {
-  if (n == 0) return PPX_OK;
-  PPX_REQUIRE(acc_host && progress_host && scratch_host && out_host && n >= 0 && n <= 0x7fffffffll, "np_shuffle_apply32_stream: bad arguments");
-  int32_t* __restrict__ a = scratch_host;
-  for (int64_t i = 0; i < n; ++i) a[i] = (int32_t)i;
-  int64_t avail = 0;
-  for (int64_t r = 0; r + 1 < n; ++r) {
-    if (r >= avail) {
-      int spins = 0;
-      while ((avail = __atomic_load_n(progress_host, __ATOMIC_ACQUIRE)) <= r) {
-        if (++spins < 256) _mm_pause();
-        else { struct timespec ts = {0, 20000}; nanosleep(&ts, nullptr); }     // be polite on shared / throttled hosts
-      }
-    }
-    const int64_t i = n - 1 - r;
-    const int32_t j = acc_host[r];
-    const int32_t t = a[j];
-    a[j] = a[i];
-    a[i] = t;
-  }
-  for (int64_t i = 0; i < n; ++i) out_host[i] = (int64_t)a[i];
   return PPX_OK;
 }

@@ -22,8 +22,10 @@ namespace {
 
 constexpr int kScanBlock = 1024;       // elements per scan block (256 threads x 4)
 
+// n < 2^31: every index, count and scan offset fits an int (the offsets sum to at most n - 1 steps).  The grid-stride
+// loops count in int64_t because their last step may pass 2^31.
 __global__ void __launch_bounds__(256) fy_count_kernel(const int32_t* __restrict__ j, int n, int rev, int32_t* __restrict__ cnt) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x + 1; i < n; i += gridDim.x * blockDim.x) {
+  for (int64_t i = blockIdx.x * blockDim.x + threadIdx.x + 1; i < n; i += gridDim.x * blockDim.x) {
     const int t = j[rev ? n - 1 - i : i];
     if (t != i) atomicAdd(&cnt[t], 1);
   }
@@ -51,7 +53,7 @@ __global__ void __launch_bounds__(256) fy_scan1_kernel(const int32_t* __restrict
   for (int k = 0; k < 4; ++k) { if (base + k < n) out[base + k] = run; run += v[k]; }
   if (threadIdx.x == 0) bsum[blockIdx.x] = total;
 }
-// pass 2: one block turns the block totals into exclusive offsets (nb <= 16384)
+// pass 2: one block turns the block totals into exclusive offsets (any nb: each thread scans `per` of them)
 __global__ void __launch_bounds__(1024) fy_scan2_kernel(int32_t* __restrict__ bsum, int nb) {
   __shared__ int32_t s_w[32];
   const int per = (nb + 1023) / 1024, b0 = threadIdx.x * per;
@@ -73,16 +75,16 @@ __global__ void __launch_bounds__(1024) fy_scan2_kernel(int32_t* __restrict__ bs
 __global__ void __launch_bounds__(256) fy_scatter_kernel(const int32_t* __restrict__ j, int n, int rev, const int32_t* __restrict__ local,
                                                          const int32_t* __restrict__ bsum, int32_t* __restrict__ cursor,
                                                          int32_t* __restrict__ grp) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x + 1; i < n; i += gridDim.x * blockDim.x) {
+  for (int64_t i = blockIdx.x * blockDim.x + threadIdx.x + 1; i < n; i += gridDim.x * blockDim.x) {
     const int t = j[rev ? n - 1 - i : i];
-    if (t != i) grp[local[t] + bsum[t / kScanBlock] + atomicAdd(&cursor[t], 1)] = i;
+    if (t != i) grp[local[t] + bsum[t / kScanBlock] + atomicAdd(&cursor[t], 1)] = (int)i;
   }
 }
 // one thread per target: sort its (tiny) group by step index, emit first[p] and the nxt links
 __global__ void __launch_bounds__(256) fy_links_kernel(int n, const int32_t* __restrict__ cnt, const int32_t* __restrict__ local,
                                                        const int32_t* __restrict__ bsum, int32_t* __restrict__ grp,
                                                        int32_t* __restrict__ first, int32_t* __restrict__ nxt) {
-  for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < n; p += gridDim.x * blockDim.x) {
+  for (int64_t p = blockIdx.x * blockDim.x + threadIdx.x; p < n; p += gridDim.x * blockDim.x) {
     const int m = cnt[p];
     if (m == 0) { first[p] = -1; continue; }
     int32_t* g = grp + local[p] + bsum[p / kScanBlock];
@@ -100,10 +102,10 @@ __global__ void __launch_bounds__(256) fy_links_kernel(int n, const int32_t* __r
 // out[i]: follow the (strictly increasing) first[] chain from the step that last wrote the source position
 __global__ void __launch_bounds__(256) fy_resolve_kernel(const int32_t* __restrict__ j, int n, int rev, const int32_t* __restrict__ first,
                                                          const int32_t* __restrict__ nxt, int64_t* __restrict__ out) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+  for (int64_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const int t = i ? j[rev ? n - 1 - i : i] : 0;
     int q;
-    if (t == i) q = i;                                       // self-swap (and position 0): the content position i ends up with
+    if (t == i) q = (int)i;                                 // self-swap (and position 0): the content position i ends up with
     else { q = nxt[i]; if (q < 0) { out[i] = t; continue; } }
     int f;
     while ((f = first[q]) >= 0) q = f;
@@ -117,14 +119,14 @@ __global__ void __launch_bounds__(256) fy_resolve_kernel(const int32_t* __restri
 using namespace ppx;
 
 extern "C" int64_t ppx_np_shuffle_apply_device_workspace(int64_t n) {
-  if (n < 0 || n > (1ll << 24)) return -1;
+  if (n < 0 || n >= (1ll << 31)) return -1;
   const int64_t nb = ceil_div(std::max<int64_t>(n, 1), kScanBlock);
   return (int64_t)sizeof(int32_t) * (6 * std::max<int64_t>(n, 1) + nb + 64);
 }
 
 extern "C" int ppx_np_shuffle_apply_device(const int32_t* j_dev, int64_t n, int acceptance_order, void* workspace, int64_t* out_dev,
                                            void* stream) {
-  PPX_REQUIRE(n >= 0 && n <= (1ll << 24), "np_shuffle_apply_device: n=%lld (supported up to 2^24)", (long long)n);
+  PPX_REQUIRE(n >= 0 && n < (1ll << 31), "np_shuffle_apply_device: n=%lld (supported below 2^31)", (long long)n);
   if (n == 0) return PPX_OK;
   PPX_REQUIRE(j_dev && workspace && out_dev, "np_shuffle_apply_device: null pointer");
   cudaStream_t st = (cudaStream_t)stream;
@@ -153,7 +155,7 @@ extern "C" int ppx_np_shuffle_apply_device(const int32_t* j_dev, int64_t n, int 
 // worker thread of a rank > 0 needs no device bookkeeping of its own.
 extern "C" int ppx_np_shuffle_stage(const int32_t* j_host_pinned, int64_t n, int32_t* j_dev, void* workspace, int64_t* out_dev,
                                     void* stream, void* copied_event, void* ready_event) {
-  PPX_REQUIRE(n >= 2 && n <= (1ll << 24), "np_shuffle_stage: n=%lld (supported: 2 .. 2^24)", (long long)n);
+  PPX_REQUIRE(n >= 1 && n < (1ll << 31), "np_shuffle_stage: n=%lld (supported: 1 .. 2^31 - 1)", (long long)n);
   PPX_REQUIRE(j_host_pinned && j_dev && workspace && out_dev, "np_shuffle_stage: null pointer");
   cudaPointerAttributes at;
   PPX_CUDA(cudaPointerGetAttributes(&at, j_dev));

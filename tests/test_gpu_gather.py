@@ -74,7 +74,7 @@ def test_gather_vs_oracle_sizes(T, N, D, A, B):
     np.testing.assert_allclose(tot, arrs["returns"].astype(np.float64).sum(), rtol=1e-9)
 
 
-@pytest.mark.parametrize("n", [2, 3, 7, 1000, 4097, 524288, (1 << 21) + 5])
+@pytest.mark.parametrize("n", [1, 2, 3, 7, 1000, 4097, 524288, (1 << 21) + 5, 1 << 24, (1 << 24) + 1, (1 << 25) + 3])
 def test_device_shuffle_apply_matches_numpy(n):
     """Fisher-Yates swaps resolved in parallel on the device (shuffle_dev.cu) == np.random.permutation, bit for bit;
     the draws (the RNG stream itself) stay on the host and leave numpy's state where numpy would."""
@@ -91,8 +91,8 @@ def test_device_shuffle_apply_matches_numpy(n):
     assert np.array_equal(key, after[1]) and pos.value == after[2]
     # the streaming (AVX-512) draw loop leaves the same list in acceptance order: entry r belongs to position n-1-r
     key2 = np.ascontiguousarray(st[1], dtype=np.uint32).copy()
-    pos2, acc, prog = C.c_int(int(st[2])), np.zeros(n, np.int32), np.zeros(1, np.int64)
-    L.call("ppx_np_shuffle_draws32_stream", key2.ctypes.data, C.byref(pos2), n, acc.ctypes.data, prog.ctypes.data)
+    pos2, acc = C.c_int(int(st[2])), np.zeros(n, np.int32)
+    L.call("ppx_np_shuffle_draws32_stream", key2.ctypes.data, C.byref(pos2), n, acc.ctypes.data)
     assert np.array_equal(key2, after[1]) and pos2.value == after[2]
     ws = torch.empty(L.call("ppx_np_shuffle_apply_device_workspace", n), dtype=torch.uint8, device="cuda")
     out = torch.full((n,), -1, dtype=torch.int64, device="cuda")
@@ -104,27 +104,39 @@ def test_device_shuffle_apply_matches_numpy(n):
         assert np.array_equal(out.cpu().numpy(), want)
 
 
-def test_train_identical_with_device_shuffle():
-    """PPO.train() with the swaps applied on the device consumes the same RNG stream and produces the same minibatches:
-    bit-identical weights and the same numpy state afterwards (speculative streams included)."""
+def _check_train_stages_numpy_permutations(T, N, batch_size, n_epochs, calls):
+    """Every PPO.train() call stages each epoch's np.random.permutation(T*N) on the device bit for bit, drawn from the
+    global numpy stream as the reference draws it, and leaves numpy's state where those draws leave it."""
     import ppo_exploration_b200 as ppx
-    rs = np.random.RandomState(0)
-    T, N, D, A = 32, 16, 8, 2
-    arrs = dict(observations=rs.randn(T, N, D).astype(np.float32), actions=rs.randn(T, N, A), rewards=rs.randn(T, N).astype(np.float32),
-                values=rs.randn(T, N).astype(np.float32), masks=(rs.rand(T, N) < 0.05).astype(np.uint8),
-                action_log_probs=(-1.0 + 0.1 * rs.randn(T, N, A)).astype(np.float32))
-    res = []
-    for dev in (False, True):
-        np.random.seed(3); torch.manual_seed(3)
-        env = ppx.SyntheticVecEnv(N, D, ppx.Box((A,)), seed=0)
-        m = ppx.PPO(env=env, nstep=T, hidden_size=64, batch_size=128, n_epochs=3)
-        m.device_shuffle = dev
-        m.rollout.load_rollout(**arrs)
-        m.rollout.compute_returns_and_advantages(torch.zeros(N), arrs["masks"][-1])
-        for _ in range(3):                                   # the 2nd and 3rd calls run on the speculative stream
-            m.train()
-        torch.cuda.synchronize()
-        res.append(({k: v.clone() for k, v in m.policy.state_dict().items()}, np.random.get_state()))
-    for k in res[0][0]:
-        assert torch.equal(res[0][0][k], res[1][0][k]), k
-    assert np.array_equal(res[0][1][1], res[1][1][1]) and res[0][1][2] == res[1][1][2]
+    D, A, total = 8, 2, T * N
+    np.random.seed(3)
+    want = [np.random.permutation(total) for _ in range(calls * n_epochs)]
+    after = np.random.get_state()
+    env = ppx.SyntheticVecEnv(N, D, ppx.Box((A,)), seed=0)
+    m = ppx.PPO(env=env, nstep=T, hidden_size=64, batch_size=batch_size, n_epochs=n_epochs)
+    g = torch.Generator(device="cuda").manual_seed(0)
+    rnd = lambda *shape: torch.randn(*shape, generator=g, device="cuda")
+    m.rollout.load_rollout(observations=rnd(T, N, D), actions=rnd(T, N, A).double(), rewards=rnd(T, N), values=rnd(T, N),
+                           masks=(torch.rand(T, N, generator=g, device="cuda") < 0.05).to(torch.uint8),
+                           action_log_probs=-1.0 + 0.1 * rnd(T, N, A))
+    m.rollout.compute_returns_and_advantages(torch.zeros(N), torch.zeros(N))
+    np.random.seed(3)
+    for c in range(calls):
+        spec = m._spec[0] if m._spec is not None else None
+        m.train()
+        assert c == 0 or m._last_rng is spec
+        got = m._perm_all.view(n_epochs, total).cpu().numpy()
+        for e in range(n_epochs):
+            assert np.array_equal(got[e], want[c * n_epochs + e]), (c, e)
+    st = np.random.get_state()
+    assert np.array_equal(st[1], after[1]) and st[2] == after[2]
+
+
+def test_train_stages_numpy_permutations():
+    """Three train() calls: the 2nd and 3rd run on the stream pre-drawn by the call before."""
+    _check_train_stages_numpy_permutations(32, 16, 128, 3, 3)
+
+
+def test_train_stages_numpy_permutations_above_2_24():
+    """2^24 + 4096 indices per epoch, in minibatches of C2's size."""
+    _check_train_stages_numpy_permutations(4097, 4096, 131072, 2, 1)

@@ -18,15 +18,14 @@ for n in (524288, 1 << 20, 1 << 21, 1 << 22):
     st = np.random.get_state()
     key, pos = np.ascontiguousarray(st[1], dtype=np.uint32).copy(), C.c_int(int(st[2]))
     acc = torch.empty(n, dtype=torch.int32, pin_memory=True)
-    prog = np.zeros(1, np.int64)
     best = 1e9
     for _ in range(5):
         t0 = time.perf_counter()
-        L.call("ppx_np_shuffle_draws32_stream", key.ctypes.data, C.byref(pos), n, acc.data_ptr(), prog.ctypes.data)
+        L.call("ppx_np_shuffle_draws32_stream", key.ctypes.data, C.byref(pos), n, acc.data_ptr())
         best = min(best, time.perf_counter() - t0)
     line = f"n={n}: bare draws {best * 1e3:.3f} ms = {best / n * 1e9:.3f} ns/draw"
     for rep in range(3):
-        s = HostRngStream([('perm', n)] * 10, device_apply=True)
+        s = HostRngStream([('perm', n)] * 10)
         t0 = time.perf_counter()
         for _ in range(10):
             s.next().release()                          # as the learner does once the H2D copy is queued

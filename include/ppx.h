@@ -495,6 +495,23 @@ int ppx_rollout_record_step(const void* rewards, int rewards_f64, const uint8_t*
                             float* rewards_row, double* rewards_f64_row, uint8_t* masks_row, float* int_rewards_row,
                             int64_t* episodes, void* stream);
 
+/* ---------------------------------------------------------------- policy evaluation --------- */
+/* Env-facing actions of an evaluation step (evaluate.cu; DESIGN.md §3.17) from the policy forward's actor_out [N,A] (log_std
+ * [A]: Box only): Box f64 [N,A], Discrete int64 [N] into env_actions.  deterministic: Box (double)tanhf(actor_out), the
+ * sampled action of ppx_policy_sample at z = 0; Discrete the index of the largest logit, lowest on ties.  Otherwise one
+ * draw with ppx_policy_sample's arithmetic, Philox counter (row_offset + n, draw): rows of a sharded call equal the same rows
+ * of one call over all envs.  `draw` must have bit 63 set (the training stream counts up from 1).  One launch. */
+int ppx_policy_act_eval(const float* actor_out, const float* log_std, int64_t N, int A, int discrete, int deterministic,
+                        uint64_t seed, uint64_t draw, int64_t row_offset, void* env_actions, void* stream);
+/* After env.step of evaluation step `step`: env n (global env g = env_offset + n of total_envs) records its first
+ * (n_eval_episodes + g) / total_envs finished episodes (dones[n] != 0): ep_returns[n] (f64), ep_lengths[n] (int64) and
+ * `step` go to row n, column counts[n] of the [N, kmax] tables (kmax >= ceil(n_eval_episodes / total_envs)), then
+ * counts[n] += 1.  Later episodes are ignored.  state: int64 [3], zero before the first step; state[2] receives the number
+ * of episodes this rank still misses (the other two words are re-armed scratch).  One launch. */
+int ppx_eval_episode_step(const uint8_t* dones, const double* ep_returns, const int64_t* ep_lengths, int64_t N,
+                          int64_t n_eval_episodes, int64_t env_offset, int64_t total_envs, int64_t step, int64_t* counts,
+                          double* out_ret, int64_t* out_len, int64_t* out_end, int64_t kmax, int64_t* state, void* stream);
+
 /* ---------------------------------------------------------------- classic control ----------- */
 /* Gym 0.17 classic-control envs with TimeLimit, on the device (classic_control.cu; DESIGN.md §3.13).  env: 0 CartPole-v1,
  * 1 MountainCar-v0, 2 MountainCarContinuous-v0, 3 Pendulum-v0.  State f64 [S, N] (S = 4, 2, 2, 2), observations f32 [N, D]

@@ -15,8 +15,9 @@ from .evolution_strategies import EvolutionStrategy
 from .spaces import Box, Discrete, SyntheticVecEnv
 from .env import VecNormalize
 from .classic_control import ClassicControlVecEnv, EpisodeMonitor, ToNumpy, make_env
+from .evaluation import evaluate_policy
 
 __all__ = ["BaseBuffer", "RolloutStorage", "IntrinsicStorage", "CountTable", "discount_with_dones", "Policy",
            "RndNetwork", "IntrinsicCuriosityModule", "ActionConverter", "RunningMeanStd", "normalize_obs",
            "BaseAlgorithm", "PPO", "PPO_RND", "PPO_ICM", "EvolutionStrategy", "Box", "Discrete", "SyntheticVecEnv", "logger", "VecNormalize", "ConvTrunk", "ParamBank",
-           "ClassicControlVecEnv", "EpisodeMonitor", "ToNumpy", "make_env"]
+           "ClassicControlVecEnv", "EpisodeMonitor", "ToNumpy", "make_env", "evaluate_policy"]

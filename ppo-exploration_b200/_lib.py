@@ -134,6 +134,8 @@ SIGNATURES = {
     "ppx_policy_sample": (c_i, [c_p, c_p, c_l, c_i, c_i, c_u, c_u, c_p, c_p, c_p]),
     "ppx_policy_act_record": (c_i, [c_p, c_p, c_p, c_p, c_p, c_l, c_i, c_i, c_i, c_u, c_u, c_p, c_p, c_p, c_p, c_p, c_p, c_p]),
     "ppx_rollout_record_step": (c_i, [c_p, c_i, c_p, c_p, c_l, c_p, c_p, c_p, c_p, c_p, c_p]),
+    "ppx_policy_act_eval": (c_i, [c_p, c_p, c_l, c_i, c_i, c_i, c_u, c_u, c_l, c_p, c_p]),
+    "ppx_eval_episode_step": (c_i, [c_p, c_p, c_p, c_l, c_l, c_l, c_l, c_l, c_p, c_p, c_p, c_p, c_l, c_p, c_p]),
     "ppx_classic_step": (c_i, [c_i, c_l, c_l, c_u, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_p, c_p, c_p]),
     "ppx_classic_reset": (c_i, [c_i, c_l, c_l, c_u, c_p, c_p, c_p, c_p, c_p, c_p, c_p]),
     "ppx_episode_monitor_step": (c_i, [c_p, c_i, c_p, c_l, c_p, c_p, c_p, c_p, c_p]),

@@ -148,7 +148,7 @@ class BaseAlgorithm(object):
                      "count_table": ro.count_table.state_dict() if ro.count_table is not None else None},
             counters={"num_timesteps": int(self.num_timesteps), "num_episodes": int(self.num_episodes),
                       "n_updates": int(self._n_updates), "draws": int(self.policy._draws),
-                      "sample_seed": int(self.policy._sample_seed)},
+                      "sample_seed": int(self.policy._sample_seed), "eval_draws": int(self.policy._eval_draws)},
             host={"ep_info_buffer": [{k: scalar(v) for k, v in e.items()} for e in self.ep_info_buffer],
                   "ep_info_maxlen": self._ep_info_buffer.maxlen, "last_obs": pack(self.last_obs),
                   "device_env": bool(self.device_env), "last_dones": pack(getattr(self, "last_dones", None)),
@@ -178,7 +178,7 @@ class BaseAlgorithm(object):
         return self
 
     def _load_state(self, ck):
-        from .checkpoint import np_rng_tuple, unpack
+        from .checkpoint import counters, np_rng_tuple, unpack
         for k, b in self._ckpt_banks().items():
             b.load_state_dict(ck["banks"][k])
         for k, r in self._ckpt_rms().items():
@@ -191,9 +191,9 @@ class BaseAlgorithm(object):
             raise ValueError("the checkpoint and this learner disagree on sim_hash")
         if ro.count_table is not None:
             ro.count_table.load_state_dict(sh["count_table"])
-        c, h = ck["counters"], ck["host"]
+        c, h = counters(ck), ck["host"]
         self.num_timesteps, self.num_episodes, self._n_updates = c["num_timesteps"], c["num_episodes"], c["n_updates"]
-        self.policy._draws, self.policy._sample_seed = c["draws"], c["sample_seed"]
+        self.policy._draws, self.policy._sample_seed, self.policy._eval_draws = c["draws"], c["sample_seed"], c["eval_draws"]
         load_env = getattr(self.env, "load_state_dict", None)
         self.resumed_env_state = callable(load_env) and ck["env"] is not None
         if self.resumed_env_state:
@@ -299,6 +299,11 @@ class BaseAlgorithm(object):
         self.device_env = isinstance(self.last_obs, torch.Tensor) and self.last_obs.is_cuda
         if self.device_env and self._episodes_dev is None:
             self._episodes_dev = torch.zeros(1, dtype=torch.int64, device=self.device)
+
+    def predict(self, obs, deterministic=True):
+        """The policy's actions for `obs` (`Policy.predict`: numpy or CUDA, [N, D] or [D]); draws nothing from the
+        training's random streams."""
+        return self.policy.predict(obs, deterministic)
 
     # ---- shared pieces of the fused update --------------------------------------------------
     def _record(self, key, value):
@@ -707,9 +712,18 @@ class BaseAlgorithm(object):
             self._record(k, float(np.mean(losses[:, i])))
         self._n_updates += self.n_epochs
 
-    def _learn_loop(self, total_timesteps, log_interval, reward_target, log_name=None, log_to_file=False):
+    def _learn_loop(self, total_timesteps, log_interval, reward_target, log_name=None, log_to_file=False, eval_env=None,
+                    eval_freq=1, n_eval_episodes=10):
         """algorithms.py:261-308 / 504-543 / 715-756.  With log_to_file (or when no logger was passed) the run is logged
-        through ppx's own logger module, which writes the reference's CSV schema (logger.py:13-52, :222-246)."""
+        through ppx's own logger module, which writes the reference's CSV schema (logger.py:13-52, :222-246).
+
+        eval_env (an env on the GPU with `episode_stats()`, ppx.evaluate_policy): every eval_freq-th iteration, after
+        collect_samples() and before the log row is written, the current policy plays n_eval_episodes deterministic
+        episodes there and eval/mean_reward, eval/std_reward and eval/mean_ep_length are recorded.  The evaluation draws
+        nothing from the training's random streams and writes nothing the training reads, so the run itself is the one
+        without eval_env, bit for bit.  reward_target stays a bound on the training episodes' mean return."""
+        if eval_env is not None and (int(eval_freq) < 1 or int(n_eval_episodes) < 1):
+            raise ValueError(f"eval_freq={eval_freq} and n_eval_episodes={n_eval_episodes} must be >= 1")
         if log_to_file or self.logger is None:
             from . import logger as ppx_logger
             ppx_logger.configure(log_name or type(self).__name__, str(self.env_id), log_to_file)
@@ -718,6 +732,12 @@ class BaseAlgorithm(object):
         while self.num_timesteps < total_timesteps:
             self.collect_samples()
             iteration += 1
+            if eval_env is not None and iteration % int(eval_freq) == 0:
+                from .evaluation import evaluate_policy
+                rets, lens = evaluate_policy(self, eval_env, n_eval_episodes)
+                self._record("eval/mean_reward", float(np.mean(rets)))
+                self._record("eval/std_reward", float(np.std(rets)))
+                self._record("eval/mean_ep_length", float(np.mean(lens)))
             if log_interval is not None and iteration % log_interval == 0:
                 self._record("time/total timesteps", self.num_timesteps)
                 if len(self.ep_info_buffer) > 0 and len(self.ep_info_buffer[0]) > 0:
@@ -821,9 +841,11 @@ class PPO(BaseAlgorithm):
         self._finish_train(step, ("train/total_loss", "train/policy_gradient_loss", "train/value_loss",
                                   "train/entropy_loss"))
 
-    def learn(self, total_timesteps, log_interval, reward_target=None, log_to_file=False):
+    def learn(self, total_timesteps, log_interval, reward_target=None, log_to_file=False, eval_env=None, eval_freq=1,
+              n_eval_episodes=10):
         name = "PPO_SimHash" if self.sim_hash else "PPO"                       # algorithms.py:270-275
-        return self._learn_loop(total_timesteps, log_interval, reward_target, name, log_to_file)
+        return self._learn_loop(total_timesteps, log_interval, reward_target, name, log_to_file, eval_env, eval_freq,
+                                n_eval_episodes)
 
 
 class PPO_RND(BaseAlgorithm):
@@ -972,8 +994,10 @@ class PPO_RND(BaseAlgorithm):
         self._finish_train(step, ("train/total_loss", "train/policy_gradient_loss", "train/value_loss",
                                   "train/entropy_loss", "train/intrinsic_loss"))
 
-    def learn(self, total_timesteps, log_interval, reward_target=None, log_to_file=False):
-        return self._learn_loop(total_timesteps, log_interval, reward_target, "PPO_RND", log_to_file)
+    def learn(self, total_timesteps, log_interval, reward_target=None, log_to_file=False, eval_env=None, eval_freq=1,
+              n_eval_episodes=10):
+        return self._learn_loop(total_timesteps, log_interval, reward_target, "PPO_RND", log_to_file, eval_env, eval_freq,
+                                n_eval_episodes)
 
 
 class PPO_ICM(BaseAlgorithm):
@@ -1101,5 +1125,7 @@ class PPO_ICM(BaseAlgorithm):
         self._finish_train(step, keys)
         self._record("train/icm_loss", float(np.mean(self.last_losses[:, 5])))
 
-    def learn(self, total_timesteps, log_interval=5, reward_target=None, log_to_file=False):
-        return self._learn_loop(total_timesteps, log_interval, reward_target, "PPO_ICM", log_to_file)
+    def learn(self, total_timesteps, log_interval=5, reward_target=None, log_to_file=False, eval_env=None, eval_freq=1,
+              n_eval_episodes=10):
+        return self._learn_loop(total_timesteps, log_interval, reward_target, "PPO_ICM", log_to_file, eval_env, eval_freq,
+                                n_eval_episodes)

@@ -31,6 +31,15 @@ def check(ck, cls_name):
         raise ValueError(f"the checkpoint holds a {ck.get('class')!r}, not a {cls_name!r}")
 
 
+# counters added after version 1 was first written, with the value a file without them stands for
+_COUNTER_DEFAULTS = {"eval_draws": 0}
+
+
+def counters(ck):
+    """The checkpoint's counters, with the default of every counter the file predates."""
+    return dict(_COUNTER_DEFAULTS, **ck["counters"])
+
+
 def np_rng_state(state=None):
     """numpy's legacy MT19937 state (default: the global `np.random` one) as a uint32 key tensor plus ints and a float."""
     name, key, pos, has_gauss, cached = np.random.get_state() if state is None else state

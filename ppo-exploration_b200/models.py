@@ -648,6 +648,7 @@ class Policy:
         self.mlp = ParallelMLP(self.bank, self.names, self.state_dim, hidden_size, self.outs, self.scratch)
         self.net = self                                           # reference code reaches policy.net.parameters()
         self._sample_seed, self._draws = int(torch.initial_seed()) & 0x7FFFFFFFFFFFFFFF, 0
+        self._eval_draws = 0                                      # stochastic predict / evaluate_policy calls (EVAL_DRAW)
         self._init_like_reference()
 
     # ---- initialisation / weight exchange ----
@@ -755,6 +756,45 @@ class Policy:
                rollout.action_log_probs[p].data_ptr(), vals[0].data_ptr(), vals[1].data_ptr() if self.intrinsic else None,
                env_actions.data_ptr(), L.stream())
         return (env_actions, *vals)
+
+    # Draw numbers of the evaluation stream: bit 63 set (the training stream counts up from 1, so the two never meet), the
+    # evaluation call (`_eval_draws`) in bits 32-62 and the step within the call in bits 0-31.
+    EVAL_DRAW = 1 << 63
+
+    def eval_actions(self, obs, deterministic, draw=0, row_offset=0, out=None):
+        """The env-facing actions for `obs` (CUDA f32 [N, D], contiguous): one forward, then ONE launch (evaluate.cu) --
+        deterministic: Box tanh(mean) f64 [N, A], Discrete the argmax of the logits int64 [N]; otherwise one draw from the
+        policy's distribution with the Philox counter (row_offset + n, draw).  No rollout row, log-prob or value is written
+        and neither draw counter moves.  `out`: the action buffer to write (default a new one)."""
+        outs = self.forward_raw(obs)
+        N, A = outs[0].shape
+        discrete = self.action_type == "Discrete"
+        if out is None:
+            out = torch.empty((N,) if discrete else (N, A), dtype=torch.int64 if discrete else torch.float64, device=self.device)
+        L.call("ppx_policy_act_eval", outs[0].data_ptr(), None if discrete else self.bank.p("action_log_std"), N, A, int(discrete),
+               int(bool(deterministic)), self._sample_seed, int(draw), int(row_offset), out.data_ptr(), L.stream())
+        return out
+
+    def predict(self, obs, deterministic=True):
+        """Actions for observations `obs` ([N, D] or one [D]; numpy or a CUDA tensor), on the side they came from: a CUDA
+        tensor gives a CUDA tensor, anything else numpy.  Box: f64 [N, A] ([A] for one observation); Discrete: int64 [N]
+        (a scalar array for one).  deterministic=True: the distribution's mode as `eval_actions` forms it.  deterministic=False:
+        one draw from the evaluation stream, a Philox stream of its own -- the training stream (`_draws`) is not touched, so
+        calling predict() changes nothing in a run that goes on training."""
+        on_gpu = isinstance(obs, torch.Tensor) and obs.is_cuda
+        x = obs if isinstance(obs, torch.Tensor) else torch.as_tensor(np.asarray(obs, dtype=np.float32))
+        if x.dim() not in (1, 2) or x.shape[-1] != self.state_dim:
+            raise ValueError(f"predict: observations must be [N, {self.state_dim}] or [{self.state_dim}], got {tuple(x.shape)}")
+        single = x.dim() == 1
+        x = x.reshape(-1, self.state_dim).to(self.device, torch.float32).contiguous()
+        draw = 0
+        if not deterministic:
+            self._eval_draws += 1
+            draw = self.EVAL_DRAW | (self._eval_draws << 32)
+        a = self.eval_actions(x, deterministic, draw)
+        if single:
+            a = a[0]
+        return a if on_gpu else a.cpu().numpy()
 
     def evaluate(self, obs, actions):
         """models.py:52-73 / 101-124 as plain tensors (train() uses the fused loss kernel instead)."""

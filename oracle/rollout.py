@@ -273,26 +273,37 @@ class VecNormalizeRef(object):
     """numpy restatement of stable_baselines3.common.vec_env.VecNormalize.step_wait with norm_obs / norm_reward (the wrapper
     the reference puts around its envs, env.py:11) -- NOT part of the reference tree and not installed here: PARITY UNPINNED
     upstream; the arithmetic below is the published one (running moments = the reference's own util.py:9-44 rule, which is
-    pinned by tests/golden/rnd_bonus.npz)."""
+    pinned by tests/golden/rnd_bonus.npz).
 
-    def __init__(self, n_envs, obs_shape, clip_obs=10.0, clip_reward=10.0, gamma=0.99, epsilon=1e-8):
+    `training` and `norm_reward` follow the published step_wait / _update_reward: the observation and return statistics
+    are updated, and the discounted returns accumulated, only while training (`norm_reward` does not matter for that);
+    the rewards are divided only with norm_reward; a done zeroes its return in every mode.  This flag logic is equally a
+    restatement of the published code, not checked against an installed stable_baselines3: parity is still unpinned."""
+
+    def __init__(self, n_envs, obs_shape, clip_obs=10.0, clip_reward=10.0, gamma=0.99, epsilon=1e-8, training=True,
+                 norm_reward=True):
         self.obs_rms, self.ret_rms = RunningMeanStd(shape=obs_shape), RunningMeanStd(shape=())
         self.ret = np.zeros(n_envs)
         self.clip_obs, self.clip_reward, self.gamma, self.epsilon = clip_obs, clip_reward, gamma, epsilon
+        self.training, self.norm_reward = training, norm_reward
 
     def reset(self, obs):
         self.ret = np.zeros_like(self.ret)
-        self.obs_rms.update(obs)
+        if self.training:
+            self.obs_rms.update(obs)
         return self.normalize_obs(obs)
 
     def normalize_obs(self, obs):
         return np.clip((obs - self.obs_rms.mean) / np.sqrt(self.obs_rms.var + self.epsilon), -self.clip_obs, self.clip_obs)
 
     def step(self, obs, rews, dones):
-        self.ret = self.ret * self.gamma + rews
-        self.obs_rms.update(obs)
+        if self.training:
+            self.obs_rms.update(obs)
         obs_n = self.normalize_obs(obs)
-        self.ret_rms.update(self.ret)
-        rews_n = np.clip(rews / np.sqrt(self.ret_rms.var + self.epsilon), -self.clip_reward, self.clip_reward)
+        if self.training:                                   # _update_reward
+            self.ret = self.ret * self.gamma + rews
+            self.ret_rms.update(self.ret)
+        if self.norm_reward:
+            rews = np.clip(rews / np.sqrt(self.ret_rms.var + self.epsilon), -self.clip_reward, self.clip_reward)
         self.ret[dones] = 0
-        return obs_n, rews_n
+        return obs_n, rews

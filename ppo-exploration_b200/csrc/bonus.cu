@@ -226,15 +226,12 @@ extern "C" int ppx_obs_istd(const double* var, int dim, double* istd, void* stre
 extern "C" int ppx_normalize_obs(const float* obs, int64_t n, int dim, const double* mean, const double* var, float* out, void* stream) {
   PPX_REQUIRE(obs && mean && var && out && n >= 0 && dim >= 1, "normalize_obs: bad arguments");
   if (n == 0) return PPX_OK;
-  static double* istd = nullptr; static int istd_cap = 0;       // per-process scratch (stream-ordered, one learner thread)
-  if (dim > istd_cap) {
-    PPX_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
-    if (istd) cudaFree(istd);
-    PPX_CUDA(cudaMalloc((void**)&istd, (size_t)dim * sizeof(double)));
-    istd_cap = dim;
-  }
+  static GrowOnlyScratch scratch;                               // stream-ordered, one learner thread
+  int rc = grow_scratch(scratch, (size_t)dim * sizeof(double));
+  if (rc) return rc;
+  double* istd = (double*)scratch.p;
   obs_istd_kernel<<<(unsigned)ceil_div(dim, 256), 256, 0, (cudaStream_t)stream>>>(var, dim, istd);
-  int rc = after_launch("normalize_obs(istd)");
+  rc = after_launch("normalize_obs(istd)");
   if (rc) return rc;
   const unsigned gx = (unsigned)ceil_div(dim, 1024);
   const unsigned gy = (unsigned)std::max<int64_t>(1, std::min<int64_t>(n, ceil_div((int64_t)sm_count() * 16, gx)));
@@ -252,14 +249,12 @@ extern "C" int ppx_rnd_sqerr(const float* pred, const float* target, int64_t n, 
 extern "C" int ppx_rnd_normalize_rollout(float* r, int T, int N, double* mean, double* var, double* count, void* stream) {
   PPX_REQUIRE(r && mean && var && count && T >= 1 && N >= 1, "rnd_normalize_rollout: bad arguments");
   cudaStream_t st = (cudaStream_t)stream;
-  static double* mom = nullptr; static int mom_cap = 0;
-  if (T > mom_cap) {
-    if (mom) cudaFree(mom);
-    PPX_CUDA(cudaMalloc((void**)&mom, (size_t)T * 2 * sizeof(double)));
-    mom_cap = T;
-  }
+  static GrowOnlyScratch scratch;
+  int rc = grow_scratch(scratch, (size_t)T * 2 * sizeof(double));
+  if (rc) return rc;
+  double* mom = (double*)scratch.p;
   row_moments_kernel<<<T, 256, 0, st>>>(r, N, mom);
-  int rc = after_launch("rnd_normalize_rollout(moments)");
+  rc = after_launch("rnd_normalize_rollout(moments)");
   if (rc) return rc;
   merge_rows_kernel<<<1, 32, 0, st>>>(mom, T, N, mean, var, count);
   rc = after_launch("rnd_normalize_rollout(merge)");
@@ -316,29 +311,32 @@ vecnorm_obs_kernel(const float* __restrict__ obs, int64_t n, int dim, const doub
   }
 }
 
-// one CTA: ret = ret * gamma + r; ret_rms.update(ret); r_out = clip(r / sqrt(ret_var + eps), +-clip); ret[done] = 0
+// one CTA.  While training (update): ret = ret * gamma + r; ret_rms.update(ret).  Then r_out = clip(r / sqrt(ret_var + eps),
+// +-clip) and ret[done] = 0.  As in stable_baselines3's step_wait, the returns do not accumulate when not training.
 __global__ void __launch_bounds__(1024)
 vecnorm_reward_kernel(const float* __restrict__ r, const uint8_t* __restrict__ done, double* __restrict__ ret, int n, double gamma,
                       double* mean, double* var, double* count, double eps, float clip, int update, float* __restrict__ out) {
   __shared__ double s_red[32];
   __shared__ double s_var;
-  double a = 0.0;
-  for (int i = threadIdx.x; i < n; i += blockDim.x) {
-    const double v = ret[i] * gamma + (double)r[i];
-    ret[i] = v;
-    a += v;
-  }
-  const double bm = block_sum(a, s_red) / (double)n;
-  a = 0.0;
-  for (int i = threadIdx.x; i < n; i += blockDim.x) { const double d = ret[i] - bm; a += d * d; }
-  const double bv = block_sum(a, s_red) / (double)n;
-  if (threadIdx.x == 0) {
-    double m = *mean, v = *var;
-    if (update) {
+  if (update) {
+    double a = 0.0;
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+      const double v = ret[i] * gamma + (double)r[i];
+      ret[i] = v;
+      a += v;
+    }
+    const double bm = block_sum(a, s_red) / (double)n;
+    a = 0.0;
+    for (int i = threadIdx.x; i < n; i += blockDim.x) { const double d = ret[i] - bm; a += d * d; }
+    const double bv = block_sum(a, s_red) / (double)n;
+    if (threadIdx.x == 0) {
+      double m = *mean, v = *var;
       merge_moments(bm, bv, (double)n, m, v, *count);
       *mean = m; *var = v; *count += (double)n;
+      s_var = v;
     }
-    s_var = v;
+  } else if (threadIdx.x == 0) {
+    s_var = *var;
   }
   __syncthreads();
   const double inv = 1.0 / sqrt(s_var + eps);

@@ -23,6 +23,25 @@ inline int after_launch(const char* what, int n = 1) {
 
 inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
+// Per-process device scratch of an entry point that only grows.  A CUDA graph captured by an earlier call holds the
+// address of the block it saw, so a call that needs more allocates a new block and never frees the old one (at least
+// doubling, so the retired blocks add up to less than the live one).  Nothing is synchronised.  A learner's warm pass
+// sizes the block before it captures a graph; a block a graph holds is never freed.
+struct GrowOnlyScratch {
+  void* p = nullptr;
+  size_t cap = 0;
+};
+inline int grow_scratch(GrowOnlyScratch& s, size_t bytes) {
+  if (bytes <= s.cap) return PPX_OK;
+  const size_t n = std::max(bytes, 2 * s.cap);
+  void* q = nullptr;
+  const cudaError_t e = cudaMalloc(&q, n);
+  if (e != cudaSuccess) return fail(PPX_ERR_CUDA, "scratch of %zu bytes: %s", n, cudaGetErrorString(e));
+  s.p = q;
+  s.cap = n;
+  return PPX_OK;
+}
+
 }  // namespace ppx
 
 #define PPX_REQUIRE(cond, ...)                                    \

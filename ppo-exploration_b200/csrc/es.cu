@@ -707,18 +707,12 @@ extern "C" int ppx_knn_novelty(const double* archive, int64_t M, const double* q
   // archive split: enough warps to fill the machine for few queries, >= 256 points per warp
   int splits = (int)std::max<int64_t>(1, std::min<int64_t>(ceil_div(M, 256), ceil_div(8 * (int64_t)sm_count(), Q)));
   splits = std::min(splits, 1024);
-  static double* cand = nullptr;                       // per-process scratch; calls are stream-ordered (one learner thread)
-  static size_t cand_cap = 0;
-  const size_t need = (size_t)Q * splits * K * sizeof(double);
-  if (need > cand_cap) {
-    PPX_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
-    cudaFree(cand);
-    cand = nullptr; cand_cap = 0;
-    PPX_CUDA(cudaMalloc((void**)&cand, need));
-    cand_cap = need;
-  }
-  dim3 grid((unsigned)splits, (unsigned)Q);
   PPX_REQUIRE(Q <= 65535, "knn_novelty: Q=%d exceeds grid.y; call in slices", Q);
+  static GrowOnlyScratch scratch;                      // calls are stream-ordered (one learner thread)
+  const int rs = grow_scratch(scratch, (size_t)Q * splits * K * sizeof(double));
+  if (rs) return rs;
+  double* cand = (double*)scratch.p;
+  dim3 grid((unsigned)splits, (unsigned)Q);
   if (K <= 16) {
     knn_slice_kernel<16><<<grid, 32, 0, (cudaStream_t)stream>>>(archive, M, queries, dim, K, splits, cand);
     int rc = after_launch("knn_novelty(slices)");

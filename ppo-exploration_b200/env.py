@@ -110,16 +110,21 @@ class VecNormalize(object):
         if self.training and self.norm_obs:
             self.obs_rms.update(obs_d)
         obs_n = self.normalize_obs(obs_d)
-        if self.norm_reward:
-            out = torch.empty_like(r_d)
-            L.call("ppx_vecnorm_reward", r_d.data_ptr(), d_d.data_ptr(), self.ret.data_ptr(), self.num_envs, self.gamma,
-                   self.ret_rms.mean_dev.data_ptr(), self.ret_rms.var_dev.data_ptr(), self.ret_rms.count_dev.data_ptr(), self.epsilon,
-                   self.clip_reward, int(self.training), out.data_ptr(), L.stream())
-            r_d = out
-        else:
-            self.ret.mul_(self.gamma).add_(r_d.double())
-            self.ret[d_d.bool()] = 0.0
-        return obs_n, r_d, dones, infos
+        out = self._reward_step(r_d, d_d)
+        return obs_n, r_d if out is None else out, dones, infos
+
+    def _reward_step(self, r_d, d_d):
+        """stable_baselines3's step_wait: while training, the discounted returns accumulate and update ret_rms, with or
+        without norm_reward; the rewards are divided only with norm_reward; a done zeroes its return either way.
+        Returns the normalised rewards (f32 CUDA), or None without norm_reward."""
+        if not (self.training or self.norm_reward):
+            self.ret.masked_fill_(d_d.bool(), 0.0)                  # not boolean indexing: that syncs
+            return None
+        out = torch.empty_like(r_d)
+        L.call("ppx_vecnorm_reward", r_d.data_ptr(), d_d.data_ptr(), self.ret.data_ptr(), self.num_envs, self.gamma,
+               self.ret_rms.mean_dev.data_ptr(), self.ret_rms.var_dev.data_ptr(), self.ret_rms.count_dev.data_ptr(), self.epsilon,
+               self.clip_reward, int(self.training), out.data_ptr(), L.stream())
+        return out if self.norm_reward else None
 
     # ---- inner env on the GPU: the same arithmetic, no host upload ----
     def _reset_cuda(self, o):
@@ -140,13 +145,5 @@ class VecNormalize(object):
         if self.training and self.norm_obs:
             self.obs_rms.update(obs_d)
         obs_n = self.normalize_obs(obs_d)
-        out = torch.empty_like(r_d)
-        if self.norm_reward:
-            L.call("ppx_vecnorm_reward", r_d.data_ptr(), d_d.data_ptr(), self.ret.data_ptr(), self.num_envs, self.gamma,
-                   self.ret_rms.mean_dev.data_ptr(), self.ret_rms.var_dev.data_ptr(), self.ret_rms.count_dev.data_ptr(), self.epsilon,
-                   self.clip_reward, int(self.training), out.data_ptr(), L.stream())
-        else:
-            out.copy_(r_d)
-            self.ret.mul_(self.gamma).add_(r_d.double())
-            self.ret.masked_fill_(d_d.bool(), 0.0)                  # not boolean indexing: that syncs
-        return obs_n, out, d_d, infos
+        out = self._reward_step(r_d, d_d)
+        return obs_n, r_d.clone() if out is None else out, d_d, infos

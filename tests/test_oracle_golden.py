@@ -114,6 +114,33 @@ def test_running_mean_std():
     assert np.array_equal(rv.mean, g["rmsv_mean"]) and np.array_equal(rv.var, g["rmsv_var"])
 
 
+@pytest.mark.parametrize("norm_reward", [True, False])
+def test_vecnormalize_restatement_flags(norm_reward):
+    """VecNormalizeRef's training / norm_reward logic (stable_baselines3's step_wait / _update_reward): the statistics
+    and the returns move only while training, whatever norm_reward; rewards are divided only with norm_reward; a done
+    zeroes its return in every mode."""
+    rs = np.random.RandomState(0)
+    n, gamma = 5, 0.9
+    v = OR.VecNormalizeRef(n, (2,), gamma=gamma, norm_reward=norm_reward)
+    v.reset(rs.randn(n, 2))
+    ret = np.zeros(n)
+    for step in range(12):
+        v.training = not (4 <= step < 8)
+        obs, r, done = rs.randn(n, 2), rs.randn(n) * 3, rs.rand(n) < 0.3
+        before = (v.obs_rms.count, v.ret_rms.count, v.ret_rms.var.copy(), v.obs_rms.mean.copy())
+        _, out = v.step(obs, r, done)
+        if v.training:
+            ret = ret * gamma + r
+            assert v.obs_rms.count == before[0] + n and v.ret_rms.count == before[1] + n
+        else:
+            assert (v.obs_rms.count, v.ret_rms.count) == before[:2]
+            assert np.array_equal(v.ret_rms.var, before[2]) and np.array_equal(v.obs_rms.mean, before[3])
+        want = np.clip(r / np.sqrt(v.ret_rms.var + 1e-8), -10, 10) if norm_reward else r
+        assert np.array_equal(out, want)
+        ret[done] = 0
+        assert np.array_equal(v.ret, ret)
+
+
 def _params(g, prefix, requires_grad=True):
     out = {}
     for k, v in g.group(prefix).items():

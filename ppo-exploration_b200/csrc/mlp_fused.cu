@@ -61,8 +61,10 @@ struct RedP {
 __host__ __device__ constexpr int round4(int x) { return (x + 3) & ~3; }
 
 // tanh(x) = 1 - 2 / (1 + e^{2x}) with ex2.approx / rcp.approx: 5 instructions instead of ~17 for tanhf, ABSOLUTE
-// error <= ~2e-7 on [-1, 1] outputs (the hidden activations enter the next layer as absolute values; measured against
-// the fp64 reference in tests/test_gpu_mlp_fused.py).  Saturates correctly: e -> inf gives 1, e -> 0 gives -1.
+// error <= 3e-7 on [-1, 1] outputs (the hidden activations enter the next layer as absolute values).  The bound: about
+// one ulp of r = 1 / (1 + e) from rcp.approx and half an ulp of 1 + e (each worth up to 1.2e-7 once doubled), two ulp
+// of e from ex2.approx (up to 1.2e-7 near x = 0), the final fma's rounding.  Measured maximum 2.2e-7 (at x = -2.66) on
+// exact arguments over [-32, 32] in tests/test_gpu_mlp_edges.py.  Saturates correctly: e -> inf gives 1, e -> 0 gives -1.
 __device__ __forceinline__ float tanh_fast(float x) {
   float e, r;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(x * 2.8853900817779268f));
